@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--env snake|crypto|traffic|climate|builder]   # this repo's CUDA engine
     python bench.py --impl reference [--gpus N] --steps K --warmup W [--env …]  # CPU arm: the reference's step loop
+    python bench.py … --dump-outputs DIR   # also write the last timed step's outputs as DIR/*.npy (dump_step_outputs)
 
 A "step" is ONE launch of the fused step kernel over the whole batch, inputs resident in HBM; `value` =
 envs x steps x ranks / max-over-ranks device time (CUDA events).  `e2e` is the same metric through the
@@ -447,6 +448,54 @@ def pcie_ceiling(torch, dev, nbytes):
     return out
 
 
+DUMP_MAX_BYTES = 64_000_000
+
+
+def _flatten(name, value, out):
+    if isinstance(value, dict):  # a Dict observation or the infos (nested "episode" dict, lazily computed entries)
+        for k in value.keys():
+            _flatten(f"{name}.{k}", value[k], out)
+    else:
+        out[name] = value
+
+
+def dump_step_outputs(directory, step_out, n):
+    """Write what one step() returned -- (obs, reward, terminated, truncated, infos) -- as <directory>/<name>.npy, dict
+    entries under dotted names (obs.grid, info.episode.r, ...).  Values float32 holds exactly (float32 and narrower
+    floats, bool, 8- and 16-bit integers) are written as float32, the rest as float64.  float64 holds integers exactly
+    only up to 2**53 in magnitude, so a wider integer value (a 64-bit counter or hash) is refused rather than written
+    rounded.  Arrays with one row per env keep
+    the rows of a fixed sample of envs when all of them would pass DUMP_MAX_BYTES: the sample is drawn from a fixed seed
+    and sorted, the same for every array, and written as env_index.npy, so that two runs with the same arguments write
+    the same files and two builds can be compared array by array."""
+    import numpy as np
+    import torch
+
+    narrow = (torch.float32, torch.float16, torch.bfloat16, torch.bool, torch.int8, torch.uint8, torch.int16)
+    arrays = {}
+    for name, value in zip(("obs", "reward", "terminated", "truncated", "info"), step_out):
+        _flatten(name, value, arrays)
+    arrays = {k: torch.as_tensor(v) for k, v in arrays.items()}
+    for k, v in arrays.items():
+        wide = v.to(torch.int64) if not v.dtype.is_floating_point and v.dtype != torch.bool and v.numel() else None
+        if wide is not None and (int(wide.max()) > 2 ** 53 or int(wide.min()) < -2 ** 53):
+            raise ValueError(f"--dump-outputs: {k} holds integers beyond 2**53, which float64 cannot store exactly")
+    out_dtype = {k: torch.float32 if v.dtype in narrow else torch.float64 for k, v in arrays.items()}
+    per_env = [k for k, v in arrays.items() if v.dim() >= 1 and v.shape[0] == n]
+    row_bytes = 8 + sum(arrays[k][0].numel() * out_dtype[k].itemsize for k in per_env)  # 8: the env_index entry
+    other_bytes = sum(v.numel() * out_dtype[k].itemsize for k, v in arrays.items() if k not in per_env)
+    keep = min(n, (DUMP_MAX_BYTES - other_bytes - 128 * (len(arrays) + 1)) // row_bytes)  # 128: one .npy header
+    index = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "env_index.npy"), index.astype(np.float64))
+    for k, v in arrays.items():
+        if k in per_env and keep < n:
+            v = v.index_select(0, torch.as_tensor(index, device=v.device))
+        np.save(os.path.join(directory, f"{k}.npy"), v.to(out_dtype[k]).cpu().numpy())
+    print(f"bench: wrote {len(arrays) + 1} arrays of the last timed step ({keep} of {n} envs) to {directory}",
+          file=sys.stderr)
+
+
 def bench_env(ctx, env_name, n, steps, warmup, e2e_steps):
     """Time one env's step kernel (device-resident) and its host-buffer C-ABI call (end to end) on every rank.
     Returns the measurement block on rank 0 (None elsewhere).  All ranks must call this in the same order."""
@@ -499,7 +548,7 @@ def bench_env(ctx, env_name, n, steps, warmup, e2e_steps):
     sampler.start()
     ev0.record(stream)
     for t in range(steps):
-        env.step(tapes[(warmup + t) % pool])
+        last = env.step(tapes[(warmup + t) % pool])
     ev1.record(stream)
     torch.cuda.synchronize(dev)
     launches = lib.beng_launch_count() - launches0
@@ -512,13 +561,16 @@ def bench_env(ctx, env_name, n, steps, warmup, e2e_steps):
         for t in range(steps):
             scratch.fill_(t & 0xFF)  # evicts the previous step's lines from L2 (not timed)
             pairs[t][0].record(stream)
-            env.step(tapes[(warmup + t) % pool])
+            last = env.step(tapes[(warmup + t) % pool])
             pairs[t][1].record(stream)
         torch.cuda.synchronize(dev)
         launches = lib.beng_launch_count() - launches0
         ms = sum(a.elapsed_time(b) for a, b in pairs)
         del scratch
     sampler.stop()
+    if args.dump_outputs and env_name == args.env and rank == 0:
+        # here, not later: step() returns the env's own buffers, which the steps below overwrite
+        dump_step_outputs(args.dump_outputs, last, n)
     barrier()
     ms_t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -652,9 +704,12 @@ def run_b200_arm(args):
     if os.environ.get("NCCL_DEBUG", "").upper() in ("VERSION", "INFO") and not os.environ.get("NCCL_DEBUG_FILE"):
         # NCCL's banner and communicator lines would precede the JSON line on stdout.  Each rank logs to its own file
         # (eight ranks writing to one stderr pipe garble each other's lines); rank 0 replays the version and
-        # "comm ... rank R nranks N" lines to stderr at the end, where whoever asked for them (the driver's rank check)
-        # sees them whole.  stdout carries the JSON line only.
-        nccl_logs = os.path.join(ROOT, "gpurun_out")
+        # "comm ... rank R nranks N" lines to stderr at the end, where whoever asked for them sees them whole.  stdout
+        # carries the JSON line only.  The files go to one temporary directory per user that every rank of the host
+        # can name before NCCL starts, never into the source tree.
+        import tempfile
+
+        nccl_logs = os.path.join(tempfile.gettempdir(), f"bench_nccl_logs_{os.getuid()}")
         os.makedirs(nccl_logs, exist_ok=True)
         os.environ["NCCL_DEBUG_FILE"] = os.path.join(nccl_logs, "nccl.%h.%p.log")
     t_start = time.time()
@@ -752,7 +807,15 @@ def main():
     ap.add_argument("--no-secondary", action="store_true",
                     help="snake only: skip the crypto and traffic blocks that the default run appends as `secondary`")
     ap.add_argument("--no-l2-flush", action="store_true", help="traffic only: time back-to-back steps (L2-warm)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="b200 arm only: after the timed steps, write what the last one returned (--env's step(), rank 0) as "
+                         "DIR/<name>.npy, float32/float64, at most 64 MB in all (a fixed sample of envs when larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what this repo's CUDA engine computed; the reference arm has nothing to dump")
+    sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
     args.warmup = max(args.warmup, 3)
     if args.envs_per_gpu is None:
         args.envs_per_gpu = WORKLOADS[args.env].envs_per_gpu

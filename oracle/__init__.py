@@ -13,6 +13,7 @@ Contents
   snake_port.py    pure-Python restatement of SnakeEnvClassic (the CPU-baseline "port")
   c/               plain-C restatement (fast checker for GPU-scale parity), built into oracle/_c/
   gen_golden.py    drives the real reference and writes tests/golden/*.npz
+  golden_files.py  reads and writes tests/golden/*.npz (one env's vectors split over files of at most 1 MB)
 
 Parity pin: the reference holds no golden vectors (SURVEY.md section 4: zero asserts).
 The pin is tests/golden/*.npz, produced by gen_golden.py from the reference itself run

@@ -23,9 +23,8 @@ import zlib
 
 import numpy as np
 
-from . import philox, ref_loader, replay
+from . import golden_files, philox, ref_loader, replay
 
-OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden", "snake_golden.npz")
 
 # name, grid, n_envs, n_steps, seed, env_id_base, policy
 CASES = [
@@ -138,8 +137,8 @@ def main():
               "max final score", int(blob[f"{n}/final_score"].max()))
     blob.update(frozen_case(mod))
     blob["cases"] = np.array([c[0] for c in CASES])
-    np.savez_compressed(OUT, **blob)
-    print("wrote", os.path.normpath(OUT), os.path.getsize(OUT), "bytes")
+    for path in golden_files.save("snake", blob):
+        print("wrote", os.path.relpath(path), os.path.getsize(path), "bytes")
 
 
 if __name__ == "__main__":

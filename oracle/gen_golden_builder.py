@@ -14,9 +14,8 @@ import os
 
 import numpy as np
 
-from . import ref_loader, replay
+from . import golden_files, ref_loader, replay
 
-OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden", "builder_golden.npz")
 
 # name, n_envs, n_steps, seed, env_id_base, policy, grid
 CASES = [
@@ -92,8 +91,8 @@ def main():
     finally:
         gl.np = real_np
     blob["cases"] = np.array([c[0] for c in CASES])
-    np.savez_compressed(OUT, **blob)
-    print("wrote", os.path.normpath(OUT), os.path.getsize(OUT), "bytes")
+    for path in golden_files.save("builder", blob):
+        print("wrote", os.path.relpath(path), os.path.getsize(path), "bytes")
 
 
 if __name__ == "__main__":

@@ -13,9 +13,8 @@ import os
 
 import numpy as np
 
-from . import ref_loader, replay
+from . import golden_files, ref_loader, replay
 
-OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden", "climate_golden.npz")
 
 # name, n_envs, n_steps, seed, env_id_base, policy, ctor kwargs
 CASES = [
@@ -84,8 +83,8 @@ def main():
               float(blob[f"{n}/room_temp"].min()), float(blob[f"{n}/room_temp"].max()),
               "people max", int(blob[f"{n}/num_people"].max()))
     blob["cases"] = np.array([c[0] for c in CASES])
-    np.savez_compressed(OUT, **blob)
-    print("wrote", os.path.normpath(OUT), os.path.getsize(OUT), "bytes")
+    for path in golden_files.save("climate", blob):
+        print("wrote", os.path.relpath(path), os.path.getsize(path), "bytes")
 
 
 if __name__ == "__main__":

@@ -18,9 +18,8 @@ import os
 
 import numpy as np
 
-from . import philox, ref_loader, replay
+from . import golden_files, philox, ref_loader, replay
 
-OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden", "crypto_golden.npz")
 SNAP_EVERY = 23
 
 # name, n_envs, n_steps, seed, env_id_base, action mode
@@ -115,8 +114,8 @@ def main():
     blob["custom_cfg"] = np.array([CUSTOM_CFG[k] for k in ("initial_balance", "trading_fee_rate", "slippage_rate",
                                                            "min_price", "max_price", "volatility_base",
                                                            "market_psychology_factor")])
-    np.savez_compressed(OUT, **blob)
-    print("wrote", os.path.normpath(OUT), os.path.getsize(OUT), "bytes")
+    for path in golden_files.save("crypto", blob):
+        print("wrote", os.path.relpath(path), os.path.getsize(path), "bytes")
 
 
 if __name__ == "__main__":

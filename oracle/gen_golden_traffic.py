@@ -13,9 +13,8 @@ import zlib
 
 import numpy as np
 
-from . import philox, ref_loader, replay
+from . import golden_files, philox, ref_loader, replay
 
-OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden", "traffic_golden.npz")
 SNAP_EVERY = 9
 PHASE = {"NS_GREEN": 0, "NS_YELLOW": 1, "EW_GREEN": 2, "EW_YELLOW": 3}
 
@@ -95,8 +94,8 @@ def main():
         print(n, "episodes", int(blob[f"{n}/terminated"].sum()), "max vehicles", int(blob[f"{n}/num_vehicles"].max()),
               "max queue", int(blob[f"{n}/qlen"].max()), "last reward", blob[f"{n}/reward"][0, -1])
     blob["cases"] = np.array([c[0] for c in CASES])
-    np.savez_compressed(OUT, **blob)
-    print("wrote", os.path.normpath(OUT), os.path.getsize(OUT), "bytes")
+    for path in golden_files.save("traffic", blob):
+        print("wrote", os.path.relpath(path), os.path.getsize(path), "bytes")
 
 
 if __name__ == "__main__":

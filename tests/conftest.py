@@ -25,9 +25,9 @@ def pytest_sessionstart(session):
 
 @pytest.fixture(scope="session")
 def golden():
-    import numpy as np
+    from oracle import golden_files
 
-    return np.load(os.path.join(ROOT, "tests", "golden", "snake_golden.npz"))
+    return golden_files.load("snake")
 
 
 @pytest.fixture(scope="session")

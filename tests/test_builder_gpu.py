@@ -1,13 +1,13 @@
 """GPU parity tests for world_builder_env (SURVEY.md section 8f rank 3): CUDA path (through the C ABI) against the CPU
 oracle and the golden vectors recorded from the reference.  Integer dynamics: EXACT (array equality everywhere)."""
-import os
 
 import numpy as np
 import pytest
 import torch
 
+from oracle import golden_files
+
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DEV = "cuda:0"
 CASES = ["random_g10", "random_hi_ids", "farmer_g10", "spam_g10", "farmer_g4"]
 
@@ -23,7 +23,7 @@ def pkg():
 
 @pytest.fixture(scope="module")
 def bgold():
-    return np.load(os.path.join(ROOT, "tests", "golden", "builder_golden.npz"))
+    return golden_files.load("builder")
 
 
 def np_(t):

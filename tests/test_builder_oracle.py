@@ -1,20 +1,18 @@
 """The C oracle of WorldBuilderEnv (SURVEY.md section 8f rank 3) against golden vectors produced by the reference itself
 (tests/golden/builder_golden.npz) and, in the build container, the live reference.  Integer dynamics: EXACT."""
-import os
 
 import numpy as np
 import pytest
 
-from oracle import ref_loader, replay
+from oracle import golden_files, ref_loader, replay
 from oracle.c_oracle import BuilderOracle
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CASES = ["random_g10", "random_hi_ids", "farmer_g10", "spam_g10", "farmer_g4"]
 
 
 @pytest.fixture(scope="module")
 def bgold():
-    return np.load(os.path.join(ROOT, "tests", "golden", "builder_golden.npz"))
+    return golden_files.load("builder")
 
 
 def meta(g, name):
@@ -66,7 +64,8 @@ def test_invalid_action_and_modes():
     assert dis.terminated.all() and (dis.reward == -100).all() and (dis.resources[:, 3] == 0).all()
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="needs /root/reference (build container)")
+@pytest.mark.skipif(not ref_loader.reference_available(),
+                    reason="needs the original project's sources (BENG_REFERENCE_ROOT=<its checkout>)")
 def test_c_oracle_matches_live_reference():
     env_mod, gl = ref_loader.load_builder()
     real_np = gl.np

@@ -4,14 +4,14 @@ CPU oracle and the golden vectors recorded from the reference.
 Tolerances: float32 observations and float64 state/rewards are compared at rtol 1e-5 / atol 1e-6 and rtol 1e-9 (the only
 source of difference is CUDA's log/cos vs glibc's in the Box-Muller normal draw); integer fields (people, step, comfort
 time, RNG counter, terminated) are exact."""
-import os
 
 import numpy as np
 import pytest
 import torch
 
+from oracle import golden_files
+
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DEV = "cuda:0"
 RTOL, ATOL, RTOL64 = 1e-5, 1e-6, 1e-9
 CASES = ["random_default", "random_hi_ids", "thermostat", "extremes", "small_office"]
@@ -28,7 +28,7 @@ def pkg():
 
 @pytest.fixture(scope="module")
 def kgold():
-    return np.load(os.path.join(ROOT, "tests", "golden", "climate_golden.npz"))
+    return golden_files.load("climate")
 
 
 def np_(t):

@@ -2,21 +2,19 @@
 reference itself (tests/golden/climate_golden.npz) and, in the build container, the live reference.  EXACT: the
 oracle evaluates the reference's float64 expressions in the same order on the same libm."""
 import logging
-import os
 
 import numpy as np
 import pytest
 
-from oracle import ref_loader, replay
+from oracle import golden_files, ref_loader, replay
 from oracle.c_oracle import ClimateOracle
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CASES = ["random_default", "random_hi_ids", "thermostat", "extremes", "small_office"]
 
 
 @pytest.fixture(scope="module")
 def kgold():
-    return np.load(os.path.join(ROOT, "tests", "golden", "climate_golden.npz"))
+    return golden_files.load("climate")
 
 
 def meta(g, name):
@@ -53,7 +51,8 @@ def test_reference_facts(kgold):
     assert g["small_office/num_people"].max() <= 3
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="needs /root/reference (build container)")
+@pytest.mark.skipif(not ref_loader.reference_available(),
+                    reason="needs the original project's sources (BENG_REFERENCE_ROOT=<its checkout>)")
 def test_c_oracle_matches_live_reference():
     mod = ref_loader.load_climate()
     n, T, seed = 3, 1600, 44

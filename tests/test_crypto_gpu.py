@@ -13,6 +13,8 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import golden_files
+
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -34,7 +36,7 @@ def pkg():
 
 @pytest.fixture(scope="module")
 def cgold():
-    return np.load(os.path.join(ROOT, "tests", "golden", "crypto_golden.npz"))
+    return golden_files.load("crypto")
 
 
 def np_(t):

@@ -7,17 +7,16 @@ import os
 import numpy as np
 import pytest
 
-from oracle import ref_loader, replay
+from oracle import golden_files, ref_loader, replay
 from oracle.c_oracle import CRYPTO_DEFAULT_CFG, CryptoOracle
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CASES = ["discrete_random", "discrete_hi_ids", "discrete_buyer", "discrete_seller", "discrete_hold",
          "continuous_random", "custom_config"]
 
 
 @pytest.fixture(scope="module")
 def cgold():
-    return np.load(os.path.join(ROOT, "tests", "golden", "crypto_golden.npz"))
+    return golden_files.load("crypto")
 
 
 def meta(g, name):
@@ -93,7 +92,8 @@ def test_next_step_and_disabled_modes(cgold):
     assert (nxt.state()["step"][only_limit] == 2).all() and (same.state()["step"][only_limit] == 3).all()
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="needs /root/reference (build container)")
+@pytest.mark.skipif(not ref_loader.reference_available(),
+                    reason="needs the original project's sources (BENG_REFERENCE_ROOT=<its checkout>)")
 def test_c_oracle_matches_live_reference():
     mod = ref_loader.load_crypto()
     real_np = mod.np

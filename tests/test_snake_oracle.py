@@ -139,7 +139,8 @@ def test_full_board_leaves_no_food():
     assert seen_full
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="needs /root/reference (build container)")
+@pytest.mark.skipif(not ref_loader.reference_available(),
+                    reason="needs the original project's sources (BENG_REFERENCE_ROOT=<its checkout>)")
 @pytest.mark.parametrize("G,seed,policy", [(20, 21, "random"), (8, 22, "greedy"), (6, 23, "greedy")])
 def test_c_oracle_matches_live_reference(G, seed, policy):
     from oracle.gen_golden import greedy_action

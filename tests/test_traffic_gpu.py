@@ -1,16 +1,16 @@
 """GPU parity tests for traffic_management_env: the CUDA path (through the C ABI) against the CPU oracle and the
 golden vectors recorded from the reference.  Integer dynamics and float64-of-integer reward/observation: EXACT
 (observations compared bit for bit via array equality / crc32; float64 rewards compared with ==)."""
-import os
 import zlib
 
 import numpy as np
 import pytest
 import torch
 
+from oracle import golden_files
+
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DEV = "cuda:0"
 CASES = ["random_default", "random_hi_ids", "all_zero", "all_ns", "all_ew", "alternate", "custom_grid"]
 
@@ -26,7 +26,7 @@ def pkg():
 
 @pytest.fixture(scope="module")
 def tgold():
-    return np.load(os.path.join(ROOT, "tests", "golden", "traffic_golden.npz"))
+    return golden_files.load("traffic")
 
 
 def np_(t):

@@ -1,22 +1,20 @@
 """The C oracle of TrafficManagementEnv against golden vectors produced by the reference itself
 (tests/golden/traffic_golden.npz) and, in the build container, the live reference.  Everything is integer
 dynamics + float64 expressions of integers in the reference's order: the comparison is EXACT."""
-import os
 import zlib
 
 import numpy as np
 import pytest
 
-from oracle import philox, ref_loader, replay
+from oracle import golden_files, philox, ref_loader, replay
 from oracle.c_oracle import TrafficOracle
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CASES = ["random_default", "random_hi_ids", "all_zero", "all_ns", "all_ew", "alternate", "custom_grid"]
 
 
 @pytest.fixture(scope="module")
 def tgold():
-    return np.load(os.path.join(ROOT, "tests", "golden", "traffic_golden.npz"))
+    return golden_files.load("traffic")
 
 
 def meta(g, name):
@@ -83,7 +81,8 @@ def test_modes_and_masked_reset(tgold):
     assert same.state()["timestep"].tolist() == [0, 3, 0]
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="needs /root/reference (build container)")
+@pytest.mark.skipif(not ref_loader.reference_available(),
+                    reason="needs the original project's sources (BENG_REFERENCE_ROOT=<its checkout>)")
 def test_c_oracle_matches_live_reference():
     env_mod, utils_mod = ref_loader.load_traffic()
     n, T, seed = 3, 1100, 31
