@@ -50,9 +50,10 @@ __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.p
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
-// Launch `kern<<<grid, block, smem, stream>>>(arg)` with the PDL attribute (BENG_NO_PDL=1 disables it).
-template <typename Kern, typename Arg>
-inline cudaError_t launch_pdl(Kern kern, dim3 grid, dim3 block, size_t smem, cudaStream_t stream, const Arg &arg) {
+// Launch `kern<<<grid, block, smem, stream>>>(args...)` with the PDL attribute (BENG_NO_PDL=1 disables it) and count
+// the attempt in g_launch_count.
+template <typename Kern, typename... Args>
+inline cudaError_t launch_pdl(Kern kern, dim3 grid, dim3 block, size_t smem, cudaStream_t stream, const Args &...args) {
     static const bool use_pdl = getenv("BENG_NO_PDL") == nullptr;
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = grid;
@@ -64,7 +65,14 @@ inline cudaError_t launch_pdl(Kern kern, dim3 grid, dim3 block, size_t smem, cud
     attr[0].val.programmaticStreamSerializationAllowed = use_pdl ? 1 : 0;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kern, arg);
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args...);
+    g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    return e;
+}
+
+// Device -> host copy of `bytes` on `stream` for an optional output: a null `dst` is skipped.
+inline cudaError_t d2h(void *dst, const void *src, size_t bytes, cudaStream_t stream) {
+    return dst ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, stream) : cudaSuccess;
 }
 
 // streaming (evict-first) 128-bit / 64-bit global loads for read-once inputs

@@ -307,9 +307,7 @@ int launch(const BArgs &a, cudaStream_t stream) {
     auto kern = cells == 100 ? builder_kernel<BUILDER_T, IS_RESET, 100> : builder_kernel<BUILDER_T, IS_RESET, 0>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
-    e = launch_pdl(kern, dim3((unsigned)((a.n + BUILDER_T - 1) / BUILDER_T)), dim3(BUILDER_T), smem, stream, a);
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    return (int)e;
+    return (int)launch_pdl(kern, dim3((unsigned)((a.n + BUILDER_T - 1) / BUILDER_T)), dim3(BUILDER_T), smem, stream, a);
 }
 
 int check(const beng_builder_params *p, const beng_builder_state *st, const beng_builder_io *io, int64_t n) {
@@ -359,16 +357,12 @@ int beng_builder_step_host(const beng_builder_params *p, const beng_builder_stat
     cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, n * sizeof(int64_t), cudaMemcpyHostToDevice, s);
     if (e != cudaSuccess) return (int)e;
     if (int rc = beng_builder_step(p, st, actions_dev, io, n_envs, stream)) return rc;
-#define BENG_D2H(dst, src, bytes) \
-    if (dst) { e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s); if (e != cudaSuccess) return (int)e; }
-    BENG_D2H(reward_host, io->reward, n * sizeof(float))
-    BENG_D2H(terminated_host, io->terminated, n)
-    BENG_D2H(resources_host, io->resources, n * 4 * sizeof(float))
-    BENG_D2H(capacity_host, io->capacity, n * sizeof(float))
-    BENG_D2H(win_steps_host, io->win_steps, n * sizeof(int32_t))
-    BENG_D2H(grid_host, io->grid, n * cells)
-#undef BENG_D2H
-    return 0;
+    if (int rc = beng::d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
+    if (int rc = beng::d2h(terminated_host, io->terminated, n, s)) return rc;
+    if (int rc = beng::d2h(resources_host, io->resources, n * 4 * sizeof(float), s)) return rc;
+    if (int rc = beng::d2h(capacity_host, io->capacity, n * sizeof(float), s)) return rc;
+    if (int rc = beng::d2h(win_steps_host, io->win_steps, n * sizeof(int32_t), s)) return rc;
+    return beng::d2h(grid_host, io->grid, n * cells, s);
 }
 
 }  // extern "C"

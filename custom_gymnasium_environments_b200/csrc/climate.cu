@@ -10,7 +10,6 @@
 // choice(4 values, p) as an inverse-CDF lookup (numpy Generator.choice's own rule; the cdf tables are the float64
 // values numpy computes, see oracle/c/climate_oracle.c).  HBM-bound on paper (~160 B per env-step).
 #include <cstdint>
-#include <cstdlib>
 
 #include "beng_common.cuh"
 #include "beng_rng.cuh"
@@ -193,8 +192,11 @@ __device__ __forceinline__ void step_env(const KArgs &a, long long env, const KI
     }
 }
 
-template <int T, bool IS_RESET>
-__global__ void __launch_bounds__(T, 8) climate_kernel(const KArgs a) {
+constexpr int CLIMATE_T = 128;
+
+// Reset kernel: one tile of CLIMATE_T envs per CTA.
+__global__ void __launch_bounds__(CLIMATE_T, 8) climate_kernel(const KArgs a) {
+    constexpr int T = CLIMATE_T;
     __shared__ __align__(128) float tile[T * KOBS];
     const int tid = threadIdx.x;
     const long long n = a.n;
@@ -206,8 +208,8 @@ __global__ void __launch_bounds__(T, 8) climate_kernel(const KArgs a) {
     bool ended = false;
     double st_ret = 0.0, st_len = 0.0;
     if (env < n) {
-        const KIn in = load_env<IS_RESET>(a, env);
-        step_env<IS_RESET>(a, env, in, tile + tid * KOBS, ended, st_ret, st_len);
+        const KIn in = load_env<true>(a, env);
+        step_env<true>(a, env, in, tile + tid * KOBS, ended, st_ret, st_len);
     }
 
     fence_proxy_async_smem();
@@ -220,33 +222,20 @@ __global__ void __launch_bounds__(T, 8) climate_kernel(const KArgs a) {
         bulk_commit();
         for (uint32_t i = bulk / 4; i < bytes / 4; ++i) a.io.obs[first * KOBS + i] = tile[i];  // ragged last tile
     }
-    if constexpr (!IS_RESET) {
-        if (a.io.stats) {
-            const unsigned done_mask = __ballot_sync(0xFFFFFFFFu, ended);
-            if (done_mask) {
-                double r = st_ret, l = st_len;
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) {
-                    r += __shfl_xor_sync(0xFFFFFFFFu, r, o);
-                    l += __shfl_xor_sync(0xFFFFFFFFu, l, o);
-                }
-                if ((tid & 31) == 0) {
-                    atomicAdd(&a.io.stats[0], (double)__popc(done_mask));
-                    atomicAdd(&a.io.stats[1], r);
-                    atomicAdd(&a.io.stats[2], l);
-                }
-            }
-        }
-    }
     if (tid == 0) bulk_wait_read<0>();
 }
 
-// Step kernel, persistent form: a CTA walks the tiles blockIdx.x, blockIdx.x + gridDim.x, ... and requests the NEXT
+// Step kernel: a persistent CTA walks the tiles blockIdx.x, blockIdx.x + gridDim.x, ... and requests the NEXT
 // tile's state and action words before it computes the current one, so that the memory round trip of a tile (40 % of
 // the one-tile kernel's stall samples) runs under the float64 arithmetic of the previous one.  Three observation
 // buffers: the bulk copy of tile k is only awaited before tile k+2 is drained, one CTA barrier per tile.
-template <int T, int MINB>
-__global__ void __launch_bounds__(T, MINB) climate_step_persistent_kernel(const KArgs a) {
+// 5 CTAs of 128 threads per SM (94 registers, no spills).  Same-box A/B at 1,048,576 envs, L2 flushed, us per step: the
+// one-tile kernel 47.1; persistent (CTAs per SM x threads) 5 x 128 **41.1**, 10 x 64 41.2, 4 x 128 42.8, 3 x 192 43.3,
+// 2 x 256 44.6; shapes that need a register cap below 94 spill and are slower than the one-tile kernel (6 x 128 at 80
+// registers 53.8, 8 x 128 at 64 registers 58.4).
+constexpr int CLIMATE_STEP_CTAS_PER_SM = 5;
+__global__ void __launch_bounds__(CLIMATE_T, CLIMATE_STEP_CTAS_PER_SM) climate_step_persistent_kernel(const KArgs a) {
+    constexpr int T = CLIMATE_T;
     __shared__ __align__(128) float tiles[3][T * KOBS];
     const int tid = threadIdx.x;
     const long long n = a.n;
@@ -300,38 +289,16 @@ __global__ void __launch_bounds__(T, MINB) climate_step_persistent_kernel(const 
     if (tid == 0) bulk_wait_read<0>();
 }
 
-constexpr int CLIMATE_T = 128;
-
-template <int T, int MINB>
-int launch_persistent(const KArgs &a, cudaStream_t stream) {
-    const long long n_tiles = (a.n + T - 1) / T;
-    const long long slots = (long long)device_sm_count() * MINB;
-    const unsigned grid = (unsigned)(n_tiles < slots ? n_tiles : slots);
-    cudaError_t e = launch_pdl(climate_step_persistent_kernel<T, MINB>, dim3(grid), dim3(T), 0, stream, a);
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    return (int)e;
+int launch_reset(const KArgs &a, cudaStream_t stream) {
+    const unsigned grid = (unsigned)((a.n + CLIMATE_T - 1) / CLIMATE_T);
+    return (int)launch_pdl(climate_kernel, dim3(grid), dim3(CLIMATE_T), 0, stream, a);
 }
 
-template <bool IS_RESET>
-int launch(const KArgs &a, cudaStream_t stream) {
-    if constexpr (!IS_RESET) {
-        // Default: 5 persistent CTAs of 128 threads per SM (94 registers, no spills).  Same-box A/B at 1,048,576 envs, L2
-        // flushed, us per step: the one-tile kernel 47.1; persistent (CTAs per SM x threads) 5 x 128 **41.1**, 10 x 64
-        // 41.2, 4 x 128 42.8, 3 x 192 43.3, 2 x 256 44.6; shapes that need a register cap below 94 spill and are slower
-        // than the one-tile kernel (6 x 128 at 80 registers 53.8, 8 x 128 at 64 registers 58.4).
-        // BENG_CLIMATE_CFG = "tile" | "p4" | "p10" selects the others (A/B runs, profiles/cfg_probe.py).
-        if (const char *cfg = getenv("BENG_CLIMATE_CFG")) {
-            if (cfg[0] == 'p' && atoi(cfg + 1) == 4) return launch_persistent<128, 4>(a, stream);
-            if (cfg[0] == 'p' && atoi(cfg + 1) == 10) return launch_persistent<64, 10>(a, stream);
-            if (cfg[0] != 't') return BENG_ERR_BAD_ARG;
-        } else {
-            return launch_persistent<128, 5>(a, stream);
-        }
-    }
-    const unsigned grid = (unsigned)((a.n + CLIMATE_T - 1) / CLIMATE_T);
-    cudaError_t e = launch_pdl(climate_kernel<CLIMATE_T, IS_RESET>, dim3(grid), dim3(CLIMATE_T), 0, stream, a);
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    return (int)e;
+int launch_step(const KArgs &a, cudaStream_t stream) {
+    const long long n_tiles = (a.n + CLIMATE_T - 1) / CLIMATE_T;
+    const long long slots = (long long)device_sm_count() * CLIMATE_STEP_CTAS_PER_SM;
+    const unsigned grid = (unsigned)(n_tiles < slots ? n_tiles : slots);
+    return (int)launch_pdl(climate_step_persistent_kernel, dim3(grid), dim3(CLIMATE_T), 0, stream, a);
 }
 
 int check(const beng_climate_params *p, const beng_climate_state *st, const beng_climate_io *io, int64_t n) {
@@ -353,7 +320,7 @@ int beng_climate_reset(const beng_climate_params *p, const beng_climate_state *s
     if (int rc = beng::check(p, st, io, n_envs)) return rc;
     if (n_envs == 0) return 0;
     beng::KArgs a{*p, *st, *io, nullptr, nullptr, mask_dev, (long long)n_envs, first_call};
-    return beng::launch<true>(a, (cudaStream_t)stream);
+    return beng::launch_reset(a, (cudaStream_t)stream);
 }
 
 int beng_climate_step(const beng_climate_params *p, const beng_climate_state *st, const float *ac_temp_dev,
@@ -363,7 +330,7 @@ int beng_climate_step(const beng_climate_params *p, const beng_climate_state *st
     if (((uintptr_t)lights_dev & 3) || ((uintptr_t)ac_temp_dev & 3)) return BENG_ERR_BAD_ARG;  // lights are read as one uint32 per env
     if (n_envs == 0) return 0;
     beng::KArgs a{*p, *st, *io, ac_temp_dev, lights_dev, nullptr, (long long)n_envs, 0};
-    return beng::launch<false>(a, (cudaStream_t)stream);
+    return beng::launch_step(a, (cudaStream_t)stream);
 }
 
 int beng_climate_step_host(const beng_climate_params *p, const beng_climate_state *st, float *ac_temp_dev,
@@ -381,14 +348,10 @@ int beng_climate_step_host(const beng_climate_params *p, const beng_climate_stat
     e = cudaMemcpyAsync(lights_dev, lights_host, n * 4, cudaMemcpyHostToDevice, s);
     if (e != cudaSuccess) return (int)e;
     if (int rc = beng_climate_step(p, st, ac_temp_dev, lights_dev, io, n_envs, stream)) return rc;
-#define BENG_D2H(dst, src, bytes) \
-    if (dst) { e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s); if (e != cudaSuccess) return (int)e; }
-    BENG_D2H(reward_host, io->reward, n * sizeof(float))
-    BENG_D2H(terminated_host, io->terminated, n)
-    BENG_D2H(truncated_host, io->truncated, n)
-    BENG_D2H(obs_host, io->obs, n * BENG_CLIMATE_OBS_DIM * sizeof(float))
-#undef BENG_D2H
-    return 0;
+    if (int rc = beng::d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
+    if (int rc = beng::d2h(terminated_host, io->terminated, n, s)) return rc;
+    if (int rc = beng::d2h(truncated_host, io->truncated, n, s)) return rc;
+    return beng::d2h(obs_host, io->obs, n * BENG_CLIMATE_OBS_DIM * sizeof(float), s);
 }
 
 }  // extern "C"

@@ -28,8 +28,6 @@
 
 #include <cfloat>
 #include <cstdint>
-#include <cstdio>
-#include <cstdlib>
 
 #include "beng_common.cuh"
 #include "beng_rng.cuh"
@@ -357,33 +355,31 @@ __device__ __forceinline__ double warp_sum(double v) {
 // price walk, psychology, reward).  What does not: the 11 indicator features, float32 outputs checked at rtol 1e-5 /
 // atol 1e-6 (tests/test_crypto_gpu.py); their error against the oracle is ~1e-7.
 //
-// The window comes in through the TMA: a ring of two 38.4 KB shared-memory stages filled by cp.async.bulk.tensor (one
-// [50 slots][32 envs] box of the close tensor and one of the open/high/low/volume tensor per unit, completion on an
-// mbarrier), so the next unit's window is in flight whatever the threads are doing.  What a box fetched early cannot contain is
-// handled explicitly: the newest candle (written by the dynamics after the box may have been read) comes from shared
-// memory, and a unit in which some env reset in this call (its whole window was rewritten) is re-read with ordinary loads.
+// In the step, the window comes in through the TMA: a ring of two 38.4 KB shared-memory stages filled by
+// cp.async.bulk.tensor (one [50 slots][32 envs] box of the close tensor and one of the open/high/low/volume tensor per
+// unit, completion on an mbarrier), so the next unit's window is in flight whatever the threads are doing.  What a box
+// fetched early cannot contain is handled explicitly: the newest candle (written by the dynamics after the box may have
+// been read) comes from shared memory, and a unit in which some env reset in this call (its whole window was rewritten)
+// is re-read with ordinary loads.
 //
-// Two kernels share these stages:
+// Two kernels run these stages:
 //   crypto5_kernel (the step)  warp-specialised, 768 threads, one CTA per SM: 16 OBSERVATION warps (64 registers after
 //       setmaxnreg.dec) and 8 DYNAMICS warps (112 registers after setmaxnreg.inc) that run up to 16 units ahead; a
 //       dynamics warp hands its unit over through a slot of a 16-deep shared-memory ring (mbarriers ready[]/freed[]).
 //       The ~13,000-cycle dependency chain of a unit's dynamics therefore never sits on the observation path
 //       (in the bulk-synchronous kernel it was 29 % of the step, profiles/crypto_step_r2_ncu_summary.txt).
-//   crypto4_kernel (reset(), and BENG_CRYPTO_VARIANT=4 for A/B)  bulk-synchronous, 512 threads: rounds of 16 units,
-//       all warps run the dynamics of the round, then the observation stage of its units one after the other.
+//   crypto4_kernel (reset())  bulk-synchronous, 512 threads: rounds of 16 units, all warps run the dynamics of the
+//       round, then the observation stage of its units one after the other.  Every window is rewritten in this
+//       launch, so it reads them back with ordinary loads: nothing to prefetch through the TMA or to run ahead of.
+//       (Run as the step kernel it measures ~8 % slower than crypto5_kernel, DESIGN.md section 7.)
 constexpr int C3_SUB = 32;      // envs per unit
 constexpr int C3_RNGW = 20;     // Philox words per env-step: <= 3 (block offset) + 2 (slippage) + 2 + 2 + 3 + 4 + 2 + 2
 constexpr int C3_LAST = 20;     // closes kept for Bollinger / RSI
 constexpr int C3_COOP_MAX = 8;  // resets per warp up to which each one is rebuilt by the whole warp
 constexpr int C3_TILE_BYTES = C3_SUB * OBS * (int)sizeof(float);
 static_assert(C3_TILE_BYTES % 128 == 0, "tile buffers stay 128-byte aligned");
-#ifndef BENG_TMA_STAGES
-#define BENG_TMA_STAGES 2  /* measured: 2 stages = 3 stages (133 vs 136 us); the third one buys nothing */
-#endif
-#ifndef BENG_C5_RING
-#define BENG_C5_RING 16  /* measured: 8 slots 133-144 us, 16 slots 126-133 us (the dynamics warps run further ahead) */
-#endif
-constexpr int OBS_WARPS = 16, OBS_T = OBS_WARPS * 32, OBS_PER = (HIST + OBS_WARPS - 1) / OBS_WARPS, TMA_STAGES = BENG_TMA_STAGES;
+constexpr int TMA_STAGES = 2;  // measured: 2 stages = 3 stages (133 vs 136 us); the third one buys nothing
+constexpr int OBS_WARPS = 16, OBS_T = OBS_WARPS * 32, OBS_PER = (HIST + OBS_WARPS - 1) / OBS_WARPS;
 constexpr int STAGE_O = HIST * C3_SUB * 16, STAGE_C = HIST * C3_SUB * 8;  // bytes per stage: 25600 + 12800
 
 struct MacdWeights {
@@ -868,29 +864,23 @@ __device__ __forceinline__ void issue_window_loads(uint8_t *smem_raw, int stage,
 constexpr size_t C4_OFF_CUR = OFF_COMMON_END;                        // double [512]
 constexpr size_t C4_OFF_NEWX = C4_OFF_CUR + (size_t)OBS_T * 8;       // float4 [512]
 constexpr size_t C4_OFF_PORT = C4_OFF_NEWX + (size_t)OBS_T * 16;     // float4 [512]
-constexpr size_t C4_OFF_URESET = C4_OFF_PORT + (size_t)OBS_T * 16;   // uint32 [16]
-constexpr size_t C4_SMEM_BYTES = C4_OFF_URESET + OBS_WARPS * 4;
+constexpr size_t C4_SMEM_BYTES = C4_OFF_PORT + (size_t)OBS_T * 16;
 static_assert(C4_SMEM_BYTES <= 227 * 1024, "one CTA per SM: everything has to fit in 227 KB");
 static_assert((size_t)C3_RNGW * OBS_T * 4 <= 2 * (size_t)C3_TILE_BYTES, "the Philox table aliases the two tile buffers");
 
-template <bool IS_RESET>
-__global__ void __launch_bounds__(OBS_T, 1) crypto4_kernel(const CArgs a, const __grid_constant__ CUtensorMap tm_close,
-                                                           const __grid_constant__ CUtensorMap tm_ohlv) {
-    constexpr bool USE_TMA = !IS_RESET;  // reset(): every window is rewritten in this launch, nothing to prefetch
+__global__ void __launch_bounds__(OBS_T, 1) crypto4_kernel(const CArgs a) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     float *tiles = reinterpret_cast<float *>(smem_raw);                        // [2][32][261]
     uint32_t *s_rng = reinterpret_cast<uint32_t *>(smem_raw);                  // [20][512], dynamics phase only
     double *s_cur = reinterpret_cast<double *>(smem_raw + C4_OFF_CUR);
     float4 *s_newx = reinterpret_cast<float4 *>(smem_raw + C4_OFF_NEWX);
     float4 *s_port = reinterpret_cast<float4 *>(smem_raw + C4_OFF_PORT);
-    uint32_t *s_ureset = reinterpret_cast<uint32_t *>(smem_raw + C4_OFF_URESET);
-    const uint32_t mbar0 = smem_u32(smem_raw + OFF_MBAR);
 
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const long long n = a.n;
     const long long n_units = (n + C3_SUB - 1) / C3_SUB;
     const uint32_t pitch32 = (uint32_t)a.pitch;
-    const int head = IS_RESET ? a.p.window_head : (a.p.window_head + 1 == HIST ? 0 : a.p.window_head + 1);
+    const int head = a.p.window_head;
     const int oldest = head + 1 == HIST ? 0 : head + 1;
     const double inv_ib = 1.0 / a.p.initial_balance;  // (features divide by it; the product differs by <= 1 ulp of float64)
     // units of this CTA: u(q) = blockIdx.x + gridDim.x * q, q = 0 .. total-1
@@ -903,23 +893,9 @@ __global__ void __launch_bounds__(OBS_T, 1) crypto4_kernel(const CArgs a, const 
         const int slot = oldest + wid + OBS_WARPS * i;
         slot_of[i] = slot >= HIST ? slot - HIST : slot;
     }
-    if constexpr (USE_TMA) {
-        if (tid == 0) {
-#pragma unroll
-            for (int s = 0; s < TMA_STAGES; ++s) mbar_init(mbar0 + 8u * s, 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            fence_proxy_async_smem();
-        }
-    }
     pdl_launch_dependents();  // the next step's grid may become resident as this one drains ...
     pdl_wait();               // ... and this one touches nothing before the previous step's grid has flushed
     __syncthreads();
-    if constexpr (USE_TMA) {
-        if (tid == 0) {
-            for (long long q = 0; q < TMA_STAGES && q < total; ++q)
-                issue_window_loads(smem_raw, (int)q, (int)(unit_of(q) * C3_SUB), &tm_close, &tm_ohlv);
-        }
-    }
 
 #pragma unroll 1
     for (long long q0 = 0; q0 < total; q0 += OBS_WARPS) {
@@ -928,7 +904,7 @@ __global__ void __launch_bounds__(OBS_T, 1) crypto4_kernel(const CArgs a, const 
         __syncthreads();
         {
             const long long qw = q0 + wid;
-            const unsigned resets = dynamics_phase<IS_RESET, OBS_T>(
+            dynamics_phase<true, OBS_T>(
                 a, unit_of(qw), qw < total, head, s_rng + tid, reinterpret_cast<double *>(s_rng + wid * C3_SUB), OBS_T / 2,
                 [&](double cur, double cash, double holdings, double psych, float4 newest) {
                     const double hv = holdings * cur;  // portfolio features :519-527, psychology :559
@@ -937,7 +913,6 @@ __global__ void __launch_bounds__(OBS_T, 1) crypto4_kernel(const CArgs a, const 
                     s_port[tid] = make_float4((float)(cash * inv_ib), (float)(hv * inv_ib), (float)((cash + hv) * inv_ib),
                                               (float)psych);
                 });
-            if (lane == 0) s_ureset[wid] = resets;
         }
         __syncthreads();  // orders this CTA's window writes (the new candle, a reset's whole window) before its reads below
 
@@ -948,21 +923,11 @@ __global__ void __launch_bounds__(OBS_T, 1) crypto4_kernel(const CArgs a, const 
             const long long sub_first = unit_of(q) * C3_SUB;
             const long long env = sub_first + lane;
             const int le = sub * C3_SUB + lane;  // where the dynamics left this env's values
-            const int stage = (int)(q % TMA_STAGES);
             float *tile = tiles + (q & 1) * (C3_SUB * OBS);
             float *dst = tile + lane * OBS;
-            const ObsSmem sm = obs_smem(smem_raw, stage);
-            const bool direct = IS_RESET || s_ureset[sub] != 0;  // CTA-uniform
-            if constexpr (USE_TMA) mbar_wait(mbar0 + 8u * stage, (uint32_t)((q / TMA_STAGES) & 1));  // (keeps the phases in step)
-            if (env < n) {
-                if (direct) compose_unit<true>(a, sm, lane, wid, env, slot_of, pitch32, s_cur[le], s_newx[le], dst);
-                else compose_unit<false>(a, sm, lane, wid, env, slot_of, pitch32, s_cur[le], s_newx[le], dst);
-            }
-            __syncthreads();  // the stage has been consumed; partial sums and the last 20 closes are visible
-            if constexpr (USE_TMA) {
-                if (tid == OBS_T - 1 && q + TMA_STAGES < total)  // refill the stage just freed
-                    issue_window_loads(smem_raw, stage, (int)(unit_of(q + TMA_STAGES) * C3_SUB), &tm_close, &tm_ohlv);
-            }
+            const ObsSmem sm = obs_smem(smem_raw, 0);
+            if (env < n) compose_unit<true>(a, sm, lane, wid, env, slot_of, pitch32, s_cur[le], s_newx[le], dst);
+            __syncthreads();  // partial sums and the last 20 closes are visible
             if (env < n && wid < 4) finish_unit(sm, lane, wid, s_port[le], dst);
             fence_proxy_async_smem();
             if (tid == 0) bulk_wait_read<0>();  // the copy issued one unit ago has read the other tile buffer
@@ -974,16 +939,15 @@ __global__ void __launch_bounds__(OBS_T, 1) crypto4_kernel(const CArgs a, const 
 }
 
 // ---- crypto5: warp-specialised -------------------------------------------------------------------------------------
-#ifndef BENG_C5_OBS_REGS
-#define BENG_C5_OBS_REGS 64  /* measured: 64 / 112 is 3 us faster than 72 / 96 */
-#define BENG_C5_DYN_REGS 112
-#endif
 constexpr int DYN_WARPS = 8, C5_T = OBS_T + DYN_WARPS * 32;      // 768 threads = 6 warpgroups (4 observation + 2 dynamics)
 // setmaxnreg moves registers inside the CTA's OWN pool (what it was launched with: 768 threads x 80), it cannot draw on
 // the rest of the register file: 512 * 64 + 256 * 112 = 61440 = 768 * 80.
-constexpr int C5_LAUNCH_REGS = 80, C5_REGS_OBS = BENG_C5_OBS_REGS, C5_REGS_DYN = BENG_C5_DYN_REGS;
+// Measured: 64 / 112 is 3 us faster than 72 / 96.
+constexpr int C5_LAUNCH_REGS = 80, C5_REGS_OBS = 64, C5_REGS_DYN = 112;
 static_assert(OBS_T * C5_REGS_OBS + DYN_WARPS * 32 * C5_REGS_DYN <= C5_T * C5_LAUNCH_REGS, "setmaxnreg budget");
-constexpr int C5_RING = BENG_C5_RING;  // hand-over slots: unit q uses slot q % C5_RING (a multiple of DYN_WARPS)
+// Hand-over slots: unit q uses slot q % C5_RING (a multiple of DYN_WARPS).  Measured: 8 slots 133-144 us, 16 slots
+// 126-133 us (the dynamics warps run further ahead).
+constexpr int C5_RING = 16;
 static_assert(C5_RING % DYN_WARPS == 0 && C5_RING <= 16, "each dynamics warp owns C5_RING / DYN_WARPS slots");
 constexpr size_t C5_OFF_CUR = OFF_COMMON_END;                                 // double [ring][32]
 constexpr size_t C5_OFF_NEWX = C5_OFF_CUR + (size_t)C5_RING * C3_SUB * 8;     // float4 [ring][32]
@@ -1122,46 +1086,26 @@ int make_window_map(CUtensorMap *map, void *base, long long pitch, CUtensorMapDa
     return r == CUDA_SUCCESS ? 0 : BENG_ERR_BAD_ARG;
 }
 
-template <typename Kern>
-int launch_tma(Kern kern, int threads, size_t smem, const CArgs &a, cudaStream_t stream) {
-    CUtensorMap tm_close, tm_ohlv;
-    if (int rc = make_window_map(&tm_close, a.st.close, a.pitch, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 8, 1)) return rc;
-    if (int rc = make_window_map(&tm_ohlv, a.st.ohlv, a.pitch, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, 4)) return rc;
+// One persistent CTA per SM (at most one per unit) of `threads` threads and `smem` bytes of dynamic shared memory.
+template <typename Kern, typename... Extra>
+int launch_persistent(Kern kern, int threads, size_t smem, const CArgs &a, cudaStream_t stream, const Extra &...extra) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     const long long n_units = (a.n + C3_SUB - 1) / C3_SUB;
-    long long grid = device_sm_count();  // one persistent CTA per SM
+    long long grid = device_sm_count();
     if (grid > n_units) grid = n_units;
-    static const bool use_pdl = getenv("BENG_NO_PDL") == nullptr;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3((unsigned)threads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = use_pdl ? 1 : 0;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    e = cudaLaunchKernelEx(&cfg, kern, a, tm_close, tm_ohlv);
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    return (int)e;
+    return (int)launch_pdl(kern, dim3((unsigned)grid), dim3((unsigned)threads), smem, stream, a, extra...);
 }
 
-template <bool IS_RESET>
-int launch(const CArgs &a, cudaStream_t stream) {
-    // reset(): the bulk-synchronous kernel (every window is rewritten, nothing to prefetch or to run ahead of).
-    // step(): the warp-specialised kernel; BENG_CRYPTO_VARIANT=4 (read once) selects the bulk-synchronous one for A/Bs.
-    if constexpr (IS_RESET) {
-        return launch_tma(crypto4_kernel<true>, OBS_T, C4_SMEM_BYTES, a, stream);
-    } else {
-        static const int variant = [] {
-            const char *v = getenv("BENG_CRYPTO_VARIANT");
-            return v ? atoi(v) : 5;
-        }();
-        if (variant == 4) return launch_tma(crypto4_kernel<false>, OBS_T, C4_SMEM_BYTES, a, stream);
-        return launch_tma(crypto5_kernel, C5_T, C5_SMEM_BYTES, a, stream);
-    }
+int launch_reset(const CArgs &a, cudaStream_t stream) {
+    return launch_persistent(crypto4_kernel, OBS_T, C4_SMEM_BYTES, a, stream);
+}
+
+int launch_step(const CArgs &a, cudaStream_t stream) {
+    CUtensorMap tm_close, tm_ohlv;
+    if (int rc = make_window_map(&tm_close, a.st.close, a.pitch, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 8, 1)) return rc;
+    if (int rc = make_window_map(&tm_ohlv, a.st.ohlv, a.pitch, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, 4)) return rc;
+    return launch_persistent(crypto5_kernel, C5_T, C5_SMEM_BYTES, a, stream, tm_close, tm_ohlv);
 }
 
 int check(const beng_crypto_params *p, const beng_crypto_state *st, const beng_crypto_io *io, int64_t n) {
@@ -1187,7 +1131,7 @@ int beng_crypto_reset(const beng_crypto_params *p, const beng_crypto_state *st, 
     if (int rc = beng::check(p, st, io, n_envs)) return rc;
     if (n_envs == 0) return 0;
     beng::CArgs a{*p, *st, *io, nullptr, mask_dev, (long long)n_envs, beng_crypto_window_pitch(n_envs), first_call};
-    return beng::launch<true>(a, (cudaStream_t)stream);
+    return beng::launch_reset(a, (cudaStream_t)stream);
 }
 
 int beng_crypto_step(const beng_crypto_params *p, const beng_crypto_state *st, const void *actions_dev,
@@ -1197,7 +1141,7 @@ int beng_crypto_step(const beng_crypto_params *p, const beng_crypto_state *st, c
     if ((uintptr_t)actions_dev & 7) return BENG_ERR_BAD_ARG;  // 64-bit action loads (int64, or float32 pairs)
     if (n_envs == 0) return 0;
     beng::CArgs a{*p, *st, *io, actions_dev, nullptr, (long long)n_envs, beng_crypto_window_pitch(n_envs), 0};
-    return beng::launch<false>(a, (cudaStream_t)stream);
+    return beng::launch_step(a, (cudaStream_t)stream);
 }
 
 int beng_crypto_step_host(const beng_crypto_params *p, const beng_crypto_state *st, void *actions_dev,
@@ -1213,14 +1157,10 @@ int beng_crypto_step_host(const beng_crypto_params *p, const beng_crypto_state *
     cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, abytes, cudaMemcpyHostToDevice, s);
     if (e != cudaSuccess) return (int)e;
     if (int rc = beng_crypto_step(p, st, actions_dev, io, n_envs, stream)) return rc;
-#define BENG_D2H(dst, src, bytes) \
-    if (dst) { e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s); if (e != cudaSuccess) return (int)e; }
-    BENG_D2H(reward_host, io->reward, n * sizeof(float))
-    BENG_D2H(terminated_host, io->terminated, n)
-    BENG_D2H(truncated_host, io->truncated, n)
-    BENG_D2H(obs_host, io->obs, n * BENG_CRYPTO_OBS_DIM * sizeof(float))
-#undef BENG_D2H
-    return 0;
+    if (int rc = beng::d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
+    if (int rc = beng::d2h(terminated_host, io->terminated, n, s)) return rc;
+    if (int rc = beng::d2h(truncated_host, io->truncated, n, s)) return rc;
+    return beng::d2h(obs_host, io->obs, n * BENG_CRYPTO_OBS_DIM * sizeof(float), s);
 }
 
 }  // extern "C"

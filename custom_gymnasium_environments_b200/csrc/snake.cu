@@ -14,8 +14,8 @@
 //     global memory, so the tile is composed in shared memory (zero fill, scatter body cells, food
 //     last) and drained with ONE bulk asynchronous copy (cp.async.bulk shared->global, the TMA
 //     engine, SASS UBLKCP) issued by a single thread -- no per-thread obs stores at all;
-//   * CTAs are persistent over tiles with a STAGES-deep ring of tile buffers, so the copy engine
-//     drains tile k while the threads compose tile k+1;
+//   * CTAs are persistent over tiles with one tile buffer each; several CTAs per SM keep the copy
+//     engine draining one CTA's tile while the others compose theirs;
 //   * the shared-memory tile doubles as the O(1) occupancy map for self-collision and for the
 //     food rejection loop (the reference scans a Python list for both);
 //   * finished episodes are counted with warp votes, accumulated per CTA in shared memory and
@@ -26,8 +26,6 @@
 // write); there is nothing GEMM-shaped here and no tensor-core path is wanted.
 #include <climits>
 #include <cstdint>
-#include <cstdio>
-#include <cstdlib>
 
 #include "beng_common.cuh"
 #include "beng_rng.cuh"
@@ -176,9 +174,9 @@ __device__ __forceinline__ Loaded load_inputs(const Args &a, long long env) {
 // OWNROW: every thread zero-fills its own env row with 16-byte stores (needs G*G % 16 == 0, and is
 // bank-conflict free when G*G/16 is odd, e.g. G = 20: consecutive rows are 25 x 16 B apart so eight
 // threads cover all 32 banks).  Otherwise the tile is zero-filled cooperatively + one more barrier.
-template <int T, int STAGES, bool IS_RESET, bool OWNROW>
+template <int T, bool IS_RESET, bool OWNROW>
 __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
-    extern __shared__ __align__(128) uint8_t smem[];
+    extern __shared__ __align__(128) uint8_t buf[];  // the tile: T x G*G observation bytes
     __shared__ int s_stats[5];  // per-CTA, per-launch: n_episodes, sum_return, sum_length, sum_score, max_score
 
     const int tid = threadIdx.x;
@@ -211,7 +209,6 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
     }
     int it = 0;
     for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
-        uint8_t *buf = smem + (size_t)(it % STAGES) * tile_bytes;
         const long long env = tile * T + tid;
         const bool active = env < a.n_envs;
 
@@ -228,9 +225,9 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
             }
         }
 
-        // The bulk copy that last used this buffer (tile it - STAGES) must have finished reading it.
-        if (it >= STAGES) {
-            if (tid == 0) bulk_wait_read<STAGES - 1>();
+        // The bulk copy of the previous tile must have finished reading the buffer.
+        if (it > 0) {
+            if (tid == 0) bulk_wait_read<0>();
             __syncthreads();
         }
         uint8_t *row = buf + tid * cells;
@@ -463,8 +460,7 @@ __global__ void __launch_bounds__(256) snake_export_kernel(const uint4 *__restri
 
 // ---- launch configuration ---------------------------------------------------------------------
 struct Config {
-    int tile;      // envs (= threads) per CTA tile
-    int stages;    // tile buffers per CTA
+    int tile;  // envs (= threads) per CTA tile
     int ctas_per_sm;
 };
 
@@ -472,20 +468,10 @@ struct Config {
 // >= 2 CTAs resident per SM reaches the same ~11.5 G env-steps/s (the kernel is DRAM-bound), two-stage shapes
 // with fewer CTAs are ~15 % slower.  So: one tile buffer per CTA, as many CTAs per SM as shared memory
 // allows, and the largest tile that still gives every SM >= 2 tiles of work.
-// BENG_SNAKE_CFG="tile,stages,ctas_per_sm" overrides (read once; profiling sweeps).
 Config pick_config(int G, long long n_envs) {
-    static int env_tile = -1, env_stages = 0, env_ctas = 0;
-    if (env_tile < 0) {
-        env_tile = 0;
-        if (const char *e = getenv("BENG_SNAKE_CFG")) {
-            int t = 0, s = 0, c = 0;
-            if (sscanf(e, "%d,%d,%d", &t, &s, &c) == 3) { env_tile = t; env_stages = s; env_ctas = c; }
-        }
-    }
     const long long cells = (long long)G * G;
     const long long budget = 200 * 1024;  // of 227 KB: leaves room for static smem + 1 KB/CTA reservation
-    if (env_tile > 0) return Config{env_tile, env_stages, env_ctas};
-    Config c{256, 1, 2};
+    Config c{256, 2};
     const long long sms = device_sm_count();
     while (c.tile > 32 && (c.tile * cells * 2 > budget || (n_envs + c.tile - 1) / c.tile < 2 * sms)) c.tile >>= 1;
     c.ctas_per_sm = (int)(budget / (c.tile * cells));
@@ -494,32 +480,29 @@ Config pick_config(int G, long long n_envs) {
     return c;
 }
 
-template <int T, int STAGES, bool IS_RESET, bool OWNROW>
+template <int T, bool IS_RESET, bool OWNROW>
 int launch_one(const Args &a, const Config &c, cudaStream_t stream) {
-    const size_t smem = (size_t)T * a.G * a.G * STAGES;
-    auto kern = snake_kernel<T, STAGES, IS_RESET, OWNROW>;
+    const size_t smem = (size_t)T * a.G * a.G;
+    auto kern = snake_kernel<T, IS_RESET, OWNROW>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     const long long n_tiles = (a.n_envs + T - 1) / T;
     long long grid = (long long)device_sm_count() * c.ctas_per_sm;
     if (grid > n_tiles) grid = n_tiles;
-    e = launch_pdl(kern, dim3((unsigned)grid), dim3(T), smem, stream, a);
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    return (int)e;
+    return (int)launch_pdl(kern, dim3((unsigned)grid), dim3(T), smem, stream, a);
 }
 
 template <bool IS_RESET>
 int launch(const Args &a, cudaStream_t stream) {
     const Config c = pick_config(a.G, a.n_envs);
     const int cells = a.G * a.G;
-    const bool ownrow = (cells % 16 == 0) && ((cells / 16) % 2 == 1) && !getenv("BENG_SNAKE_COOPZERO");
-#define BENG_CASE(TT, SS)                                                                   \
-    if (c.tile == TT && c.stages == SS)                                                     \
-        return ownrow ? launch_one<TT, SS, IS_RESET, true>(a, c, stream)                    \
-                      : launch_one<TT, SS, IS_RESET, false>(a, c, stream);
-    BENG_CASE(256, 1) BENG_CASE(256, 2) BENG_CASE(128, 1) BENG_CASE(128, 2) BENG_CASE(128, 3) BENG_CASE(64, 1)
-    BENG_CASE(224, 1) BENG_CASE(192, 1) BENG_CASE(160, 1) BENG_CASE(96, 1)  /* non-power-of-two tiles (round-2 sweep) */
-    BENG_CASE(64, 2) BENG_CASE(64, 3) BENG_CASE(64, 4) BENG_CASE(32, 1) BENG_CASE(32, 2) BENG_CASE(32, 4)
+    const bool ownrow = (cells % 16 == 0) && ((cells / 16) % 2 == 1);
+#define BENG_CASE(TT)                                                                       \
+    case TT:                                                                                \
+        return ownrow ? launch_one<TT, IS_RESET, true>(a, c, stream) : launch_one<TT, IS_RESET, false>(a, c, stream);
+    switch (c.tile) {
+        BENG_CASE(256) BENG_CASE(128) BENG_CASE(64) BENG_CASE(32)
+    }
 #undef BENG_CASE
     return BENG_ERR_UNSUPPORTED;
 }
@@ -558,7 +541,7 @@ int beng_snake_launch_config(int32_t grid_size, int64_t n_envs, int32_t *tile, i
     if (grid_size < 2 || grid_size > 64 || n_envs < 0) return BENG_ERR_BAD_ARG;
     const beng::Config c = beng::pick_config(grid_size, n_envs);
     if (tile) *tile = c.tile;
-    if (stages) *stages = c.stages;
+    if (stages) *stages = 1;
     if (ctas_per_sm) *ctas_per_sm = c.ctas_per_sm;
     return 0;
 }
@@ -604,16 +587,12 @@ int beng_snake_step_host(const beng_snake_params *p, const beng_snake_state *st,
     cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, n * sizeof(int64_t), cudaMemcpyHostToDevice, s);
     if (e != cudaSuccess) return (int)e;
     if (int rc = beng_snake_step(p, st, actions_dev, io, n_envs, stream)) return rc;
-#define BENG_D2H(dst, src, bytes) \
-    if (dst) { e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s); if (e != cudaSuccess) return (int)e; }
-    BENG_D2H(reward_host, io->reward, n * sizeof(float))
-    BENG_D2H(terminated_host, io->terminated, n)
-    BENG_D2H(truncated_host, io->truncated, n)
-    BENG_D2H(score_host, io->score, n * sizeof(int32_t))
-    BENG_D2H(snake_length_host, io->snake_length, n * sizeof(int32_t))
-    BENG_D2H(obs_host, io->obs, n * cells)
-#undef BENG_D2H
-    return 0;
+    if (int rc = beng::d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
+    if (int rc = beng::d2h(terminated_host, io->terminated, n, s)) return rc;
+    if (int rc = beng::d2h(truncated_host, io->truncated, n, s)) return rc;
+    if (int rc = beng::d2h(score_host, io->score, n * sizeof(int32_t), s)) return rc;
+    if (int rc = beng::d2h(snake_length_host, io->snake_length, n * sizeof(int32_t), s)) return rc;
+    return beng::d2h(obs_host, io->obs, n * cells, s);
 }
 
 int beng_snake_export_state(const beng_snake_params *p, const beng_snake_state *st, int64_t n_envs, int32_t *head_r,

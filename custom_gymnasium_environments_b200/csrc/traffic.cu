@@ -22,8 +22,6 @@
 // env-step) and in practice at 1M envs (0.94 of the measured copy bandwidth); at the BASELINE 65,536 envs the grid is
 // two waves of a tile whose serial chain is loads -> lights -> spawn -> queues -> reward, see the kernel comment.
 #include <cstdint>
-#include <cstdio>
-#include <cstdlib>
 
 #include "beng_common.cuh"
 #include "beng_rng.cuh"
@@ -306,9 +304,16 @@ __device__ __forceinline__ double step_reward(int tot_passed, int tot_wait, int 
 // short: its Philox blocks are computed ahead of barrier 1 (CachedStream), the global metrics are warp 0's, the two
 // float64 divisions by NI of the variance are FMA sequences instead of the division subroutine (div_const).
 constexpr int WPI_E = 32;  // envs per CTA
+// The default grid (9 intersections) runs 3 intersections per warp, 4-warp CTAs capped at 72 registers (7 CTAs per SM,
+// the 2048 CTAs of 65,536 envs are 1.98 waves).  Same-box sweeps, us per step at 65,536 / 1,048,576 envs (L2 flushed),
+// (intersections per warp, registers): before the queues were packed (1, 40) 30.4 / 256, (2, 48) 29.7 / 263,
+// (2, 56) 28.3-29.0 / 225-253, (2, 64) 28.1-28.5 / 250-258, (3, 64) 30.7 / 255, (3, 72) 28.2 / 223, (3, 80) 30.3 / 233;
+// with packed queues (2, 56) 28.2 / 220, (2, 64) 28.3 / 229, (3, 56) 28.9 / 230, (3, 64) 27.7 / 234,
+// **(3, 72) 26.3-27.8 / 217**, (5, 80) 30.8 / 292, (5, 96) 31.7 / 285, (9, 128) 36.0 / 372.
+constexpr int TRAFFIC_MAXREG = 72;
 
-template <int NI_T, int IPW, int MAXREG, bool IS_RESET>
-__global__ void __maxnreg__(MAXREG) traffic_step_kernel(const TArgs a) {
+template <int NI_T, int IPW, bool IS_RESET>
+__global__ void __maxnreg__(TRAFFIC_MAXREG) traffic_step_kernel(const TArgs a) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     const int NI = NI_T ? NI_T : a.ni;
     const int NW = (NI + IPW - 1) / IPW;  // intersection warps; warp NW is the env warp
@@ -546,42 +551,22 @@ __global__ void __maxnreg__(MAXREG) traffic_step_kernel(const TArgs a) {
     }
 }
 
-template <int NI_T, int IPW, int MAXREG, bool IS_RESET>
+template <int NI_T, int IPW, bool IS_RESET>
 int launch_shape(const TArgs &a, cudaStream_t stream) {
     const int od = a.ni * 14 + 4, nw = (a.ni + IPW - 1) / IPW;
     const size_t smem = 256 * sizeof(double) + (size_t)WPI_E * od * sizeof(float) +
                         (size_t)(4 * a.ni * WPI_E + WPI_E + SPEC_BLOCKS * 4 * WPI_E + a.ni) * sizeof(int32_t);
     const unsigned grid = (unsigned)((a.n + WPI_E - 1) / WPI_E);
-    auto kern = traffic_step_kernel<NI_T, IPW, MAXREG, IS_RESET>;
+    auto kern = traffic_step_kernel<NI_T, IPW, IS_RESET>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
-    e = launch_pdl(kern, dim3(grid), dim3((nw + 1) * 32), smem, stream, a);
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    return (int)e;
+    return (int)launch_pdl(kern, dim3(grid), dim3((nw + 1) * 32), smem, stream, a);
 }
 
+// The default grid's 9 intersections get their own instantiation; any other count runs one intersection per warp.
 template <bool IS_RESET>
 int launch(const TArgs &a, cudaStream_t stream) {
-    // Default grid (9 intersections): 3 intersections per warp, 4-warp CTAs capped at 72 registers (7 CTAs per SM, the
-    // 2048 CTAs of 65,536 envs are 1.98 waves).  Same-box sweeps, us per step at 65,536 / 1,048,576 envs (L2 flushed),
-    // (intersections per warp, registers): before the queues were packed (1, 40) 30.4 / 256, (2, 48) 29.7 / 263,
-    // (2, 56) 28.3-29.0 / 225-253, (2, 64) 28.1-28.5 / 250-258, (3, 64) 30.7 / 255, (3, 72) 28.2 / 223, (3, 80) 30.3 / 233;
-    // with packed queues (2, 56) 28.2 / 220, (2, 64) 28.3 / 229, (3, 56) 28.9 / 230, (3, 64) 27.7 / 234,
-    // **(3, 72) 26.3-27.8 / 217**, (5, 80) 30.8 / 292, (5, 96) 31.7 / 285, (9, 128) 36.0 / 372.
-    // BENG_TRAFFIC_CFG="ipw,maxreg" selects one of the other instantiated shapes for A/B runs.
-    if (a.ni == 9) {
-        if (const char *cfg = getenv("BENG_TRAFFIC_CFG")) {
-            int ipw = 0, maxreg = 0;
-            if (sscanf(cfg, "%d,%d", &ipw, &maxreg) == 2) {
-                if (ipw == 2 && maxreg == 56) return launch_shape<9, 2, 56, IS_RESET>(a, stream);
-                if (ipw == 2 && maxreg == 64) return launch_shape<9, 2, 64, IS_RESET>(a, stream);
-                if (ipw == 3 && maxreg == 72) return launch_shape<9, 3, 72, IS_RESET>(a, stream);
-            }
-            return BENG_ERR_BAD_ARG;
-        }
-        return launch_shape<9, 3, 72, IS_RESET>(a, stream);
-    }
-    return launch_shape<0, 1, 72, IS_RESET>(a, stream);
+    return a.ni == 9 ? launch_shape<9, 3, IS_RESET>(a, stream) : launch_shape<0, 1, IS_RESET>(a, stream);
 }
 
 int check(const beng_traffic_params *p, const beng_traffic_state *st, const beng_traffic_io *io, int64_t n) {
@@ -652,14 +637,10 @@ int beng_traffic_step_host(const beng_traffic_params *p, const beng_traffic_stat
     cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, n * a.ni * sizeof(int64_t), cudaMemcpyHostToDevice, s);
     if (e != cudaSuccess) return (int)e;
     if (int rc = beng_traffic_step(p, st, actions_dev, io, n_envs, stream)) return rc;
-#define BENG_D2H(dst, src, bytes) \
-    if (dst) { e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s); if (e != cudaSuccess) return (int)e; }
-    BENG_D2H(reward_host, io->reward, n * sizeof(float))
-    BENG_D2H(terminated_host, io->terminated, n)
-    BENG_D2H(truncated_host, io->truncated, n)
-    BENG_D2H(obs_host, io->obs, n * (a.ni * 14 + 4) * sizeof(float))
-#undef BENG_D2H
-    return 0;
+    if (int rc = beng::d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
+    if (int rc = beng::d2h(terminated_host, io->terminated, n, s)) return rc;
+    if (int rc = beng::d2h(truncated_host, io->truncated, n, s)) return rc;
+    return beng::d2h(obs_host, io->obs, n * (a.ni * 14 + 4) * sizeof(float), s);
 }
 
 }  // extern "C"

@@ -7,8 +7,6 @@ Tolerances (BASELINE.json north_star: "float envs must match within a stated rto
       thousands of steps -- the only differences are the last-ulp results of CUDA's log/cos vs glibc's
   integer fields (terminated, step, regime, trade kind, RNG counter): exact
 """
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -17,7 +15,6 @@ from oracle import golden_files
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DEV = "cuda:0"
 RTOL, ATOL = 1e-5, 1e-6
 RTOL64 = 1e-9
@@ -303,38 +300,3 @@ def test_single_env_facade(pkg, cgold):
     env2.reset()
     obs, r, *_ = env2.step(np.array([0.5, -0.2], dtype=np.float32))
     assert obs.shape == (261,) and r < 0
-
-
-_ALT_KERNEL_CHECK = r"""
-import os, sys, numpy as np, torch
-sys.path.insert(0, sys.argv[1])
-import custom_gymnasium_environments_b200 as pkg
-from oracle.c_oracle import CryptoOracle
-n, seed = 3001, 12
-env = pkg.BatchedCryptoTradingEnv(n, None, "discrete", device="cuda:0", seed=seed, max_steps=40)
-orc = CryptoOracle(n, seed=seed, max_steps=40)
-np.testing.assert_allclose(env.reset()[0].cpu().numpy(), orc.reset(), rtol=1e-5, atol=1e-6)
-g = torch.Generator(device="cuda:0").manual_seed(0)
-for t in range(90):   # crosses two auto-resets
-    a = torch.randint(0, 5, (n,), device="cuda:0", generator=g)
-    env.step(a); orc.step(a.cpu().numpy())
-    np.testing.assert_allclose(env.obs.cpu().numpy(), orc.obs, rtol=1e-5, atol=1e-6, err_msg=f"step {t}")
-    np.testing.assert_allclose(env.reward64.cpu().numpy(), orc.reward64, rtol=1e-9, atol=1e-9)
-    assert np.array_equal(env.terminated.cpu().numpy().astype(np.uint8), orc.terminated)
-print("alt kernel ok", os.environ.get("BENG_CRYPTO_VARIANT"))
-"""
-
-
-@pytest.mark.parametrize("envvar", [{"BENG_CRYPTO_VARIANT": "4"}])
-def test_alternative_kernels_match_oracle(envvar, tmp_path):
-    """The bulk-synchronous step kernel (crypto4_kernel: the one reset() always uses) is selected for step() by an
-    environment variable read once per process, so it is exercised in a subprocess."""
-    import subprocess
-    import sys
-
-    script = tmp_path / "alt.py"
-    script.write_text(_ALT_KERNEL_CHECK)
-    res = subprocess.run([sys.executable, str(script), ROOT], capture_output=True, text=True, timeout=600,
-                         env=dict(os.environ, **envvar))
-    assert res.returncode == 0, res.stdout + res.stderr
-    assert "alt kernel ok" in res.stdout
