@@ -107,6 +107,9 @@ SIGNATURES = {
                                   C.c_int64, C.c_void_p]),
     "beng_snake_step_host": (C.c_int, [C.POINTER(SnakeParams), C.POINTER(SnakeState), C.c_void_p, C.POINTER(SnakeIO),
                                        C.c_int64] + [C.c_void_p] * 8),
+    "beng_snake_step_host_delta": (C.c_int, [C.POINTER(SnakeParams), C.POINTER(SnakeState), C.c_void_p,
+                                             C.POINTER(SnakeIO), C.c_int64] + [C.c_void_p] * 9),
+    "beng_snake_apply_obs_delta": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32]),
     "beng_crypto_window_pitch": (C.c_int64, [C.c_int64]),
     "beng_crypto_reset": (C.c_int, [C.POINTER(CryptoParams), C.POINTER(CryptoState), C.POINTER(CryptoIO), C.c_void_p,
                                     C.c_int64, C.c_int32, C.c_void_p]),

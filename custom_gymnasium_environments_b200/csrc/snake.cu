@@ -26,6 +26,9 @@
 // write); there is nothing GEMM-shaped here and no tensor-core path is wanted.
 #include <climits>
 #include <cstdint>
+#include <cstring>
+#include <thread>
+#include <vector>
 
 #include "beng_common.cuh"
 #include "beng_rng.cuh"
@@ -78,6 +81,7 @@ struct Args {
     long long n_envs;
     uint64_t seed, env_id_base;
     int G, max_steps, mode, first_call, tl_trunc;
+    uint32_t *delta;  // DELTA step only: one BENG_OBS_DELTA record per env
 };
 
 // _place_food (snake_env.py:121-129): draw (row, col) until the cell is not part of the snake.
@@ -137,6 +141,16 @@ __device__ __forceinline__ int scan_body(const Core &s, const uint16_t *ring, ui
     return tail;
 }
 
+// Observation change records (include/beng.h, BENG_OBS_DELTA_*), built from the state record alone.
+__device__ __forceinline__ uint32_t delta_pair(int cell, int value) { return (uint32_t)cell | ((uint32_t)value << 12); }
+__device__ __forceinline__ uint32_t food_pair(const Core &s, int G) {
+    return s.food_r == FOOD_NONE ? BENG_OBS_DELTA_UNUSED : delta_pair(s.food_r * G + s.food_c, 2);
+}
+// After reset_env: the row was cleared, then the head and the food were written.
+__device__ __forceinline__ uint32_t reset_record(const Core &s, int G) {
+    return BENG_OBS_DELTA_CLEAR | delta_pair(s.head_r * G + s.head_c, 1) | (food_pair(s, G) << 14);
+}
+
 // Index of the tail entry in the ring (valid for length >= 2).
 __device__ __forceinline__ int tail_index(const Core &s, int cells) {
     const int idx = s.ring_head - (s.length - 1);
@@ -174,7 +188,10 @@ __device__ __forceinline__ Loaded load_inputs(const Args &a, long long env) {
 // OWNROW: every thread zero-fills its own env row with 16-byte stores (needs G*G % 16 == 0, and is
 // bank-conflict free when G*G/16 is odd, e.g. G = 20: consecutive rows are 25 x 16 B apart so eight
 // threads cover all 32 banks).  Otherwise the tile is zero-filled cooperatively + one more barrier.
-template <int T, bool IS_RESET, bool OWNROW>
+// DELTA (step only): also store one change record per env to a.delta, describing how this step's
+// observation row differs from the previous one.  It is assembled from the dynamics' registers (the
+// cells a move, a meal or a reset wrote), never by reading the row back.
+template <int T, bool IS_RESET, bool OWNROW, bool DELTA>
 __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
     extern __shared__ __align__(128) uint8_t buf[];  // the tile: T x G*G observation bytes
     __shared__ int s_stats[5];  // per-CTA, per-launch: n_episodes, sum_return, sum_length, sum_score, max_score
@@ -246,6 +263,7 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
         float rew = 0.0f;
         int term = 0, trunc = 0;
         bool invalid = false;
+        uint32_t rec = BENG_OBS_DELTA_NONE;  // DELTA: death and invalid actions change no cell
         Core s = unpack(cur.raw);
         if (active) {
             uint16_t *ring = a.ring + env * cells;
@@ -261,6 +279,7 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
                 const long long act = cur.act;
                 if (a.mode == BENG_AUTORESET_NEXT_STEP && (s.flags & FLAG_NEEDS_RESET)) {
                     reset_env(s, rng, row, G);  // action ignored, reward 0, not terminated
+                    if constexpr (DELTA) rec = reset_record(s, G);
                 } else if (act < 0 || act > 3) {
                     // The reference raises ValueError (snake_env.py:69-70); here the env is left
                     // untouched and the event is counted for the host to raise on.
@@ -312,6 +331,10 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
                         } else {
                             row[tail_cell] = 0;  // pop(), :107
                         }
+                        // (new_cell != tail_cell: moving into the tail is a self-hit, so the two pairs never collide)
+                        if constexpr (DELTA)
+                            rec = eat ? delta_pair(new_cell, 1) | (food_pair(s, G) << 14)
+                                      : delta_pair(tail_cell, 0) | (delta_pair(new_cell, 1) << 14);
                         s.steps = min(s.steps + 1, 65535);     // :109
                         if (s.steps >= a.max_steps) {
                             term = 1;              // :112-114, reported as terminated
@@ -332,6 +355,7 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
                                 else scan_body(s, ring, row, cells, G, 0, -1, hit);
                             }
                             reset_env(s, rng, row, G);
+                            if constexpr (DELTA) rec = reset_record(s, G);
                         } else {
                             s.flags |= FLAG_NEEDS_RESET;
                         }
@@ -360,6 +384,7 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
             a.core[env] = pack(s);
             if constexpr (!IS_RESET) {
                 a.io.reward[env] = rew;
+                if constexpr (DELTA) a.delta[env] = rec;
                 a.io.terminated[env] = (uint8_t)term;
                 if (a.io.truncated) a.io.truncated[env] = (uint8_t)trunc;  // raw class: never truncates, :119
                 if (invalid && a.io.invalid_count) atomicAdd(a.io.invalid_count, 1);
@@ -480,10 +505,10 @@ Config pick_config(int G, long long n_envs) {
     return c;
 }
 
-template <int T, bool IS_RESET, bool OWNROW>
+template <int T, bool IS_RESET, bool OWNROW, bool DELTA>
 int launch_one(const Args &a, const Config &c, cudaStream_t stream) {
     const size_t smem = (size_t)T * a.G * a.G;
-    auto kern = snake_kernel<T, IS_RESET, OWNROW>;
+    auto kern = snake_kernel<T, IS_RESET, OWNROW, DELTA>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     const long long n_tiles = (a.n_envs + T - 1) / T;
@@ -492,14 +517,15 @@ int launch_one(const Args &a, const Config &c, cudaStream_t stream) {
     return (int)launch_pdl(kern, dim3((unsigned)grid), dim3(T), smem, stream, a);
 }
 
-template <bool IS_RESET>
+template <bool IS_RESET, bool DELTA = false>
 int launch(const Args &a, cudaStream_t stream) {
     const Config c = pick_config(a.G, a.n_envs);
     const int cells = a.G * a.G;
     const bool ownrow = (cells % 16 == 0) && ((cells / 16) % 2 == 1);
 #define BENG_CASE(TT)                                                                       \
     case TT:                                                                                \
-        return ownrow ? launch_one<TT, IS_RESET, true>(a, c, stream) : launch_one<TT, IS_RESET, false>(a, c, stream);
+        return ownrow ? launch_one<TT, IS_RESET, true, DELTA>(a, c, stream)                \
+                      : launch_one<TT, IS_RESET, false, DELTA>(a, c, stream);
     switch (c.tile) {
         BENG_CASE(256) BENG_CASE(128) BENG_CASE(64) BENG_CASE(32)
     }
@@ -530,6 +556,40 @@ Args make_args(const beng_snake_params *p, const beng_snake_state *st, const ben
     a.mode = p->autoreset_mode;
     a.tl_trunc = p->time_limit_truncation;
     return a;
+}
+
+// beng_snake_step without its public name: `delta` non-null selects the DELTA kernel.
+int step(const beng_snake_params *p, const beng_snake_state *st, const int64_t *actions_dev, const beng_snake_io *io,
+         int64_t n_envs, uint32_t *delta, cudaStream_t stream) {
+    if (int rc = check_common(p, st, io, n_envs)) return rc;
+    if (!actions_dev || !io->reward || !io->terminated) return BENG_ERR_BAD_ARG;
+    if ((uintptr_t)actions_dev & 7) return BENG_ERR_BAD_ARG;  // 64-bit action loads (int64, or float32 pairs)
+    if (n_envs == 0) return 0;
+    Args a = make_args(p, st, io, n_envs);
+    a.actions = (const long long *)actions_dev;
+    if (delta) {
+        a.delta = delta;
+        return launch<false, true>(a, stream);
+    }
+    return launch<false>(a, stream);
+}
+
+// Applies the records of envs [begin, end); false on a malformed record (the rest of the range is left as it is).
+bool apply_delta_range(const uint32_t *delta, int8_t *obs, int64_t begin, int64_t end, int cells) {
+    for (int64_t e = begin; e < end; ++e) {
+        const uint32_t r = delta[e];
+        if (r == BENG_OBS_DELTA_NONE) continue;
+        if (r & 0x70000000u) return false;
+        int8_t *row = obs + e * cells;
+        if (r & BENG_OBS_DELTA_CLEAR) memset(row, 0, (size_t)cells);
+        for (const uint32_t pr : {r & 0x3FFFu, (r >> 14) & 0x3FFFu}) {
+            const uint32_t cell = pr & 0xFFFu, value = pr >> 12;
+            if (value == 3) continue;
+            if (cell >= (uint32_t)cells) return false;
+            row[cell] = (int8_t)value;
+        }
+    }
+    return true;
 }
 
 }  // namespace
@@ -564,13 +624,7 @@ int beng_snake_reset(const beng_snake_params *p, const beng_snake_state *st, con
 
 int beng_snake_step(const beng_snake_params *p, const beng_snake_state *st, const int64_t *actions_dev,
                     const beng_snake_io *io, int64_t n_envs, void *stream) {
-    if (int rc = beng::check_common(p, st, io, n_envs)) return rc;
-    if (!actions_dev || !io->reward || !io->terminated) return BENG_ERR_BAD_ARG;
-    if ((uintptr_t)actions_dev & 7) return BENG_ERR_BAD_ARG;  // 64-bit action loads (int64, or float32 pairs)
-    if (n_envs == 0) return 0;
-    beng::Args a = beng::make_args(p, st, io, n_envs);
-    a.actions = (const long long *)actions_dev;
-    return beng::launch<false>(a, (cudaStream_t)stream);
+    return beng::step(p, st, actions_dev, io, n_envs, nullptr, (cudaStream_t)stream);
 }
 
 int beng_snake_step_host(const beng_snake_params *p, const beng_snake_state *st, int64_t *actions_dev,
@@ -593,6 +647,56 @@ int beng_snake_step_host(const beng_snake_params *p, const beng_snake_state *st,
     if (int rc = beng::d2h(score_host, io->score, n * sizeof(int32_t), s)) return rc;
     if (int rc = beng::d2h(snake_length_host, io->snake_length, n * sizeof(int32_t), s)) return rc;
     return beng::d2h(obs_host, io->obs, n * cells, s);
+}
+
+int beng_snake_step_host_delta(const beng_snake_params *p, const beng_snake_state *st, int64_t *actions_dev,
+                               const beng_snake_io *io, int64_t n_envs, const int64_t *actions_host,
+                               uint32_t *delta_dev, uint32_t *delta_host, float *reward_host, uint8_t *terminated_host,
+                               uint8_t *truncated_host, int32_t *score_host, int32_t *snake_length_host, void *stream) {
+    if (!actions_host || !actions_dev || !delta_dev || !delta_host) return BENG_ERR_BAD_ARG;
+    if (((uintptr_t)delta_dev & 3) || ((uintptr_t)delta_host & 3)) return BENG_ERR_BAD_ARG;
+    if (int rc = beng::check_common(p, st, io, n_envs)) return rc;
+    if ((truncated_host && !io->truncated) || (score_host && !io->score) || (snake_length_host && !io->snake_length))
+        return BENG_ERR_BAD_ARG;
+    if (n_envs == 0) return 0;
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t n = (size_t)n_envs;
+    cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, n * sizeof(int64_t), cudaMemcpyHostToDevice, s);
+    if (e != cudaSuccess) return (int)e;
+    if (int rc = beng::step(p, st, actions_dev, io, n_envs, delta_dev, s)) return rc;
+    if (int rc = beng::d2h(delta_host, delta_dev, n * sizeof(uint32_t), s)) return rc;
+    if (int rc = beng::d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
+    if (int rc = beng::d2h(terminated_host, io->terminated, n, s)) return rc;
+    if (int rc = beng::d2h(truncated_host, io->truncated, n, s)) return rc;
+    if (int rc = beng::d2h(score_host, io->score, n * sizeof(int32_t), s)) return rc;
+    return beng::d2h(snake_length_host, io->snake_length, n * sizeof(int32_t), s);
+}
+
+int beng_snake_apply_obs_delta(const uint32_t *delta_host, int8_t *obs_host, int64_t n_envs, int32_t grid_size,
+                               int32_t n_threads) {
+    if (n_envs < 0 || (n_envs > 0 && (!delta_host || !obs_host))) return BENG_ERR_BAD_ARG;
+    if (grid_size < 2 || grid_size > 64) return BENG_ERR_UNSUPPORTED;
+    if (n_envs == 0) return 0;
+    const int cells = grid_size * grid_size;
+    const int64_t nt = n_threads < 1 ? 1 : (n_threads < n_envs ? n_threads : n_envs);
+    // Thread t applies envs [n * t / nt, n * (t + 1) / nt); the calling thread takes chunk 0.  A chunk whose thread
+    // cannot be started is applied by the calling thread instead (this function never throws).
+    std::vector<char> ok((size_t)nt, 1);
+    std::vector<std::thread> workers;
+    for (int64_t t = 1; t < nt; ++t) {
+        const int64_t b = n_envs * t / nt, en = n_envs * (t + 1) / nt;
+        auto job = [=, &ok] { ok[t] = beng::apply_delta_range(delta_host, obs_host, b, en, cells); };
+        try {
+            workers.emplace_back(job);
+        } catch (...) {
+            job();
+        }
+    }
+    ok[0] = beng::apply_delta_range(delta_host, obs_host, 0, n_envs / nt, cells);
+    for (std::thread &w : workers) w.join();
+    for (const char o : ok)
+        if (!o) return BENG_ERR_BAD_ARG;
+    return 0;
 }
 
 int beng_snake_export_state(const beng_snake_params *p, const beng_snake_state *st, int64_t n_envs, int32_t *head_r,

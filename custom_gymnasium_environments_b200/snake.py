@@ -12,6 +12,7 @@ but the direction (snake_env.py:88-94), a non-eating step has reward 0.
 from __future__ import annotations
 
 import ctypes as C
+import os
 
 import numpy as np
 import torch
@@ -88,6 +89,9 @@ class BatchedSnakeEnv(_VectorEnvBase):
         self._ios_full = [self._make_io(self.obs, 0, True), self._make_io(self.obs, 1, True)]
         self._info_fresh = True
         self._host = None
+        # True while the pinned host["obs"] equals the device observations: set by a full-copy step_host(), cleared by
+        # anything else that rewrites them.  step_host(delta_obs=True) patches the copy only while it is set.
+        self._obs_mirror_valid = False
         self._needs_first_reset = True
 
     # ------------------------------------------------------------------ plumbing
@@ -155,6 +159,7 @@ class BatchedSnakeEnv(_VectorEnvBase):
                 raise RuntimeError("the first reset() must reset every env")
         with torch.cuda.device(self.device):
             self._info_fresh = True
+            self._obs_mirror_valid = False
             rc = self.lib.beng_snake_reset(C.byref(self.params), C.byref(self._state), C.byref(self._ios_full[0]), mask_ptr,
                                            self.num_envs, int(first), stream_ptr(self.device))
         _lib.check(rc, "beng_snake_reset")
@@ -177,6 +182,7 @@ class BatchedSnakeEnv(_VectorEnvBase):
                     or out_obs.device != self.device:
                 raise ValueError("out_obs must be a contiguous int8 CUDA tensor of shape (num_envs, G, G)")
             io, obs = self._make_io(out_obs, self._parity), out_obs
+        self._obs_mirror_valid = False
         with torch.cuda.device(self.device):
             rc = self.lib.beng_snake_step(C.byref(self.params), C.byref(self._state), act.data_ptr(), C.byref(io),
                                           self.num_envs, stream_ptr(self.device))
@@ -204,33 +210,60 @@ class BatchedSnakeEnv(_VectorEnvBase):
                 "truncated": torch.zeros(n, dtype=torch.bool, **pin),
                 "score": torch.zeros(n, dtype=torch.int32, **pin),
                 "snake_length": torch.zeros(n, dtype=torch.int32, **pin),
+                "delta": torch.zeros(n, dtype=torch.int32, **pin),  # observation change records (uint32 bits)
             }
+            self._delta_dev = torch.zeros(n, dtype=torch.int32, device=self.device)
         return self._host
 
-    def step_host(self, actions, *, copy_obs: bool = True, sync: bool = True):
+    def step_host(self, actions, *, copy_obs: bool = True, sync: bool = True, delta_obs: bool = False):
         """step() for callers holding HOST arrays, like users of the reference's numpy API.
 
         Enqueues H2D(actions) -> kernel -> D2H(results) through `beng_snake_step_host` and (by
         default) waits; returns numpy views of pinned host buffers (valid until the next call).
         copy_obs=False leaves the observations in HBM (obs returned is the CUDA tensor).
+
+        delta_obs=True keeps the pinned observation buffer as a mirror of the device observations
+        and brings it up to date from one 4-byte change record per env (`beng_snake_step_host_delta`
+        + `beng_snake_apply_obs_delta`) instead of copying G*G bytes per env.  When the mirror is
+        not current (first call, or reset()/step()/load_state_dict()/step_host(copy_obs=False)
+        since the last step_host), the call copies the observations in full instead.  The returned
+        observation is read-only.  Needs sync=True and copy_obs=True.
         """
+        if delta_obs and not (sync and copy_obs):
+            raise ValueError("step_host(delta_obs=True) needs sync=True and copy_obs=True")
         if self._needs_first_reset:
             raise RuntimeError("call reset() before step()")
         h = self._host_buffers()
         src = torch.as_tensor(np.asarray(actions) if not isinstance(actions, torch.Tensor) else actions)
         src = self._host_src = host_source(src, h["actions"])
+        delta = delta_obs and self._obs_mirror_valid
+        self._obs_mirror_valid = False
+        results = (h["reward"].data_ptr(), h["terminated"].data_ptr(), h["truncated"].data_ptr(),
+                   h["score"].data_ptr(), h["snake_length"].data_ptr(), stream_ptr(self.device))
         with torch.cuda.device(self.device):
-            rc = self.lib.beng_snake_step_host(
-                C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._next_io(True)),
-                self.num_envs, src.data_ptr(), h["obs"].data_ptr() if copy_obs else None,
-                h["reward"].data_ptr(), h["terminated"].data_ptr(), h["truncated"].data_ptr(),
-                h["score"].data_ptr(), h["snake_length"].data_ptr(), stream_ptr(self.device))
-            _lib.check(rc, "beng_snake_step_host")
+            if delta:
+                rc = self.lib.beng_snake_step_host_delta(
+                    C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._next_io(True)),
+                    self.num_envs, src.data_ptr(), self._delta_dev.data_ptr(), h["delta"].data_ptr(), *results)
+                _lib.check(rc, "beng_snake_step_host_delta")
+            else:
+                rc = self.lib.beng_snake_step_host(
+                    C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._next_io(True)),
+                    self.num_envs, src.data_ptr(), h["obs"].data_ptr() if copy_obs else None, *results)
+                _lib.check(rc, "beng_snake_step_host")
             if sync:
                 torch.cuda.current_stream(self.device).synchronize()
+        if delta:
+            rc = self.lib.beng_snake_apply_obs_delta(h["delta"].data_ptr(), h["obs"].data_ptr(), self.num_envs,
+                                                     self.grid_size, len(os.sched_getaffinity(0)))
+            _lib.check(rc, "beng_snake_apply_obs_delta")
+        self._obs_mirror_valid = copy_obs
         if self.debug_checks:
             self._raise_on_invalid()
         obs = h["obs"].numpy() if copy_obs else self.obs
+        if delta_obs:
+            obs = obs.view()
+            obs.flags.writeable = False  # the mirror of the next delta step
         infos = {"score": h["score"].numpy(), "snake_length": h["snake_length"].numpy()}
         return obs, h["reward"].numpy(), h["terminated"].numpy(), h["truncated"].numpy(), infos
 
@@ -272,6 +305,7 @@ class BatchedSnakeEnv(_VectorEnvBase):
         self.stats.copy_(sd["stats"])
         self.params.seed = int(sd["seed"])
         self.params.env_id_base = int(sd["env_id_base"])
+        self._obs_mirror_valid = False
         self._needs_first_reset = False
 
     def render(self):

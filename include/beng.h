@@ -143,6 +143,40 @@ int beng_snake_step_host(const beng_snake_params *p, const beng_snake_state *st,
                          float *reward_host, uint8_t *terminated_host, uint8_t *truncated_host, int32_t *score_host,
                          int32_t *snake_length_host, void *stream);
 
+/* Observation change records of beng_snake_step_host_delta: one uint32_t per env and step, telling how the env's
+ * observation row [G*G] differs from the one the previous step or reset wrote.
+ *   pair    = cell | value << 12  (14 bits; cell = r * G + c < 4096; value 0 / 1 / 2 is written to the cell,
+ *             value 3 marks an unused pair)
+ *   record  = pair A (bits 0-13) | pair B << 14 (bits 14-27) | BENG_OBS_DELTA_CLEAR (bit 31); bits 28-30 are 0
+ *   applied = clear the whole row if bit 31 is set, then write A, then B.
+ * What the step kernel emits:
+ *   move                        A = (old tail, 0), B = (new head, 1)
+ *   eat                         A = (new head, 1), B = (new food, 2), or unused when the board is full
+ *   death, invalid action       both unused (the row does not change)
+ *   any auto-reset              CLEAR, A = (head, 1), B = (food, 2) */
+#define BENG_OBS_DELTA_CLEAR 0x80000000u
+#define BENG_OBS_DELTA_UNUSED 0x3000u                                       /* one unused pair */
+#define BENG_OBS_DELTA_NONE (BENG_OBS_DELTA_UNUSED | (BENG_OBS_DELTA_UNUSED << 14)) /* no change */
+
+/* beng_snake_step_host without the observation copy: enqueues H2D(actions) -> step kernel, which also writes one
+ * change record per env to delta_dev -> D2H(records, reward, terminated[, truncated, score, snake_length]) on
+ * `stream`.  io->obs on the device is written exactly as by beng_snake_step.  A caller that holds a host copy of
+ * the observations from before this step brings it up to date with beng_snake_apply_obs_delta once the stream has
+ * drained: 18 B per env cross the bus instead of G*G + 14.  delta_dev / delta_host (uint32_t[n_envs], device /
+ * pinned host, 4-byte aligned) are required; NULL result host pointers are skipped.  Does not synchronise. */
+int beng_snake_step_host_delta(const beng_snake_params *p, const beng_snake_state *st, int64_t *actions_dev,
+                               const beng_snake_io *io, int64_t n_envs, const int64_t *actions_host,
+                               uint32_t *delta_dev, uint32_t *delta_host, float *reward_host, uint8_t *terminated_host,
+                               uint8_t *truncated_host, int32_t *score_host, int32_t *snake_length_host, void *stream);
+
+/* Apply one step's change records (host memory, uint32_t[n_envs]) to a host copy of the observations
+ * (int8_t[n_envs][G][G]).  Pure host code: touches no CUDA state and runs without a GPU.  The envs are split into
+ * contiguous chunks over n_threads threads (<= 0 means one), all joined before it returns.  BENG_ERR_BAD_ARG for
+ * NULL buffers, n_envs < 0 or a malformed record (set bits 28-30, or a cell >= G*G; obs_host is then partly
+ * updated), BENG_ERR_UNSUPPORTED for grid_size outside [2, 64]. */
+int beng_snake_apply_obs_delta(const uint32_t *delta_host, int8_t *obs_host, int64_t n_envs, int32_t grid_size,
+                               int32_t n_threads);
+
 /* Unpack the SoA state into plain int32 arrays (tests, checkpoints, debugging).  Any output may be NULL.
  * body_cells_dev, when given, is [n_envs, G*G] int32 filled head-first with r*G+c and -1 padding. */
 int beng_snake_export_state(const beng_snake_params *p, const beng_snake_state *st, int64_t n_envs, int32_t *head_r,
