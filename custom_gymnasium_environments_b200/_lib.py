@@ -135,6 +135,9 @@ SIGNATURES = {
                                     C.POINTER(BuilderIO), C.c_int64, C.c_void_p]),
     "beng_builder_step_host": (C.c_int, [C.POINTER(BuilderParams), C.POINTER(BuilderState), C.c_void_p,
                                          C.POINTER(BuilderIO), C.c_int64] + [C.c_void_p] * 8),
+    "beng_builder_step_host_delta": (C.c_int, [C.POINTER(BuilderParams), C.POINTER(BuilderState), C.c_void_p,
+                                               C.POINTER(BuilderIO), C.c_int64] + [C.c_void_p] * 9),
+    "beng_builder_apply_obs_delta": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32]),
     "beng_snake_export_state": (C.c_int, [C.POINTER(SnakeParams), C.POINTER(SnakeState), C.c_int64] +
                                 [C.c_void_p] * 10),
 }

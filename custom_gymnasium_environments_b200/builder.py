@@ -13,6 +13,7 @@ kept.  There is no time limit: an episode ends by starvation (-100) or after 50 
 from __future__ import annotations
 
 import ctypes as C
+import os
 
 import numpy as np
 import torch
@@ -80,6 +81,9 @@ class BatchedWorldBuilderEnv(_VectorEnvBase):
                                   self.ep_return.data_ptr(), self.ep_length.data_ptr(), self.stats.data_ptr(),
                                   self.invalid_count.data_ptr())
         self._host = None
+        # True while the pinned host["grid"] equals the device grid: set by a full-copy step_host(), cleared by anything
+        # else that rewrites it.  step_host(delta_obs=True) patches the copy only while it is set.
+        self._grid_mirror_valid = False
         self._needs_first_reset = True
 
     # ------------------------------------------------------------------ state views
@@ -124,6 +128,7 @@ class BatchedWorldBuilderEnv(_VectorEnvBase):
             if mask.shape != (self.num_envs,):
                 raise ValueError("reset_mask must have shape (num_envs,)")
             mask_ptr = mask.data_ptr()
+        self._grid_mirror_valid = False
         with torch.cuda.device(self.device):
             rc = self.lib.beng_builder_reset(C.byref(self.params), C.byref(self._state), C.byref(self._io), mask_ptr,
                                              self.num_envs, int(first), stream_ptr(self.device))
@@ -136,6 +141,7 @@ class BatchedWorldBuilderEnv(_VectorEnvBase):
         if self._needs_first_reset:
             raise RuntimeError("call reset() before step()")
         act = as_device_actions(actions, self._actions)
+        self._grid_mirror_valid = False
         with torch.cuda.device(self.device):
             rc = self.lib.beng_builder_step(C.byref(self.params), C.byref(self._state), act.data_ptr(),
                                             C.byref(self._io), self.num_envs, stream_ptr(self.device))
@@ -147,8 +153,17 @@ class BatchedWorldBuilderEnv(_VectorEnvBase):
                 raise ValueError(f"Invalid action: {n_bad} action(s) outside Discrete(5)")  # :135-136
         return self._obs(), self.reward, self.terminated, self.truncated, self._infos()
 
-    def step_host(self, actions, *, copy_obs: bool = True, sync: bool = True):
-        """step() for callers holding HOST arrays (numpy in, numpy out) through `beng_builder_step_host`."""
+    def step_host(self, actions, *, copy_obs: bool = True, sync: bool = True, delta_obs: bool = False):
+        """step() for callers holding HOST arrays (numpy in, numpy out) through `beng_builder_step_host`.
+
+        delta_obs=True keeps the pinned grid buffer as a mirror of the device grid and brings it up to date from one
+        4-byte change record per env (`beng_builder_step_host_delta` + `beng_builder_apply_obs_delta`) instead of
+        copying G*G bytes per env.  When the mirror is not current (first call, or reset()/step()/load_state_dict()/
+        step_host(copy_obs=False) since the last step_host), the call copies the grid in full instead.  The returned
+        obs['grid'] is read-only.  Needs sync=True and copy_obs=True.
+        """
+        if delta_obs and not (sync and copy_obs):
+            raise ValueError("step_host(delta_obs=True) needs sync=True and copy_obs=True")
         if self._needs_first_reset:
             raise RuntimeError("call reset() before step()")
         if self._host is None:
@@ -160,20 +175,39 @@ class BatchedWorldBuilderEnv(_VectorEnvBase):
                           "capacity": torch.zeros((n, 1), dtype=torch.float32, **pin),
                           "win_steps": torch.zeros((n, 1), dtype=torch.int32, **pin),
                           "reward": torch.zeros(n, dtype=torch.float32, **pin),
-                          "terminated": torch.zeros(n, dtype=torch.bool, **pin)}
+                          "terminated": torch.zeros(n, dtype=torch.bool, **pin),
+                          "delta": torch.zeros(n, dtype=torch.int32, **pin)}  # grid change records (uint32 bits)
+            self._delta_dev = torch.zeros(n, dtype=torch.int32, device=self.device)
         h = self._host
         src = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions))
         src = self._host_src = host_source(src, h["actions"])
+        delta = delta_obs and self._grid_mirror_valid
+        self._grid_mirror_valid = False
+        results = (h["resources"].data_ptr(), h["capacity"].data_ptr(), h["win_steps"].data_ptr(),
+                   h["reward"].data_ptr(), h["terminated"].data_ptr(), stream_ptr(self.device))
         with torch.cuda.device(self.device):
-            rc = self.lib.beng_builder_step_host(
-                C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._io),
-                self.num_envs, src.data_ptr(), h["grid"].data_ptr() if copy_obs else None,
-                h["resources"].data_ptr(), h["capacity"].data_ptr(), h["win_steps"].data_ptr(),
-                h["reward"].data_ptr(), h["terminated"].data_ptr(), stream_ptr(self.device))
-            _lib.check(rc, "beng_builder_step_host")
+            if delta:
+                rc = self.lib.beng_builder_step_host_delta(
+                    C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._io),
+                    self.num_envs, src.data_ptr(), self._delta_dev.data_ptr(), h["delta"].data_ptr(), *results)
+                _lib.check(rc, "beng_builder_step_host_delta")
+            else:
+                rc = self.lib.beng_builder_step_host(
+                    C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._io),
+                    self.num_envs, src.data_ptr(), h["grid"].data_ptr() if copy_obs else None, *results)
+                _lib.check(rc, "beng_builder_step_host")
             if sync:
                 torch.cuda.current_stream(self.device).synchronize()
-        obs = {"grid": h["grid"].numpy() if copy_obs else self.grid, "resources": h["resources"].numpy(),
+        if delta:
+            rc = self.lib.beng_builder_apply_obs_delta(h["delta"].data_ptr(), h["grid"].data_ptr(), self.num_envs,
+                                                       self.grid_size, len(os.sched_getaffinity(0)))
+            _lib.check(rc, "beng_builder_apply_obs_delta")
+        self._grid_mirror_valid = copy_obs
+        grid = h["grid"].numpy() if copy_obs else self.grid
+        if delta_obs:
+            grid = grid.view()
+            grid.flags.writeable = False  # the mirror of the next delta step
+        obs = {"grid": grid, "resources": h["resources"].numpy(),
                "population_capacity": h["capacity"].numpy(), "win_steps": h["win_steps"].numpy()}
         return obs, h["reward"].numpy(), h["terminated"].numpy(), np.zeros(self.num_envs, dtype=bool), {}
 
@@ -189,6 +223,7 @@ class BatchedWorldBuilderEnv(_VectorEnvBase):
         self.grid.copy_(sd["grid"])
         self.stats.copy_(sd["stats"])
         self.params.seed, self.params.env_id_base = int(sd["seed"]), int(sd["env_id_base"])
+        self._grid_mirror_valid = False
         self._needs_first_reset = False
 
     def render(self):

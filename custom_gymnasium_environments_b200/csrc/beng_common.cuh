@@ -6,6 +6,7 @@
 #include <atomic>
 #include <cstdint>
 #include <cstdlib>
+#include <functional>
 
 #include "../../include/beng.h"
 
@@ -74,6 +75,12 @@ inline cudaError_t launch_pdl(Kern kern, dim3 grid, dim3 block, size_t smem, cud
 inline cudaError_t d2h(void *dst, const void *src, size_t bytes, cudaStream_t stream) {
     return dst ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, stream) : cudaSuccess;
 }
+
+// Host fan-out of the *_apply_obs_delta functions: runs chunk(begin, end) over [0, n) split into nt = clamp(n_threads,
+// 1, n) contiguous chunks [n * t / nt, n * (t + 1) / nt), one thread each, the calling thread taking chunk 0, and joins
+// them all.  A chunk whose thread cannot be started runs on the calling thread instead (this never throws).  True
+// when every chunk returned true.
+bool for_each_chunk(int64_t n, int32_t n_threads, const std::function<bool(int64_t, int64_t)> &chunk);
 
 // streaming (evict-first) 128-bit / 64-bit global loads for read-once inputs
 __device__ __forceinline__ uint4 ld_stream_u4(const uint4 *p) {

@@ -1,10 +1,34 @@
-// libbeng core: version / launch accounting and the synthetic action-tape kernel.
+// libbeng core: version / launch accounting, the host thread fan-out and the synthetic action-tape kernel.
+#include <thread>
+#include <vector>
+
 #include "beng_common.cuh"
 #include "beng_rng.cuh"
 
 namespace beng {
 
 std::atomic<uint64_t> g_launch_count{0};
+
+bool for_each_chunk(int64_t n, int32_t n_threads, const std::function<bool(int64_t, int64_t)> &chunk) {
+    if (n <= 0) return true;
+    const int64_t nt = n_threads < 1 ? 1 : (n_threads < n ? n_threads : n);
+    std::vector<char> ok((size_t)nt, 1);
+    std::vector<std::thread> workers;
+    for (int64_t t = 1; t < nt; ++t) {
+        const int64_t b = n * t / nt, e = n * (t + 1) / nt;
+        auto job = [=, &ok, &chunk] { ok[t] = chunk(b, e); };
+        try {
+            workers.emplace_back(job);
+        } catch (...) {
+            job();
+        }
+    }
+    ok[0] = chunk(0, n / nt);
+    for (std::thread &w : workers) w.join();
+    for (const char o : ok)
+        if (!o) return false;
+    return true;
+}
 
 int device_sm_count() {
     static int cached = 0;

@@ -12,6 +12,7 @@
 // (flatten_obs=True, :189-200) is composed in a second tile and drained the same way.
 #include <cstdint>
 #include <cstdlib>
+#include <cstring>
 
 #include "beng_common.cuh"
 #include "beng_rng.cuh"
@@ -30,10 +31,14 @@ struct BArgs {
     const uint8_t *mask;
     long long n;
     int first_call;
+    uint32_t *delta;  // DELTA step only: one BENG_BUILDER_DELTA record per env
 };
 
 // CELLS_T: G*G when it is known at compile time and a multiple of 4 (the default 10 x 10 board), 0 = any board.
-template <int T, bool IS_RESET, int CELLS_T>
+// DELTA (step only): also store one change record per env to a.delta, describing how this step's grid row differs
+// from the previous one.  It is assembled from the dynamics' registers (the cell and building of a successful build,
+// the reset_env() call sites), never by reading the row back.
+template <int T, bool IS_RESET, int CELLS_T, bool DELTA>
 __global__ void __launch_bounds__(T) builder_kernel(const BArgs a) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     __shared__ int s_stats[4];  // per-CTA: n_episodes, sum_return, sum_length, wins
@@ -91,6 +96,7 @@ __global__ void __launch_bounds__(T) builder_kernel(const BArgs a) {
         EnvStream rng(a.p.seed, a.p.env_id_base + (uint64_t)env, BENG_STREAM_ENV, ctr);
         int rew = 0, term = 0;
         bool invalid = false;
+        uint32_t rec = BENG_BUILDER_DELTA_NONE;  // DELTA: passes, failed builds, invalid actions change no cell
 
         // Rows start on 4-byte boundaries when G*G is a multiple of 4 (G even, e.g. the default 10): the three loops
         // over the row (clear, count empty cells, find the k-th empty cell) then run word-wise, 4 cells at a time.
@@ -108,6 +114,7 @@ __global__ void __launch_bounds__(T) builder_kernel(const BArgs a) {
         } else {
             if (a.p.autoreset_mode == BENG_AUTORESET_NEXT_STEP && (flags & BFLAG_NEEDS_RESET)) {
                 reset_env();
+                if constexpr (DELTA) rec = BENG_BUILDER_DELTA_CLEAR;
             } else if (act < 0 || act > 4) {
                 invalid = true;  // the reference raises ValueError (:135-136); the env is left untouched
             } else {
@@ -195,6 +202,7 @@ __global__ void __launch_bounds__(T) builder_kernel(const BArgs a) {
                         else if (action == QUARRY) wood -= 5;
                         else { wood -= 10; stone -= 5; }
                         row[pos] = (uint8_t)action;
+                        if constexpr (DELTA) rec = (uint32_t)pos | ((uint32_t)action << 8);
                         counts += 1u << (8 * (action - 1));
                         if (action == HOUSE) cap += 5;
                         rew += (action == FARM) ? 3 : (action == HOUSE) ? 4 : 2;
@@ -228,11 +236,16 @@ __global__ void __launch_bounds__(T) builder_kernel(const BArgs a) {
                     ep_len_out = steps;
                     if (a.io.ep_return) a.io.ep_return[env] = ep_ret;
                     if (a.io.ep_length) a.io.ep_length[env] = steps;
-                    if (a.p.autoreset_mode == BENG_AUTORESET_SAME_STEP) reset_env();
-                    else flags |= BFLAG_NEEDS_RESET;
+                    if (a.p.autoreset_mode == BENG_AUTORESET_SAME_STEP) {
+                        reset_env();
+                        if constexpr (DELTA) rec = BENG_BUILDER_DELTA_CLEAR;  // also undoes this step's build
+                    } else {
+                        flags |= BFLAG_NEEDS_RESET;
+                    }
                 }
             }
             a.io.reward[env] = (float)rew;
+            if constexpr (DELTA) a.delta[env] = rec;
             a.io.terminated[env] = (uint8_t)term;
             if (a.io.truncated) a.io.truncated[env] = 0;
             if (invalid && a.io.invalid_count) atomicAdd(a.io.invalid_count, 1);
@@ -299,12 +312,13 @@ __global__ void __launch_bounds__(T) builder_kernel(const BArgs a) {
 
 constexpr int BUILDER_T = 64;  // envs (= threads) per CTA; same-box sweep at 1M envs: 64 -> 75.6 us, 128 -> 76.8, 256 -> 82.7
 
-template <bool IS_RESET>
+template <bool IS_RESET, bool DELTA = false>
 int launch(const BArgs &a, cudaStream_t stream) {
     const int cells = a.p.grid_size * a.p.grid_size;
     size_t smem = ((size_t)BUILDER_T * cells + 15) & ~(size_t)15;
     if (a.io.flat_obs) smem += (size_t)BUILDER_T * (cells + 6) * sizeof(float);
-    auto kern = cells == 100 ? builder_kernel<BUILDER_T, IS_RESET, 100> : builder_kernel<BUILDER_T, IS_RESET, 0>;
+    auto kern = cells == 100 ? builder_kernel<BUILDER_T, IS_RESET, 100, DELTA>
+                             : builder_kernel<BUILDER_T, IS_RESET, 0, DELTA>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     return (int)launch_pdl(kern, dim3((unsigned)((a.n + BUILDER_T - 1) / BUILDER_T)), dim3(BUILDER_T), smem, stream, a);
@@ -318,6 +332,32 @@ int check(const beng_builder_params *p, const beng_builder_state *st, const beng
     if (p->autoreset_mode < 0 || p->autoreset_mode > 2) return BENG_ERR_BAD_ARG;
     if (p->grid_size < 2 || p->grid_size > 15) return BENG_ERR_UNSUPPORTED;
     return 0;
+}
+
+// beng_builder_step without its public name: `delta` non-null selects the DELTA kernel.
+int step(const beng_builder_params *p, const beng_builder_state *st, const int64_t *actions_dev,
+         const beng_builder_io *io, int64_t n_envs, uint32_t *delta, cudaStream_t stream) {
+    if (int rc = check(p, st, io, n_envs)) return rc;
+    if (!actions_dev || !io->reward || !io->terminated) return BENG_ERR_BAD_ARG;
+    if ((uintptr_t)actions_dev & 7) return BENG_ERR_BAD_ARG;  // 64-bit action loads (int64, or float32 pairs)
+    if (n_envs == 0) return 0;
+    BArgs a{*p, *st, *io, (const long long *)actions_dev, nullptr, (long long)n_envs, 0, delta};
+    return delta ? launch<false, true>(a, stream) : launch<false>(a, stream);
+}
+
+// Applies the records of envs [begin, end); false on a malformed record (its row and the rest of the range are left
+// as they are).
+bool apply_delta_range(const uint32_t *delta, int8_t *grid, int64_t begin, int64_t end, uint32_t cells) {
+    for (int64_t e = begin; e < end; ++e) {
+        const uint32_t r = delta[e];
+        if (r == BENG_BUILDER_DELTA_NONE) continue;
+        const uint32_t cell = r & 0xFFu, value = (r >> 8) & 7u;
+        if ((r & 0x7FFFF800u) || value > 4 || (value ? cell >= cells : cell != 0)) return false;
+        int8_t *row = grid + e * cells;
+        if (r & BENG_BUILDER_DELTA_CLEAR) memset(row, 0, cells);
+        if (value) row[cell] = (int8_t)value;
+    }
+    return true;
 }
 
 }  // namespace
@@ -335,12 +375,7 @@ int beng_builder_reset(const beng_builder_params *p, const beng_builder_state *s
 
 int beng_builder_step(const beng_builder_params *p, const beng_builder_state *st, const int64_t *actions_dev,
                       const beng_builder_io *io, int64_t n_envs, void *stream) {
-    if (int rc = beng::check(p, st, io, n_envs)) return rc;
-    if (!actions_dev || !io->reward || !io->terminated) return BENG_ERR_BAD_ARG;
-    if ((uintptr_t)actions_dev & 7) return BENG_ERR_BAD_ARG;  // 64-bit action loads (int64, or float32 pairs)
-    if (n_envs == 0) return 0;
-    beng::BArgs a{*p, *st, *io, (const long long *)actions_dev, nullptr, (long long)n_envs, 0};
-    return beng::launch<false>(a, (cudaStream_t)stream);
+    return beng::step(p, st, actions_dev, io, n_envs, nullptr, (cudaStream_t)stream);
 }
 
 int beng_builder_step_host(const beng_builder_params *p, const beng_builder_state *st, int64_t *actions_dev,
@@ -363,6 +398,40 @@ int beng_builder_step_host(const beng_builder_params *p, const beng_builder_stat
     if (int rc = beng::d2h(capacity_host, io->capacity, n * sizeof(float), s)) return rc;
     if (int rc = beng::d2h(win_steps_host, io->win_steps, n * sizeof(int32_t), s)) return rc;
     return beng::d2h(grid_host, io->grid, n * cells, s);
+}
+
+int beng_builder_step_host_delta(const beng_builder_params *p, const beng_builder_state *st, int64_t *actions_dev,
+                                 const beng_builder_io *io, int64_t n_envs, const int64_t *actions_host,
+                                 uint32_t *delta_dev, uint32_t *delta_host, float *resources_host, float *capacity_host,
+                                 int32_t *win_steps_host, float *reward_host, uint8_t *terminated_host, void *stream) {
+    if (!actions_host || !actions_dev || !delta_dev || !delta_host) return BENG_ERR_BAD_ARG;
+    if (((uintptr_t)delta_dev & 3) || ((uintptr_t)delta_host & 3)) return BENG_ERR_BAD_ARG;
+    if (int rc = beng::check(p, st, io, n_envs)) return rc;
+    if ((resources_host && !io->resources) || (capacity_host && !io->capacity) || (win_steps_host && !io->win_steps))
+        return BENG_ERR_BAD_ARG;
+    if (n_envs == 0) return 0;
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t n = (size_t)n_envs;
+    cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, n * sizeof(int64_t), cudaMemcpyHostToDevice, s);
+    if (e != cudaSuccess) return (int)e;
+    if (int rc = beng::step(p, st, actions_dev, io, n_envs, delta_dev, s)) return rc;
+    if (int rc = beng::d2h(delta_host, delta_dev, n * sizeof(uint32_t), s)) return rc;
+    if (int rc = beng::d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
+    if (int rc = beng::d2h(terminated_host, io->terminated, n, s)) return rc;
+    if (int rc = beng::d2h(resources_host, io->resources, n * 4 * sizeof(float), s)) return rc;
+    if (int rc = beng::d2h(capacity_host, io->capacity, n * sizeof(float), s)) return rc;
+    return beng::d2h(win_steps_host, io->win_steps, n * sizeof(int32_t), s);
+}
+
+int beng_builder_apply_obs_delta(const uint32_t *delta_host, int8_t *grid_host, int64_t n_envs, int32_t grid_size,
+                                 int32_t n_threads) {
+    if (n_envs < 0 || (n_envs > 0 && (!delta_host || !grid_host))) return BENG_ERR_BAD_ARG;
+    if (grid_size < 2 || grid_size > 15) return BENG_ERR_UNSUPPORTED;
+    const uint32_t cells = (uint32_t)(grid_size * grid_size);
+    const bool ok = beng::for_each_chunk(n_envs, n_threads, [=](int64_t b, int64_t e) {
+        return beng::apply_delta_range(delta_host, grid_host, b, e, cells);
+    });
+    return ok ? 0 : BENG_ERR_BAD_ARG;
 }
 
 }  // extern "C"

@@ -27,8 +27,6 @@
 #include <climits>
 #include <cstdint>
 #include <cstring>
-#include <thread>
-#include <vector>
 
 #include "beng_common.cuh"
 #include "beng_rng.cuh"
@@ -678,25 +676,10 @@ int beng_snake_apply_obs_delta(const uint32_t *delta_host, int8_t *obs_host, int
     if (grid_size < 2 || grid_size > 64) return BENG_ERR_UNSUPPORTED;
     if (n_envs == 0) return 0;
     const int cells = grid_size * grid_size;
-    const int64_t nt = n_threads < 1 ? 1 : (n_threads < n_envs ? n_threads : n_envs);
-    // Thread t applies envs [n * t / nt, n * (t + 1) / nt); the calling thread takes chunk 0.  A chunk whose thread
-    // cannot be started is applied by the calling thread instead (this function never throws).
-    std::vector<char> ok((size_t)nt, 1);
-    std::vector<std::thread> workers;
-    for (int64_t t = 1; t < nt; ++t) {
-        const int64_t b = n_envs * t / nt, en = n_envs * (t + 1) / nt;
-        auto job = [=, &ok] { ok[t] = beng::apply_delta_range(delta_host, obs_host, b, en, cells); };
-        try {
-            workers.emplace_back(job);
-        } catch (...) {
-            job();
-        }
-    }
-    ok[0] = beng::apply_delta_range(delta_host, obs_host, 0, n_envs / nt, cells);
-    for (std::thread &w : workers) w.join();
-    for (const char o : ok)
-        if (!o) return BENG_ERR_BAD_ARG;
-    return 0;
+    const bool ok = beng::for_each_chunk(n_envs, n_threads, [=](int64_t b, int64_t e) {
+        return beng::apply_delta_range(delta_host, obs_host, b, e, cells);
+    });
+    return ok ? 0 : BENG_ERR_BAD_ARG;
 }
 
 int beng_snake_export_state(const beng_snake_params *p, const beng_snake_state *st, int64_t n_envs, int32_t *head_r,

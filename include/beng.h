@@ -442,6 +442,41 @@ int beng_builder_step_host(const beng_builder_params *p, const beng_builder_stat
                            float *resources_host, float *capacity_host, int32_t *win_steps_host, float *reward_host,
                            uint8_t *terminated_host, void *stream);
 
+/* Grid change records of beng_builder_step_host_delta: one uint32_t per env and step, telling how the env's grid row
+ * [G*G] differs from the one the previous step or reset wrote.  A step changes at most one cell.
+ *   record  = cell (bits 0-7; cell = r * G + c < G*G <= 225) | value << 8 (bits 8-10; 0..4)
+ *             | BENG_BUILDER_DELTA_CLEAR (bit 31); bits 11-30 are 0
+ *   applied = clear the whole row if bit 31 is set, then, if value != 0, write value to the cell.
+ *   A record is malformed when any of bits 11-30 is set, value > 4, value != 0 with cell >= G*G, or value == 0
+ *   with cell != 0.
+ * What the step kernel emits:
+ *   successful build            cell | building << 8  (the k-th empty cell, building 1..4)
+ *   pass, failed build (unaffordable or no empty cell), invalid action, end of episode without a reset
+ *                               BENG_BUILDER_DELTA_NONE (the row does not change)
+ *   any auto-reset              BENG_BUILDER_DELTA_CLEAR alone (a next-step reset at the start of the step, or a
+ *                               same-step reset after the terminal step, which also undoes that step's build) */
+#define BENG_BUILDER_DELTA_NONE 0x00000000u
+#define BENG_BUILDER_DELTA_CLEAR 0x80000000u
+
+/* beng_builder_step_host without the grid copy: enqueues H2D(actions) -> step kernel, which also writes one change
+ * record per env to delta_dev -> D2H(records[, resources, capacity, win_steps], reward, terminated) on `stream`.
+ * io->grid (and io->flat_obs when given) on the device is written exactly as by beng_builder_step.  A caller that
+ * holds a host copy of the grids from before this step brings it up to date with beng_builder_apply_obs_delta once
+ * the stream has drained: 33 B per env cross the bus instead of 129 B.  delta_dev / delta_host (uint32_t[n_envs],
+ * device / pinned host, 4-byte aligned) are required; NULL result host pointers are skipped.  Does not synchronise. */
+int beng_builder_step_host_delta(const beng_builder_params *p, const beng_builder_state *st, int64_t *actions_dev,
+                                 const beng_builder_io *io, int64_t n_envs, const int64_t *actions_host,
+                                 uint32_t *delta_dev, uint32_t *delta_host, float *resources_host, float *capacity_host,
+                                 int32_t *win_steps_host, float *reward_host, uint8_t *terminated_host, void *stream);
+
+/* Apply one step's change records (host memory, uint32_t[n_envs]) to a host copy of the grids (int8_t[n_envs][G][G]).
+ * Pure host code: touches no CUDA state and runs without a GPU.  The envs are split into contiguous chunks over
+ * n_threads threads (<= 0 means one), all joined before it returns.  Every record is checked before it is applied:
+ * BENG_ERR_BAD_ARG for NULL buffers, n_envs < 0 or a malformed record (grid_host is then partly updated, the row of
+ * the malformed record untouched), BENG_ERR_UNSUPPORTED for grid_size outside [2, 15]. */
+int beng_builder_apply_obs_delta(const uint32_t *delta_host, int8_t *grid_host, int64_t n_envs, int32_t grid_size,
+                                 int32_t n_threads);
+
 #ifdef __cplusplus
 }
 #endif

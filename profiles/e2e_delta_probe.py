@@ -1,13 +1,15 @@
-"""End-to-end rate of BatchedSnakeEnv.step_host with the full observation copy against delta_obs=True.
+"""End-to-end rate of step_host with the full observation copy against delta_obs=True.
 
-    python profiles/e2e_delta_probe.py [--blocks 6] [--out FILE]
+    python profiles/e2e_delta_probe.py [--env snake|builder] [--blocks 6] [--out FILE]
 
-Two envs with the same seed (G = 20, same_step auto-reset) are stepped from the same pinned host action tapes, built
-like bench.py's e2e tapes (beng_fill_random_actions on the device, then pinned host copies), in alternating timed
-blocks of the full path and the delta path within one process, after warm-up.  Every step is synchronous, as a caller
-of the numpy API sees it.  The delta path's time is split into the host apply (beng_snake_apply_obs_delta, timed
-around the call) and the rest (H2D actions, kernel, D2H of records and results, stream synchronise).  At the end the
-two envs' host observations and device observations must be equal.  Prints one JSON line; needs a CUDA GPU.
+--env snake (the default): BatchedSnakeEnv, G = 20.  --env builder: BatchedWorldBuilderEnv, G = 10, whose grid is the
+part of the observation that the delta path patches.  Two envs with the same seed (same_step auto-reset) are stepped
+from the same pinned host action tapes, built like bench.py's e2e tapes (beng_fill_random_actions on the device with
+the env's bench.py action count, then pinned host copies), in alternating timed blocks of the full path and the delta
+path within one process, after warm-up.  Every step is synchronous, as a caller of the numpy API sees it.  The delta
+path's time is split into the host apply (beng_<env>_apply_obs_delta, timed around the call) and the rest (H2D
+actions, kernel, D2H of records and results, stream synchronise).  At the end the two envs' host observations and
+device observations must be equal.  Prints one JSON line; needs a CUDA GPU.
 """
 from __future__ import annotations
 
@@ -28,20 +30,53 @@ import torch  # noqa: E402
 
 import bench  # noqa: E402  (pin_to_gpu_numa_node, pcie_ceiling: the same helpers as bench.py's e2e arm)
 
-G = 20
-RESULT_BYTES = 4 + 1 + 1 + 4 + 4  # reward, terminated, truncated, score, snake_length per env
 RECORD_BYTES = 4
 
 
-class TimedApply:
-    """Stands in for env.lib and accumulates the wall time spent in beng_snake_apply_obs_delta."""
+class Snake:  # the classes themselves are the specs (never instantiated): their functions are called on the class
+    probe = "snake step_host: full observation copy vs delta_obs=True"
+    G, n_choices, apply = 20, 4, "beng_snake_apply_obs_delta"
+    result_bytes = 4 + 1 + 1 + 4 + 4  # reward, terminated, truncated, score, snake_length per env
+    steps_per_block = {1 << 20: 25, 1 << 16: 200}
 
-    def __init__(self, lib):
-        self._lib, self.seconds, self.calls = lib, 0.0, 0
+    def make(pkg, n, dev):
+        return pkg.BatchedSnakeEnv(n, Snake.G, device=dev, seed=0, autoreset_mode="same_step")
+
+    def host_obs(out):
+        return out[0]
+
+    def device_obs(env):
+        return env.obs
+
+
+class Builder:
+    probe = "world-builder step_host: full grid copy vs delta_obs=True"
+    G, n_choices, apply = 10, 5, "beng_builder_apply_obs_delta"
+    result_bytes = 16 + 4 + 4 + 4 + 1  # resources, population_capacity, win_steps, reward, terminated per env
+    steps_per_block = {1 << 20: 100, 1 << 16: 1000}
+
+    def make(pkg, n, dev):
+        return pkg.BatchedWorldBuilderEnv(n, Builder.G, device=dev, seed=0, autoreset_mode="same_step")
+
+    def host_obs(out):
+        return out[0]["grid"]
+
+    def device_obs(env):
+        return env.grid
+
+
+ENVS = {"snake": Snake, "builder": Builder}
+
+
+class TimedApply:
+    """Stands in for env.lib and accumulates the wall time spent in the env's apply function."""
+
+    def __init__(self, lib, apply):
+        self._lib, self._apply, self.seconds, self.calls = lib, apply, 0.0, 0
 
     def __getattr__(self, name):
         fn = getattr(self._lib, name)
-        if name != "beng_snake_apply_obs_delta":
+        if name != self._apply:
             return fn
 
         def timed(*args):
@@ -60,17 +95,17 @@ def gpu_facts(index):
     return dict(zip(("gpu", "power_limit_w", "sm_clock_mhz", "sm_clock_max_mhz"), out))  # as nvidia-smi prints them
 
 
-def measure(pkg, n, blocks, steps_per_block, dev):
-    lib = pkg._lib.load()
-    envs = {k: pkg.BatchedSnakeEnv(n, G, device=dev, seed=0, autoreset_mode="same_step") for k in ("full", "delta")}
+def measure(pkg, spec, n, blocks, steps_per_block, dev):
+    lib, G = pkg._lib.load(), spec.G
+    envs = {k: spec.make(pkg, n, dev) for k in ("full", "delta")}
     for e in envs.values():
         e.reset()
-    timer = envs["delta"].lib = TimedApply(envs["delta"].lib)
+    timer = envs["delta"].lib = TimedApply(envs["delta"].lib, spec.apply)
     pool = 8
     tapes = torch.empty((pool, n), dtype=torch.int64, device=dev)
     stream = torch.cuda.current_stream(dev).cuda_stream
     for t in range(pool):
-        pkg._lib.check(lib.beng_fill_random_actions(tapes[t].data_ptr(), n, 1, 4, t, 0, 0, stream),
+        pkg._lib.check(lib.beng_fill_random_actions(tapes[t].data_ptr(), n, 1, spec.n_choices, t, 0, 0, stream),
                        "beng_fill_random_actions")
     host_tapes = [tapes[t].cpu().pin_memory() for t in range(pool)]
     cursor = {"full": 0, "delta": 0}
@@ -94,8 +129,9 @@ def measure(pkg, n, blocks, steps_per_block, dev):
             secs[kind].append(dt)
             if kind == "delta":
                 apply_s += timer.seconds - before
-            last[kind] = out[0]
-    equal = bool(np.array_equal(last["full"], last["delta"]) and torch.equal(envs["full"].obs, envs["delta"].obs))
+            last[kind] = spec.host_obs(out)
+    equal = bool(np.array_equal(last["full"], last["delta"])
+                 and torch.equal(spec.device_obs(envs["full"]), spec.device_obs(envs["delta"])))
     steps = blocks * steps_per_block
 
     def rates(kind):
@@ -106,8 +142,8 @@ def measure(pkg, n, blocks, steps_per_block, dev):
                                            "max": max(per_block)}}
 
     full, delta = rates("full"), rates("delta")
-    full.update(h2d_bytes_per_step=8 * n, d2h_bytes_per_step=n * (G * G + RESULT_BYTES))
-    delta.update(h2d_bytes_per_step=8 * n, d2h_bytes_per_step=n * (RECORD_BYTES + RESULT_BYTES),
+    full.update(h2d_bytes_per_step=8 * n, d2h_bytes_per_step=n * (G * G + spec.result_bytes))
+    delta.update(h2d_bytes_per_step=8 * n, d2h_bytes_per_step=n * (RECORD_BYTES + spec.result_bytes),
                  apply_ms_per_step=1e3 * apply_s / steps,
                  device_ms_per_step=1e3 * (sum(secs["delta"]) - apply_s) / steps,
                  device_note="H2D actions + step kernel + D2H records/results + stream synchronise, Python included")
@@ -123,6 +159,7 @@ def measure(pkg, n, blocks, steps_per_block, dev):
 
 def main():
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
+    ap.add_argument("--env", choices=sorted(ENVS), default="snake")
     ap.add_argument("--blocks", type=int, default=6)
     ap.add_argument("--out", default=None, help="also write the JSON line to this file")
     args = ap.parse_args()
@@ -130,12 +167,12 @@ def main():
         raise SystemExit("e2e_delta_probe.py measures the GPU path and needs a CUDA device")
     import custom_gymnasium_environments_b200 as pkg
 
+    spec = ENVS[args.env]
     dev = torch.device("cuda:0")
     numa_bound, _ = bench.pin_to_gpu_numa_node(0)
-    result = {"probe": "snake step_host: full observation copy vs delta_obs=True", "numa_bound": numa_bound,
-              "threads": len(os.sched_getaffinity(0)), "sizes": []}
-    for n, per_block in ((1 << 20, 25), (1 << 16, 200)):
-        result["sizes"].append(measure(pkg, n, args.blocks, per_block, dev))
+    result = {"probe": spec.probe, "numa_bound": numa_bound, "threads": len(os.sched_getaffinity(0)), "sizes": []}
+    for n, per_block in spec.steps_per_block.items():
+        result["sizes"].append(measure(pkg, spec, n, args.blocks, per_block, dev))
         if n == 1 << 20:
             result.update(gpu_facts(0))  # clocks read right after the large size's timed blocks
     line = json.dumps(result)
