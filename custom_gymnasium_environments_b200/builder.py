@@ -13,38 +13,38 @@ kept.  There is no time limit: an episode ends by starvation (-100) or after 50 
 from __future__ import annotations
 
 import ctypes as C
-import os
 
 import numpy as np
 import torch
 
 from . import _lib
 from .spaces import Box, Dict, Discrete, batch_space
-from .vector import _EnvBase, AUTORESET_MODES, _VectorEnvBase, _mode_name, as_device_actions, host_source, require_cuda, stream_ptr
+from .vector import _EnvBase, AUTORESET_MODES, _BatchedEnv, as_device_actions, host_source, stream_ptr
 
 BUILDING_NAMES = ("farm", "lumberyard", "quarry", "house")
 BUILDER_STAT_NAMES = ("n_episodes", "sum_return", "sum_length", "wins")
 MAX_POPULATION, WIN_STEPS = 20, 50
 
 
-class BatchedWorldBuilderEnv(_VectorEnvBase):
+class BatchedWorldBuilderEnv(_BatchedEnv):
     """N independent WorldBuilderEnv instances; scalar state as [word][env] int32, the grid doubles as observation."""
 
     metadata = {"render_modes": [], "render_fps": 4, "autoreset_mode": "same_step"}
+    _reset_fn = "beng_builder_reset"
+    _state_tensors = ("_words", "grid")
+    _stat_names = BUILDER_STAT_NAMES
+    _host_names = ("_actions", "grid", "resources", "population_capacity", "win_steps", "reward", "terminated",
+                   "_delta_dev")
+    _mirror, _apply_delta_fn = "grid", "beng_builder_apply_obs_delta"
 
     def __init__(self, num_envs: int, grid_size: int = 10, render_mode=None, flatten_obs: bool = False, *,
                  device="cuda", seed: int = 0, env_id_base: int = 0, autoreset_mode="same_step",
                  debug_checks: bool = False):
-        self.lib = _lib.load()
-        self.device = require_cuda(device)
-        self.num_envs = n = int(num_envs)
+        super().__init__(num_envs, device, autoreset_mode, render_mode)
+        n = self.num_envs
         self.grid_size = G = int(grid_size)
         self.flatten_obs = bool(flatten_obs)
-        self.render_mode = render_mode
         self.debug_checks = bool(debug_checks)
-        self.autoreset_mode = _mode_name(autoreset_mode)
-        self.metadata = dict(type(self).metadata, autoreset_mode=self.autoreset_mode)
-        self.closed = False
 
         self.single_action_space = Discrete(5)                                            # :60
         if self.flatten_obs:
@@ -80,11 +80,6 @@ class BatchedWorldBuilderEnv(_VectorEnvBase):
                                   self.reward.data_ptr(), self.terminated.data_ptr(), self.truncated.data_ptr(),
                                   self.ep_return.data_ptr(), self.ep_length.data_ptr(), self.stats.data_ptr(),
                                   self.invalid_count.data_ptr())
-        self._host = None
-        # True while the pinned host["grid"] equals the device grid: set by a full-copy step_host(), cleared by anything
-        # else that rewrites it.  step_host(delta_obs=True) patches the copy only while it is set.
-        self._grid_mirror_valid = False
-        self._needs_first_reset = True
 
     # ------------------------------------------------------------------ state views
     food = property(lambda self: self._words[0])
@@ -113,39 +108,17 @@ class BatchedWorldBuilderEnv(_VectorEnvBase):
                 "episode": {"r": self.ep_return, "l": self.ep_length}, "_episode": self.terminated}
 
     # ------------------------------------------------------------------ VectorEnv API
-    def reset(self, *, seed=None, options=None):
-        """WorldBuilderEnv.reset for every env (:99-123) -> (obs, infos); `seed` re-keys and rewinds the stream."""
-        first = self._needs_first_reset
-        if seed is not None:
-            self.params.seed = int(seed)
-            first = True
-        mask = None if not options else options.get("reset_mask")
-        mask_ptr = None
-        if mask is not None:
-            if self._needs_first_reset:
-                raise RuntimeError("the first reset() must reset every env")
-            mask = torch.as_tensor(mask).to(device=self.device, dtype=torch.uint8).contiguous()
-            if mask.shape != (self.num_envs,):
-                raise ValueError("reset_mask must have shape (num_envs,)")
-            mask_ptr = mask.data_ptr()
-        self._grid_mirror_valid = False
-        with torch.cuda.device(self.device):
-            rc = self.lib.beng_builder_reset(C.byref(self.params), C.byref(self._state), C.byref(self._io), mask_ptr,
-                                             self.num_envs, int(first), stream_ptr(self.device))
-        _lib.check(rc, "beng_builder_reset")
-        self._needs_first_reset = False
+    def _reset_result(self):
+        """WorldBuilderEnv.reset (:99-123) -> (obs, infos)."""
         return self._obs(), self._infos()
 
     def step(self, actions):
         """One step of every env (:125-166).  actions: int64 (n,), 0 pass / 1 farm / 2 lumberyard / 3 quarry / 4 house."""
-        if self._needs_first_reset:
-            raise RuntimeError("call reset() before step()")
+        self._require_reset()
         act = as_device_actions(actions, self._actions)
-        self._grid_mirror_valid = False
-        with torch.cuda.device(self.device):
-            rc = self.lib.beng_builder_step(C.byref(self.params), C.byref(self._state), act.data_ptr(),
-                                            C.byref(self._io), self.num_envs, stream_ptr(self.device))
-        _lib.check(rc, "beng_builder_step")
+        self._mirror_valid = False
+        self._call("beng_builder_step", C.byref(self.params), C.byref(self._state), act.data_ptr(), C.byref(self._io),
+                   self.num_envs, stream_ptr(self.device))
         if self.debug_checks:
             n_bad = int(self.invalid_count.item())
             if n_bad:
@@ -162,75 +135,23 @@ class BatchedWorldBuilderEnv(_VectorEnvBase):
         step_host(copy_obs=False) since the last step_host), the call copies the grid in full instead.  The returned
         obs['grid'] is read-only.  Needs sync=True and copy_obs=True.
         """
-        if delta_obs and not (sync and copy_obs):
-            raise ValueError("step_host(delta_obs=True) needs sync=True and copy_obs=True")
-        if self._needs_first_reset:
-            raise RuntimeError("call reset() before step()")
-        if self._host is None:
-            n, G = self.num_envs, self.grid_size
-            pin = dict(pin_memory=True)
-            self._host = {"actions": torch.zeros(n, dtype=torch.int64, **pin),
-                          "grid": torch.zeros((n, G, G), dtype=torch.int8, **pin),
-                          "resources": torch.zeros((n, 4), dtype=torch.float32, **pin),
-                          "capacity": torch.zeros((n, 1), dtype=torch.float32, **pin),
-                          "win_steps": torch.zeros((n, 1), dtype=torch.int32, **pin),
-                          "reward": torch.zeros(n, dtype=torch.float32, **pin),
-                          "terminated": torch.zeros(n, dtype=torch.bool, **pin),
-                          "delta": torch.zeros(n, dtype=torch.int32, **pin)}  # grid change records (uint32 bits)
-            self._delta_dev = torch.zeros(n, dtype=torch.int32, device=self.device)
-        h = self._host
-        src = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions))
-        src = self._host_src = host_source(src, h["actions"])
-        delta = delta_obs and self._grid_mirror_valid
-        self._grid_mirror_valid = False
-        results = (h["resources"].data_ptr(), h["capacity"].data_ptr(), h["win_steps"].data_ptr(),
+        delta = self._mirror_begin(delta_obs, sync, copy_obs)
+        h = self._host_buffers()
+        src = self._host_src = host_source(actions, h["_actions"])
+        head = (C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._io),
+                self.num_envs, src.data_ptr())
+        results = (h["resources"].data_ptr(), h["population_capacity"].data_ptr(), h["win_steps"].data_ptr(),
                    h["reward"].data_ptr(), h["terminated"].data_ptr(), stream_ptr(self.device))
-        with torch.cuda.device(self.device):
-            if delta:
-                rc = self.lib.beng_builder_step_host_delta(
-                    C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._io),
-                    self.num_envs, src.data_ptr(), self._delta_dev.data_ptr(), h["delta"].data_ptr(), *results)
-                _lib.check(rc, "beng_builder_step_host_delta")
-            else:
-                rc = self.lib.beng_builder_step_host(
-                    C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._io),
-                    self.num_envs, src.data_ptr(), h["grid"].data_ptr() if copy_obs else None, *results)
-                _lib.check(rc, "beng_builder_step_host")
-            if sync:
-                torch.cuda.current_stream(self.device).synchronize()
         if delta:
-            rc = self.lib.beng_builder_apply_obs_delta(h["delta"].data_ptr(), h["grid"].data_ptr(), self.num_envs,
-                                                       self.grid_size, len(os.sched_getaffinity(0)))
-            _lib.check(rc, "beng_builder_apply_obs_delta")
-        self._grid_mirror_valid = copy_obs
-        grid = h["grid"].numpy() if copy_obs else self.grid
-        if delta_obs:
-            grid = grid.view()
-            grid.flags.writeable = False  # the mirror of the next delta step
-        obs = {"grid": grid, "resources": h["resources"].numpy(),
-               "population_capacity": h["capacity"].numpy(), "win_steps": h["win_steps"].numpy()}
+            self._call("beng_builder_step_host_delta", *head, self._delta_dev.data_ptr(), h["_delta_dev"].data_ptr(),
+                       *results)
+        else:
+            self._call("beng_builder_step_host", *head, h["grid"].data_ptr() if copy_obs else None, *results)
+        if sync:
+            self._sync()
+        obs = {"grid": self._mirror_end(delta, delta_obs, copy_obs), "resources": h["resources"].numpy(),
+               "population_capacity": h["population_capacity"].numpy(), "win_steps": h["win_steps"].numpy()}
         return obs, h["reward"].numpy(), h["terminated"].numpy(), np.zeros(self.num_envs, dtype=bool), {}
-
-    def episode_stats(self) -> dict:
-        return dict(zip(BUILDER_STAT_NAMES, self.stats.tolist()))
-
-    def state_dict(self) -> dict:
-        return {"words": self._words.clone(), "grid": self.grid.clone(), "stats": self.stats.clone(),
-                "seed": int(self.params.seed), "env_id_base": int(self.params.env_id_base)}
-
-    def load_state_dict(self, sd: dict):
-        self._words.copy_(sd["words"])
-        self.grid.copy_(sd["grid"])
-        self.stats.copy_(sd["stats"])
-        self.params.seed, self.params.env_id_base = int(sd["seed"]), int(sd["env_id_base"])
-        self._grid_mirror_valid = False
-        self._needs_first_reset = False
-
-    def render(self):
-        return None  # pygame rendering is out of scope (SURVEY.md section 2)
-
-    def close(self, **kwargs):
-        self.closed = True
 
 
 class WorldBuilderEnv(_EnvBase):

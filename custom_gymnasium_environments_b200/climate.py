@@ -18,30 +18,34 @@ import torch
 
 from . import _lib
 from .spaces import Box, Dict, MultiBinary, batch_space
-from .vector import _EnvBase, AUTORESET_MODES, _VectorEnvBase, _mode_name, host_source, require_cuda, stream_ptr
+from .vector import _EnvBase, AUTORESET_MODES, _BatchedEnv, as_device_actions, host_source, stream_ptr
 
 OBS_DIM = 9
 CLIMATE_STAT_NAMES = ("n_episodes", "sum_return", "sum_length")
 
 
-class BatchedSmartClimateEnv(_VectorEnvBase):
+def _shaped(x, shape):
+    """An action component (tensor, array or list) reshaped to `shape`."""
+    return x.reshape(shape) if isinstance(x, torch.Tensor) else np.reshape(x, shape)
+
+
+class BatchedSmartClimateEnv(_BatchedEnv):
     """N independent SmartClimateEnv instances; state resident in HBM as [field][env] arrays."""
 
     metadata = {"render_modes": [], "render_fps": 10, "autoreset_mode": "same_step"}
+    _reset_fn = "beng_climate_reset"
+    _state_tensors = ("_f64", "_i32")
+    _stat_names = CLIMATE_STAT_NAMES
+    _host_names = ("_ac", "_lights", "obs", "reward", "terminated", "truncated")
 
     def __init__(self, num_envs: int, max_occupancy: int = 8, comfort_temp_range=(20.0, 24.0),
                  episode_minutes: int = 1440, *, device="cuda", seed: int = 0, env_id_base: int = 0,
                  autoreset_mode="same_step", time_limit_truncation: bool = False, render_mode=None):
-        self.lib = _lib.load()
-        self.device = require_cuda(device)
-        self.num_envs = n = int(num_envs)
+        super().__init__(num_envs, device, autoreset_mode, render_mode)
+        n = self.num_envs
         self.max_occupancy = int(max_occupancy)
         self.comfort_temp_range = tuple(comfort_temp_range)  # kept for API parity; unused by the reference's dynamics
         self.episode_minutes = int(episode_minutes)
-        self.render_mode = render_mode
-        self.autoreset_mode = _mode_name(autoreset_mode)
-        self.metadata = dict(type(self).metadata, autoreset_mode=self.autoreset_mode)
-        self.closed = False
 
         self.single_action_space = Dict({"ac_temp": Box(16.0, 32.0, (1,), np.float32), "lights": MultiBinary(4)})
         self.single_observation_space = Box(
@@ -73,8 +77,6 @@ class BatchedSmartClimateEnv(_VectorEnvBase):
         self._io = _lib.ClimateIO(self.obs.data_ptr(), self.reward.data_ptr(), self.terminated.data_ptr(),
                                   self.truncated.data_ptr(), self.reward64.data_ptr(), self.reward_terms.data_ptr(),
                                   self.ep_return.data_ptr(), self.ep_length.data_ptr(), self.stats.data_ptr())
-        self._host = None
-        self._needs_first_reset = True
 
     # ------------------------------------------------------------------ state views
     room_temp = property(lambda self: self._f64[0])
@@ -94,112 +96,35 @@ class BatchedSmartClimateEnv(_VectorEnvBase):
                 "episode": {"r": self.ep_return, "l": self.ep_length}, "_episode": self.terminated}
 
     # ------------------------------------------------------------------ VectorEnv API
-    def reset(self, *, seed=None, options=None):
-        """SmartClimateEnv.reset for every env (env.py:62-70) -> (obs, infos); `seed` re-keys and rewinds the stream."""
-        first = self._needs_first_reset
-        if seed is not None:
-            self.params.seed = int(seed)
-            first = True
-        mask = None if not options else options.get("reset_mask")
-        mask_ptr = None
-        if mask is not None:
-            if self._needs_first_reset:
-                raise RuntimeError("the first reset() must reset every env")
-            mask = torch.as_tensor(mask).to(device=self.device, dtype=torch.uint8).contiguous()
-            if mask.shape != (self.num_envs,):
-                raise ValueError("reset_mask must have shape (num_envs,)")
-            mask_ptr = mask.data_ptr()
-        with torch.cuda.device(self.device):
-            rc = self.lib.beng_climate_reset(C.byref(self.params), C.byref(self._state), C.byref(self._io), mask_ptr,
-                                             self.num_envs, int(first), stream_ptr(self.device))
-        _lib.check(rc, "beng_climate_reset")
-        self._needs_first_reset = False
-        return self.obs, {}
-
-    def _split_action(self, actions):
-        if isinstance(actions, dict):
-            ac, lights = actions["ac_temp"], actions["lights"]
-        else:
-            ac, lights = actions
-        return ac, lights
-
-    def _to_device(self, value, buf):
-        if isinstance(value, torch.Tensor):
-            if value.device == buf.device and value.dtype == buf.dtype and value.is_contiguous() \
-                    and value.numel() == buf.numel() and value.data_ptr() % 16 == 0:  # (a misaligned view goes through buf)
-                return value
-            buf.copy_(value.reshape(buf.shape), non_blocking=True)
-            return buf
-        arr = np.asarray(value)
-        if arr.size != buf.numel():
-            raise ValueError(f"action component must have {buf.numel()} elements, got shape {arr.shape}")
-        buf.copy_(torch.from_numpy(np.ascontiguousarray(arr).reshape(tuple(buf.shape))).to(buf.dtype))
-        return buf
+    # reset(): SmartClimateEnv.reset (env.py:62-70).
 
     def step(self, actions):
         """One step of every env (env.py:84-117).  actions = {'ac_temp': float32 (n,1)|(n,), 'lights': int8 (n,4)}."""
-        if self._needs_first_reset:
-            raise RuntimeError("call reset() before step()")
-        ac, lights = self._split_action(actions)
-        ac_t, li_t = self._to_device(ac, self._ac), self._to_device(lights, self._lights)
-        with torch.cuda.device(self.device):
-            rc = self.lib.beng_climate_step(C.byref(self.params), C.byref(self._state), ac_t.data_ptr(),
-                                            li_t.data_ptr(), C.byref(self._io), self.num_envs,
-                                            stream_ptr(self.device))
-        _lib.check(rc, "beng_climate_step")
+        self._require_reset()
+        n = self.num_envs
+        ac, lights = (actions["ac_temp"], actions["lights"]) if isinstance(actions, dict) else actions
+        # (n,) / (n, 4) tensors, the usual case, go straight to the upload: no call or torch op per step for them
+        ac = ac if isinstance(ac, torch.Tensor) and ac.ndim == 1 else _shaped(ac, (n,))
+        lights = lights if isinstance(lights, torch.Tensor) and lights.ndim == 2 else _shaped(lights, (n, 4))
+        ac, lights = as_device_actions(ac, self._ac), as_device_actions(lights, self._lights)
+        self._call("beng_climate_step", C.byref(self.params), C.byref(self._state), ac.data_ptr(), lights.data_ptr(),
+                   C.byref(self._io), self.num_envs, stream_ptr(self.device))
         return self.obs, self.reward, self.terminated, self.truncated, self._infos()
 
     def step_host(self, actions, *, copy_obs: bool = True, sync: bool = True):
         """step() for callers holding HOST arrays (numpy in, numpy out) through `beng_climate_step_host`."""
-        if self._needs_first_reset:
-            raise RuntimeError("call reset() before step()")
-        if self._host is None:
-            n = self.num_envs
-            pin = dict(pin_memory=True)
-            self._host = {"ac": torch.zeros(n, dtype=torch.float32, **pin),
-                          "lights": torch.zeros((n, 4), dtype=torch.int8, **pin),
-                          "obs": torch.zeros((n, OBS_DIM), dtype=torch.float32, **pin),
-                          "reward": torch.zeros(n, dtype=torch.float32, **pin),
-                          "terminated": torch.zeros(n, dtype=torch.bool, **pin),
-                          "truncated": torch.zeros(n, dtype=torch.bool, **pin)}
-        h = self._host
-        ac, lights = self._split_action(actions)
-        ac_src = ac if isinstance(ac, torch.Tensor) else torch.as_tensor(np.asarray(ac, dtype=np.float32))
-        li_src = lights if isinstance(lights, torch.Tensor) else torch.as_tensor(np.asarray(lights, dtype=np.int8))
-        ac_src = host_source(ac_src, h["ac"])
-        li_src = host_source(li_src, h["lights"])
-        self._host_src = (ac_src, li_src)
-        with torch.cuda.device(self.device):
-            rc = self.lib.beng_climate_step_host(
-                C.byref(self.params), C.byref(self._state), self._ac.data_ptr(), self._lights.data_ptr(),
-                C.byref(self._io), self.num_envs, ac_src.data_ptr(), li_src.data_ptr(),
-                h["obs"].data_ptr() if copy_obs else None, h["reward"].data_ptr(), h["terminated"].data_ptr(),
-                h["truncated"].data_ptr(), stream_ptr(self.device))
-            _lib.check(rc, "beng_climate_step_host")
-            if sync:
-                torch.cuda.current_stream(self.device).synchronize()
+        self._require_reset()
+        h = self._host_buffers()
+        ac, lights = (actions["ac_temp"], actions["lights"]) if isinstance(actions, dict) else actions
+        ac, lights = self._host_src = (host_source(ac, h["_ac"]), host_source(lights, h["_lights"]))
+        self._call("beng_climate_step_host", C.byref(self.params), C.byref(self._state), self._ac.data_ptr(),
+                   self._lights.data_ptr(), C.byref(self._io), self.num_envs, ac.data_ptr(), lights.data_ptr(),
+                   h["obs"].data_ptr() if copy_obs else None, h["reward"].data_ptr(), h["terminated"].data_ptr(),
+                   h["truncated"].data_ptr(), stream_ptr(self.device))
+        if sync:
+            self._sync()
         obs = h["obs"].numpy() if copy_obs else self.obs
         return obs, h["reward"].numpy(), h["terminated"].numpy(), h["truncated"].numpy(), {}
-
-    def episode_stats(self) -> dict:
-        return dict(zip(CLIMATE_STAT_NAMES, self.stats.tolist()))
-
-    def state_dict(self) -> dict:
-        return {"f64": self._f64.clone(), "i32": self._i32.clone(), "stats": self.stats.clone(),
-                "seed": int(self.params.seed), "env_id_base": int(self.params.env_id_base)}
-
-    def load_state_dict(self, sd: dict):
-        self._f64.copy_(sd["f64"])
-        self._i32.copy_(sd["i32"])
-        self.stats.copy_(sd["stats"])
-        self.params.seed, self.params.env_id_base = int(sd["seed"]), int(sd["env_id_base"])
-        self._needs_first_reset = False
-
-    def render(self):
-        return None  # matplotlib visualiser is out of scope (SURVEY.md section 2)
-
-    def close(self, **kwargs):
-        self.closed = True
 
 
 class SmartClimateEnv(_EnvBase):

@@ -22,7 +22,7 @@ import torch
 
 from . import _lib
 from .spaces import Box, Discrete, batch_space
-from .vector import _EnvBase, AUTORESET_MODES, LazyInfos as _LazyInfos, _VectorEnvBase, _mode_name, host_source, require_cuda, stream_ptr
+from .vector import _EnvBase, AUTORESET_MODES, LazyInfos as _LazyInfos, _BatchedEnv, as_device_actions, host_source, stream_ptr
 
 HISTORY = 50
 OBS_DIM = 261
@@ -43,29 +43,28 @@ class TradingConfig:
     market_psychology_factor: float = 0.1
 
 
-class BatchedCryptoTradingEnv(_VectorEnvBase):
+class BatchedCryptoTradingEnv(_BatchedEnv):
     """N independent CryptoTradingEnv instances; state resident in HBM as [field][env] arrays."""
 
     metadata = {"render_modes": [], "render_fps": 30, "autoreset_mode": "same_step"}
+    _reset_fn = "beng_crypto_reset"
+    _state_tensors = ("_scal", "_meta", "_ep_return", "_close", "_ohlv")
+    _stat_names = CRYPTO_STAT_NAMES
+    _host_names = ("_actions", "obs", "reward", "terminated", "truncated")
 
     def __init__(self, num_envs: int, config: TradingConfig | None = None, action_type: str = "continuous",
                  render_mode=None, *, device="cuda", seed: int = 0, env_id_base: int = 0,
                  autoreset_mode="same_step", max_steps: int = 1000, info_outputs: bool = True,
                  time_limit_truncation: bool = False):
-        self.lib = _lib.load()
-        self.device = require_cuda(device)
-        self.num_envs = n = int(num_envs)
+        super().__init__(num_envs, device, autoreset_mode, render_mode)
+        n = self.num_envs
         self.config = config or TradingConfig()
         if self.config.history_length != HISTORY:
             raise ValueError("history_length is fixed at 50 in the CUDA engine")
         if action_type not in ("continuous", "discrete"):
             raise ValueError("action_type must be 'continuous' or 'discrete'")
         self.action_type = action_type
-        self.render_mode = render_mode
         self.max_steps = int(max_steps)
-        self.autoreset_mode = _mode_name(autoreset_mode)
-        self.metadata = dict(type(self).metadata, autoreset_mode=self.autoreset_mode)
-        self.closed = False
 
         # the reference declares (260,) but returns 261 values; the spaces here describe what is returned
         self.single_observation_space = Box(-np.inf, np.inf, (OBS_DIM,), np.float32)
@@ -111,9 +110,7 @@ class BatchedCryptoTradingEnv(_VectorEnvBase):
                                  self.truncated.data_ptr(), ptr(self.reward64), ptr(self.portfolio_value),
                                  ptr(self.current_price), ptr(self.trade_kind), self.ep_return.data_ptr(),
                                  self.ep_length.data_ptr(), self.stats.data_ptr())
-        self._host = None
         self._info_cache = None
-        self._needs_first_reset = True
 
     # ------------------------------------------------------------------ state views
     @property
@@ -168,110 +165,42 @@ class BatchedCryptoTradingEnv(_VectorEnvBase):
         return self._info_cache
 
     # ------------------------------------------------------------------ VectorEnv API
-    def reset(self, *, seed=None, options=None):
-        """CryptoTradingEnv.reset for every env (:301-340) -> (obs, infos).  `seed` re-keys and rewinds the
-        counter-based stream and re-creates the market simulators (the reference seeds both global RNGs, :305-307).
-        options={"reset_mask": bool tensor} resets only the selected envs."""
-        first = self._needs_first_reset
-        if seed is not None:
-            self.params.seed = int(seed)
-            first = True
-        mask = None if not options else options.get("reset_mask")
-        mask_ptr = None
-        if mask is not None:
-            if self._needs_first_reset:
-                raise RuntimeError("the first reset() must reset every env")
-            mask = torch.as_tensor(mask).to(device=self.device, dtype=torch.uint8).contiguous()
-            if mask.shape != (self.num_envs,):
-                raise ValueError("reset_mask must have shape (num_envs,)")
-            mask_ptr = mask.data_ptr()
-        with torch.cuda.device(self.device):
-            rc = self.lib.beng_crypto_reset(C.byref(self.params), C.byref(self._state), C.byref(self._io), mask_ptr,
-                                            self.num_envs, int(first), stream_ptr(self.device))
-        _lib.check(rc, "beng_crypto_reset")
-        self._needs_first_reset = False
-        return self.obs, {}
-
-    def _device_actions(self, actions):
-        buf = self._actions
-        if isinstance(actions, torch.Tensor):
-            if actions.device == buf.device and actions.dtype == buf.dtype and actions.is_contiguous() \
-                    and actions.shape == buf.shape and actions.data_ptr() % 16 == 0:
-                return actions
-            buf.copy_(actions.reshape(buf.shape), non_blocking=True)
-            return buf
-        arr = np.asarray(actions)
-        if arr.shape != tuple(buf.shape):
-            raise ValueError(f"actions must have shape {tuple(buf.shape)}, got {arr.shape}")
-        buf.copy_(torch.from_numpy(np.ascontiguousarray(arr)).to(buf.dtype))
-        return buf
+    # reset(): CryptoTradingEnv.reset (:301-340).  `seed` also re-creates the market simulators (the reference seeds
+    # both global RNGs, :305-307).
 
     def step(self, actions):
         """One step of every env (:342-398) -> (obs, rewards, terminations, truncations, infos).
         Discrete: int64 (n,) with 0=hold 1=buy 5% 2=buy 20% 3=sell 5% 4=sell 20% (anything else holds, like the
         reference).  Continuous: float32 (n, 2) = [buy, sell], clipped to [0, 1] x 10 % caps (:408-422)."""
-        if self._needs_first_reset:
-            raise RuntimeError("call reset() before step()")
-        act = self._device_actions(actions)
-        with torch.cuda.device(self.device):
-            rc = self.lib.beng_crypto_step(C.byref(self.params), C.byref(self._state), act.data_ptr(),
-                                           C.byref(self._io), self.num_envs, stream_ptr(self.device))
-        _lib.check(rc, "beng_crypto_step")
+        self._require_reset()
+        act = as_device_actions(actions, self._actions)
+        self._call("beng_crypto_step", C.byref(self.params), C.byref(self._state), act.data_ptr(), C.byref(self._io),
+                   self.num_envs, stream_ptr(self.device))
         self.params.window_head = (self.params.window_head + 1) % HISTORY
         return self.obs, self.reward, self.terminated, self.truncated, self._infos()
 
     def step_host(self, actions, *, copy_obs: bool = True, sync: bool = True):
         """step() for callers holding HOST arrays (numpy in, numpy out) through `beng_crypto_step_host`."""
-        if self._needs_first_reset:
-            raise RuntimeError("call reset() before step()")
-        if self._host is None:
-            n = self.num_envs
-            pin = dict(pin_memory=True)
-            self._host = {"actions": torch.zeros_like(self._actions, device="cpu", **pin),
-                          "obs": torch.zeros((n, OBS_DIM), dtype=torch.float32, **pin),
-                          "reward": torch.zeros(n, dtype=torch.float32, **pin),
-                          "terminated": torch.zeros(n, dtype=torch.bool, **pin),
-                          "truncated": torch.zeros(n, dtype=torch.bool, **pin)}
-        h = self._host
-        src = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions))
-        src = self._host_src = host_source(src, h["actions"])
-        with torch.cuda.device(self.device):
-            rc = self.lib.beng_crypto_step_host(
-                C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._io),
-                self.num_envs, src.data_ptr(), h["obs"].data_ptr() if copy_obs else None,
-                h["reward"].data_ptr(), h["terminated"].data_ptr(), h["truncated"].data_ptr(),
-                stream_ptr(self.device))
-            _lib.check(rc, "beng_crypto_step_host")
-            self.params.window_head = (self.params.window_head + 1) % HISTORY
-            if sync:
-                torch.cuda.current_stream(self.device).synchronize()
+        self._require_reset()
+        h = self._host_buffers()
+        src = self._host_src = host_source(actions, h["_actions"])
+        self._call("beng_crypto_step_host", C.byref(self.params), C.byref(self._state), self._actions.data_ptr(),
+                   C.byref(self._io), self.num_envs, src.data_ptr(), h["obs"].data_ptr() if copy_obs else None,
+                   h["reward"].data_ptr(), h["terminated"].data_ptr(), h["truncated"].data_ptr(),
+                   stream_ptr(self.device))
+        self.params.window_head = (self.params.window_head + 1) % HISTORY
+        if sync:
+            self._sync()
         obs = h["obs"].numpy() if copy_obs else self.obs
         return obs, h["reward"].numpy(), h["terminated"].numpy(), h["truncated"].numpy(), {}
 
     # ------------------------------------------------------------------ extras
-    def episode_stats(self) -> dict:
-        return dict(zip(CRYPTO_STAT_NAMES, self.stats.tolist()))
-
     def state_dict(self) -> dict:
-        return {"scal": self._scal.clone(), "meta": self._meta.clone(), "ep_return": self._ep_return.clone(),
-                "close": self._close.clone(), "ohlv": self._ohlv.clone(), "stats": self.stats.clone(),
-                "window_head": int(self.params.window_head), "seed": int(self.params.seed),
-                "env_id_base": int(self.params.env_id_base), "config": asdict(self.config)}
+        return dict(super().state_dict(), window_head=int(self.params.window_head), config=asdict(self.config))
 
     def load_state_dict(self, sd: dict):
-        for name in ("scal", "meta", "ep_return", "close", "ohlv"):
-            getattr(self, "_" + name).copy_(sd[name])
-        self.stats.copy_(sd["stats"])
+        super().load_state_dict(sd)
         self.params.window_head = int(sd["window_head"])
-        self.params.seed = int(sd["seed"])
-        self.params.env_id_base = int(sd["env_id_base"])
-        self._needs_first_reset = False
-
-    def render(self):
-        return None  # pygame/matplotlib rendering is out of scope (SURVEY.md section 2)
-
-    def close(self, **kwargs):
-        self.closed = True
 
 
 class CryptoTradingEnv(_EnvBase):

@@ -345,6 +345,31 @@ int step(const beng_builder_params *p, const beng_builder_state *st, const int64
     return delta ? launch<false, true>(a, stream) : launch<false>(a, stream);
 }
 
+// The body of beng_builder_step_host (delta_dev / delta_host null) and beng_builder_step_host_delta (grid_host null):
+// H2D(actions) -> step kernel (the DELTA one when delta_dev is set) -> D2H of the change records, the results and the
+// grid, each skipped when its host pointer is null.
+int step_host(const beng_builder_params *p, const beng_builder_state *st, int64_t *actions_dev,
+              const beng_builder_io *io, int64_t n_envs, const int64_t *actions_host, uint32_t *delta_dev,
+              uint32_t *delta_host, int8_t *grid_host, float *resources_host, float *capacity_host,
+              int32_t *win_steps_host, float *reward_host, uint8_t *terminated_host, cudaStream_t s) {
+    if (!actions_host || !actions_dev) return BENG_ERR_BAD_ARG;
+    if (int rc = check(p, st, io, n_envs)) return rc;
+    if ((resources_host && !io->resources) || (capacity_host && !io->capacity) || (win_steps_host && !io->win_steps))
+        return BENG_ERR_BAD_ARG;
+    if (n_envs == 0) return 0;
+    const size_t n = (size_t)n_envs, cells = (size_t)p->grid_size * p->grid_size;
+    cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, n * sizeof(int64_t), cudaMemcpyHostToDevice, s);
+    if (e != cudaSuccess) return (int)e;
+    if (int rc = step(p, st, actions_dev, io, n_envs, delta_dev, s)) return rc;
+    if (int rc = d2h(delta_host, delta_dev, n * sizeof(uint32_t), s)) return rc;
+    if (int rc = d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
+    if (int rc = d2h(terminated_host, io->terminated, n, s)) return rc;
+    if (int rc = d2h(resources_host, io->resources, n * 4 * sizeof(float), s)) return rc;
+    if (int rc = d2h(capacity_host, io->capacity, n * sizeof(float), s)) return rc;
+    if (int rc = d2h(win_steps_host, io->win_steps, n * sizeof(int32_t), s)) return rc;
+    return d2h(grid_host, io->grid, n * cells, s);
+}
+
 // Applies the records of envs [begin, end); false on a malformed record (its row and the rest of the range are left
 // as they are).
 bool apply_delta_range(const uint32_t *delta, int8_t *grid, int64_t begin, int64_t end, uint32_t cells) {
@@ -382,45 +407,18 @@ int beng_builder_step_host(const beng_builder_params *p, const beng_builder_stat
                            const beng_builder_io *io, int64_t n_envs, const int64_t *actions_host, int8_t *grid_host,
                            float *resources_host, float *capacity_host, int32_t *win_steps_host, float *reward_host,
                            uint8_t *terminated_host, void *stream) {
-    if (!actions_host || !actions_dev) return BENG_ERR_BAD_ARG;
-    if (int rc = beng::check(p, st, io, n_envs)) return rc;
-    if ((resources_host && !io->resources) || (capacity_host && !io->capacity) || (win_steps_host && !io->win_steps))
-        return BENG_ERR_BAD_ARG;
-    if (n_envs == 0) return 0;
-    cudaStream_t s = (cudaStream_t)stream;
-    const size_t n = (size_t)n_envs, cells = (size_t)p->grid_size * p->grid_size;
-    cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, n * sizeof(int64_t), cudaMemcpyHostToDevice, s);
-    if (e != cudaSuccess) return (int)e;
-    if (int rc = beng_builder_step(p, st, actions_dev, io, n_envs, stream)) return rc;
-    if (int rc = beng::d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
-    if (int rc = beng::d2h(terminated_host, io->terminated, n, s)) return rc;
-    if (int rc = beng::d2h(resources_host, io->resources, n * 4 * sizeof(float), s)) return rc;
-    if (int rc = beng::d2h(capacity_host, io->capacity, n * sizeof(float), s)) return rc;
-    if (int rc = beng::d2h(win_steps_host, io->win_steps, n * sizeof(int32_t), s)) return rc;
-    return beng::d2h(grid_host, io->grid, n * cells, s);
+    return beng::step_host(p, st, actions_dev, io, n_envs, actions_host, nullptr, nullptr, grid_host, resources_host,
+                           capacity_host, win_steps_host, reward_host, terminated_host, (cudaStream_t)stream);
 }
 
 int beng_builder_step_host_delta(const beng_builder_params *p, const beng_builder_state *st, int64_t *actions_dev,
                                  const beng_builder_io *io, int64_t n_envs, const int64_t *actions_host,
                                  uint32_t *delta_dev, uint32_t *delta_host, float *resources_host, float *capacity_host,
                                  int32_t *win_steps_host, float *reward_host, uint8_t *terminated_host, void *stream) {
-    if (!actions_host || !actions_dev || !delta_dev || !delta_host) return BENG_ERR_BAD_ARG;
-    if (((uintptr_t)delta_dev & 3) || ((uintptr_t)delta_host & 3)) return BENG_ERR_BAD_ARG;
-    if (int rc = beng::check(p, st, io, n_envs)) return rc;
-    if ((resources_host && !io->resources) || (capacity_host && !io->capacity) || (win_steps_host && !io->win_steps))
-        return BENG_ERR_BAD_ARG;
-    if (n_envs == 0) return 0;
-    cudaStream_t s = (cudaStream_t)stream;
-    const size_t n = (size_t)n_envs;
-    cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, n * sizeof(int64_t), cudaMemcpyHostToDevice, s);
-    if (e != cudaSuccess) return (int)e;
-    if (int rc = beng::step(p, st, actions_dev, io, n_envs, delta_dev, s)) return rc;
-    if (int rc = beng::d2h(delta_host, delta_dev, n * sizeof(uint32_t), s)) return rc;
-    if (int rc = beng::d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
-    if (int rc = beng::d2h(terminated_host, io->terminated, n, s)) return rc;
-    if (int rc = beng::d2h(resources_host, io->resources, n * 4 * sizeof(float), s)) return rc;
-    if (int rc = beng::d2h(capacity_host, io->capacity, n * sizeof(float), s)) return rc;
-    return beng::d2h(win_steps_host, io->win_steps, n * sizeof(int32_t), s);
+    if (!delta_dev || !delta_host || ((uintptr_t)delta_dev & 3) || ((uintptr_t)delta_host & 3)) return BENG_ERR_BAD_ARG;
+    return beng::step_host(p, st, actions_dev, io, n_envs, actions_host, delta_dev, delta_host, nullptr,
+                           resources_host, capacity_host, win_steps_host, reward_host, terminated_host,
+                           (cudaStream_t)stream);
 }
 
 int beng_builder_apply_obs_delta(const uint32_t *delta_host, int8_t *grid_host, int64_t n_envs, int32_t grid_size,

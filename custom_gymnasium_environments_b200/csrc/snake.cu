@@ -572,6 +572,31 @@ int step(const beng_snake_params *p, const beng_snake_state *st, const int64_t *
     return launch<false>(a, stream);
 }
 
+// The body of beng_snake_step_host (delta_dev / delta_host null) and beng_snake_step_host_delta (obs_host null):
+// H2D(actions) -> step kernel (the DELTA one when delta_dev is set) -> D2H of the change records, the results and the
+// observations, each skipped when its host pointer is null.
+int step_host(const beng_snake_params *p, const beng_snake_state *st, int64_t *actions_dev, const beng_snake_io *io,
+              int64_t n_envs, const int64_t *actions_host, uint32_t *delta_dev, uint32_t *delta_host, int8_t *obs_host,
+              float *reward_host, uint8_t *terminated_host, uint8_t *truncated_host, int32_t *score_host,
+              int32_t *snake_length_host, cudaStream_t s) {
+    if (!actions_host || !actions_dev) return BENG_ERR_BAD_ARG;
+    if (int rc = check_common(p, st, io, n_envs)) return rc;
+    if ((truncated_host && !io->truncated) || (score_host && !io->score) || (snake_length_host && !io->snake_length))
+        return BENG_ERR_BAD_ARG;
+    if (n_envs == 0) return 0;
+    const size_t n = (size_t)n_envs, cells = (size_t)p->grid_size * p->grid_size;
+    cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, n * sizeof(int64_t), cudaMemcpyHostToDevice, s);
+    if (e != cudaSuccess) return (int)e;
+    if (int rc = step(p, st, actions_dev, io, n_envs, delta_dev, s)) return rc;
+    if (int rc = d2h(delta_host, delta_dev, n * sizeof(uint32_t), s)) return rc;
+    if (int rc = d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
+    if (int rc = d2h(terminated_host, io->terminated, n, s)) return rc;
+    if (int rc = d2h(truncated_host, io->truncated, n, s)) return rc;
+    if (int rc = d2h(score_host, io->score, n * sizeof(int32_t), s)) return rc;
+    if (int rc = d2h(snake_length_host, io->snake_length, n * sizeof(int32_t), s)) return rc;
+    return d2h(obs_host, io->obs, n * cells, s);
+}
+
 // Applies the records of envs [begin, end); false on a malformed record (the rest of the range is left as it is).
 bool apply_delta_range(const uint32_t *delta, int8_t *obs, int64_t begin, int64_t end, int cells) {
     for (int64_t e = begin; e < end; ++e) {
@@ -629,45 +654,17 @@ int beng_snake_step_host(const beng_snake_params *p, const beng_snake_state *st,
                          const beng_snake_io *io, int64_t n_envs, const int64_t *actions_host, int8_t *obs_host,
                          float *reward_host, uint8_t *terminated_host, uint8_t *truncated_host, int32_t *score_host,
                          int32_t *snake_length_host, void *stream) {
-    if (!actions_host || !actions_dev) return BENG_ERR_BAD_ARG;
-    if (int rc = beng::check_common(p, st, io, n_envs)) return rc;
-    if ((truncated_host && !io->truncated) || (score_host && !io->score) || (snake_length_host && !io->snake_length))
-        return BENG_ERR_BAD_ARG;
-    if (n_envs == 0) return 0;
-    cudaStream_t s = (cudaStream_t)stream;
-    const size_t n = (size_t)n_envs, cells = (size_t)p->grid_size * p->grid_size;
-    cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, n * sizeof(int64_t), cudaMemcpyHostToDevice, s);
-    if (e != cudaSuccess) return (int)e;
-    if (int rc = beng_snake_step(p, st, actions_dev, io, n_envs, stream)) return rc;
-    if (int rc = beng::d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
-    if (int rc = beng::d2h(terminated_host, io->terminated, n, s)) return rc;
-    if (int rc = beng::d2h(truncated_host, io->truncated, n, s)) return rc;
-    if (int rc = beng::d2h(score_host, io->score, n * sizeof(int32_t), s)) return rc;
-    if (int rc = beng::d2h(snake_length_host, io->snake_length, n * sizeof(int32_t), s)) return rc;
-    return beng::d2h(obs_host, io->obs, n * cells, s);
+    return beng::step_host(p, st, actions_dev, io, n_envs, actions_host, nullptr, nullptr, obs_host, reward_host,
+                           terminated_host, truncated_host, score_host, snake_length_host, (cudaStream_t)stream);
 }
 
 int beng_snake_step_host_delta(const beng_snake_params *p, const beng_snake_state *st, int64_t *actions_dev,
                                const beng_snake_io *io, int64_t n_envs, const int64_t *actions_host,
                                uint32_t *delta_dev, uint32_t *delta_host, float *reward_host, uint8_t *terminated_host,
                                uint8_t *truncated_host, int32_t *score_host, int32_t *snake_length_host, void *stream) {
-    if (!actions_host || !actions_dev || !delta_dev || !delta_host) return BENG_ERR_BAD_ARG;
-    if (((uintptr_t)delta_dev & 3) || ((uintptr_t)delta_host & 3)) return BENG_ERR_BAD_ARG;
-    if (int rc = beng::check_common(p, st, io, n_envs)) return rc;
-    if ((truncated_host && !io->truncated) || (score_host && !io->score) || (snake_length_host && !io->snake_length))
-        return BENG_ERR_BAD_ARG;
-    if (n_envs == 0) return 0;
-    cudaStream_t s = (cudaStream_t)stream;
-    const size_t n = (size_t)n_envs;
-    cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, n * sizeof(int64_t), cudaMemcpyHostToDevice, s);
-    if (e != cudaSuccess) return (int)e;
-    if (int rc = beng::step(p, st, actions_dev, io, n_envs, delta_dev, s)) return rc;
-    if (int rc = beng::d2h(delta_host, delta_dev, n * sizeof(uint32_t), s)) return rc;
-    if (int rc = beng::d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
-    if (int rc = beng::d2h(terminated_host, io->terminated, n, s)) return rc;
-    if (int rc = beng::d2h(truncated_host, io->truncated, n, s)) return rc;
-    if (int rc = beng::d2h(score_host, io->score, n * sizeof(int32_t), s)) return rc;
-    return beng::d2h(snake_length_host, io->snake_length, n * sizeof(int32_t), s);
+    if (!delta_dev || !delta_host || ((uintptr_t)delta_dev & 3) || ((uintptr_t)delta_host & 3)) return BENG_ERR_BAD_ARG;
+    return beng::step_host(p, st, actions_dev, io, n_envs, actions_host, delta_dev, delta_host, nullptr, reward_host,
+                           terminated_host, truncated_host, score_host, snake_length_host, (cudaStream_t)stream);
 }
 
 int beng_snake_apply_obs_delta(const uint32_t *delta_host, int8_t *obs_host, int64_t n_envs, int32_t grid_size,

@@ -12,19 +12,18 @@ but the direction (snake_env.py:88-94), a non-eating step has reward 0.
 from __future__ import annotations
 
 import ctypes as C
-import os
 
 import numpy as np
 import torch
 
 from . import _lib
 from .spaces import Box, Discrete, batch_space
-from .vector import _EnvBase, AUTORESET_MODES, LazyInfos, _VectorEnvBase, _mode_name, as_device_actions, host_source, require_cuda, stream_ptr
+from .vector import _EnvBase, AUTORESET_MODES, LazyInfos, _BatchedEnv, as_device_actions, host_source, stream_ptr
 
 STAT_NAMES = ("n_episodes", "sum_return", "sum_length", "sum_score", "max_score")
 
 
-class BatchedSnakeEnv(_VectorEnvBase):
+class BatchedSnakeEnv(_BatchedEnv):
     """N independent SnakeEnvClassic instances, state resident in HBM as structure-of-arrays.
 
     step() returns CUDA tensors that are views of persistent buffers, valid until the next
@@ -34,24 +33,23 @@ class BatchedSnakeEnv(_VectorEnvBase):
     """
 
     metadata = {"render_modes": ["rgb_array"], "render_fps": 10, "autoreset_mode": "same_step"}
+    _reset_fn = "beng_snake_reset"
+    _state_tensors = ("_core", "_ring")
+    _stat_names = STAT_NAMES
+    _host_names = ("_actions", "obs", "reward", "terminated", "truncated", "_score", "_snake_length", "_delta_dev")
+    _mirror, _apply_delta_fn = "obs", "beng_snake_apply_obs_delta"
 
     def __init__(self, num_envs: int, grid_size: int = 20, render_mode=None, *, device="cuda", seed: int = 0,
                  env_id_base: int = 0, autoreset_mode="same_step", max_steps: int = 1000, debug_checks: bool = False,
                  materialize_info: bool = False, time_limit_truncation: bool = False):
-        self.lib = _lib.load()
-        self.device = require_cuda(device)
-        self.num_envs = int(num_envs)
+        super().__init__(num_envs, device, autoreset_mode, render_mode)
         self.grid_size = int(grid_size)
-        self.render_mode = render_mode
         self.max_steps = int(max_steps)
-        self.autoreset_mode = _mode_name(autoreset_mode)
-        self.metadata = dict(type(self).metadata, autoreset_mode=self.autoreset_mode)
         self.debug_checks = bool(debug_checks)
         # info["score"] / info["snake_length"] are derivable from the state record (score == length - 1).  By default
         # they are computed on access instead of being written to HBM every step (8 B per env-step);
         # materialize_info=True makes the kernel write them (the host-buffer path always does).
         self.materialize_info = bool(materialize_info)
-        self.closed = False
 
         G, n, dev = self.grid_size, self.num_envs, self.device
         self.single_action_space = Discrete(4)                                   # snake_env.py:26
@@ -88,11 +86,6 @@ class BatchedSnakeEnv(_VectorEnvBase):
         self._ios = [self._make_io(self.obs, 0), self._make_io(self.obs, 1)]
         self._ios_full = [self._make_io(self.obs, 0, True), self._make_io(self.obs, 1, True)]
         self._info_fresh = True
-        self._host = None
-        # True while the pinned host["obs"] equals the device observations: set by a full-copy step_host(), cleared by
-        # anything else that rewrites them.  step_host(delta_obs=True) patches the copy only while it is set.
-        self._obs_mirror_valid = False
-        self._needs_first_reset = True
 
     # ------------------------------------------------------------------ plumbing
     def _make_io(self, obs: torch.Tensor, parity: int, with_info: bool | None = None) -> "_lib.SnakeIO":
@@ -137,33 +130,13 @@ class BatchedSnakeEnv(_VectorEnvBase):
         return info
 
     # ------------------------------------------------------------------ VectorEnv API
-    def reset(self, *, seed=None, options=None):
-        """SnakeEnvClassic.reset for every env (snake_env.py:49-65) -> (obs, infos).
+    def _reset_io(self):
+        return self._ios_full[0]
 
-        `seed` re-keys the counter-based stream and rewinds it.  (The reference ignores `seed` for
-        food placement -- it draws from the global `random`, SURVEY.md section 3.1.)
-        options={"reset_mask": bool tensor} resets only the selected envs.
-        """
-        first = self._needs_first_reset
-        if seed is not None:
-            self.params.seed = int(seed)
-            first = True
-        mask = None if not options else options.get("reset_mask")
-        mask_ptr = None
-        if mask is not None:
-            mask = torch.as_tensor(mask).to(device=self.device, dtype=torch.uint8).contiguous()
-            if mask.shape != (self.num_envs,):
-                raise ValueError("reset_mask must have shape (num_envs,)")
-            mask_ptr = mask.data_ptr()
-            if self._needs_first_reset:
-                raise RuntimeError("the first reset() must reset every env")
-        with torch.cuda.device(self.device):
-            self._info_fresh = True
-            self._obs_mirror_valid = False
-            rc = self.lib.beng_snake_reset(C.byref(self.params), C.byref(self._state), C.byref(self._ios_full[0]), mask_ptr,
-                                           self.num_envs, int(first), stream_ptr(self.device))
-        _lib.check(rc, "beng_snake_reset")
-        self._needs_first_reset = False
+    def _reset_result(self):
+        """SnakeEnvClassic.reset (snake_env.py:49-65) -> (obs, infos).  (The reference ignores `seed` for food
+        placement -- it draws from the global `random`, SURVEY.md section 3.1.)"""
+        self._info_fresh = True
         return self.obs, {"score": self._score, "snake_length": self._snake_length}
 
     def step(self, actions, out_obs: torch.Tensor | None = None):
@@ -173,8 +146,7 @@ class BatchedSnakeEnv(_VectorEnvBase):
         `out_obs`: optional (num_envs, G, G) int8 CUDA tensor to receive the observations (e.g. a slice
         of a rollout buffer) instead of the persistent `self.obs`.
         """
-        if self._needs_first_reset:
-            raise RuntimeError("call reset() before step()")
+        self._require_reset()
         act = as_device_actions(actions, self._actions)
         io, obs = self._next_io(), self.obs
         if out_obs is not None:
@@ -182,11 +154,9 @@ class BatchedSnakeEnv(_VectorEnvBase):
                     or out_obs.device != self.device:
                 raise ValueError("out_obs must be a contiguous int8 CUDA tensor of shape (num_envs, G, G)")
             io, obs = self._make_io(out_obs, self._parity), out_obs
-        self._obs_mirror_valid = False
-        with torch.cuda.device(self.device):
-            rc = self.lib.beng_snake_step(C.byref(self.params), C.byref(self._state), act.data_ptr(), C.byref(io),
-                                          self.num_envs, stream_ptr(self.device))
-        _lib.check(rc, "beng_snake_step")
+        self._mirror_valid = False
+        self._call("beng_snake_step", C.byref(self.params), C.byref(self._state), act.data_ptr(), C.byref(io),
+                   self.num_envs, stream_ptr(self.device))
         if self.debug_checks:
             self._raise_on_invalid()
         return obs, self.reward, self.terminated, self.truncated, self._infos()
@@ -198,23 +168,6 @@ class BatchedSnakeEnv(_VectorEnvBase):
             raise ValueError(f"Invalid action: {n_bad} action(s) outside Discrete(4)")  # snake_env.py:69-70
 
     # ------------------------------------------------------------------ host-buffer path (numpy in / numpy out)
-    def _host_buffers(self):
-        if self._host is None:
-            n, G = self.num_envs, self.grid_size
-            pin = dict(pin_memory=True)
-            self._host = {
-                "actions": torch.zeros(n, dtype=torch.int64, **pin),
-                "obs": torch.zeros((n, G, G), dtype=torch.int8, **pin),
-                "reward": torch.zeros(n, dtype=torch.float32, **pin),
-                "terminated": torch.zeros(n, dtype=torch.bool, **pin),
-                "truncated": torch.zeros(n, dtype=torch.bool, **pin),
-                "score": torch.zeros(n, dtype=torch.int32, **pin),
-                "snake_length": torch.zeros(n, dtype=torch.int32, **pin),
-                "delta": torch.zeros(n, dtype=torch.int32, **pin),  # observation change records (uint32 bits)
-            }
-            self._delta_dev = torch.zeros(n, dtype=torch.int32, device=self.device)
-        return self._host
-
     def step_host(self, actions, *, copy_obs: bool = True, sync: bool = True, delta_obs: bool = False):
         """step() for callers holding HOST arrays, like users of the reference's numpy API.
 
@@ -229,42 +182,24 @@ class BatchedSnakeEnv(_VectorEnvBase):
         since the last step_host), the call copies the observations in full instead.  The returned
         observation is read-only.  Needs sync=True and copy_obs=True.
         """
-        if delta_obs and not (sync and copy_obs):
-            raise ValueError("step_host(delta_obs=True) needs sync=True and copy_obs=True")
-        if self._needs_first_reset:
-            raise RuntimeError("call reset() before step()")
+        delta = self._mirror_begin(delta_obs, sync, copy_obs)
         h = self._host_buffers()
-        src = torch.as_tensor(np.asarray(actions) if not isinstance(actions, torch.Tensor) else actions)
-        src = self._host_src = host_source(src, h["actions"])
-        delta = delta_obs and self._obs_mirror_valid
-        self._obs_mirror_valid = False
+        src = self._host_src = host_source(actions, h["_actions"])
+        head = (C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._next_io(True)),
+                self.num_envs, src.data_ptr())
         results = (h["reward"].data_ptr(), h["terminated"].data_ptr(), h["truncated"].data_ptr(),
-                   h["score"].data_ptr(), h["snake_length"].data_ptr(), stream_ptr(self.device))
-        with torch.cuda.device(self.device):
-            if delta:
-                rc = self.lib.beng_snake_step_host_delta(
-                    C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._next_io(True)),
-                    self.num_envs, src.data_ptr(), self._delta_dev.data_ptr(), h["delta"].data_ptr(), *results)
-                _lib.check(rc, "beng_snake_step_host_delta")
-            else:
-                rc = self.lib.beng_snake_step_host(
-                    C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._next_io(True)),
-                    self.num_envs, src.data_ptr(), h["obs"].data_ptr() if copy_obs else None, *results)
-                _lib.check(rc, "beng_snake_step_host")
-            if sync:
-                torch.cuda.current_stream(self.device).synchronize()
+                   h["_score"].data_ptr(), h["_snake_length"].data_ptr(), stream_ptr(self.device))
         if delta:
-            rc = self.lib.beng_snake_apply_obs_delta(h["delta"].data_ptr(), h["obs"].data_ptr(), self.num_envs,
-                                                     self.grid_size, len(os.sched_getaffinity(0)))
-            _lib.check(rc, "beng_snake_apply_obs_delta")
-        self._obs_mirror_valid = copy_obs
+            self._call("beng_snake_step_host_delta", *head, self._delta_dev.data_ptr(), h["_delta_dev"].data_ptr(),
+                       *results)
+        else:
+            self._call("beng_snake_step_host", *head, h["obs"].data_ptr() if copy_obs else None, *results)
+        if sync:
+            self._sync()
+        obs = self._mirror_end(delta, delta_obs, copy_obs)
         if self.debug_checks:
             self._raise_on_invalid()
-        obs = h["obs"].numpy() if copy_obs else self.obs
-        if delta_obs:
-            obs = obs.view()
-            obs.flags.writeable = False  # the mirror of the next delta step
-        infos = {"score": h["score"].numpy(), "snake_length": h["snake_length"].numpy()}
+        infos = {"score": h["_score"].numpy(), "snake_length": h["_snake_length"].numpy()}
         return obs, h["reward"].numpy(), h["terminated"].numpy(), h["truncated"].numpy(), infos
 
     # ------------------------------------------------------------------ extras
@@ -273,11 +208,6 @@ class BatchedSnakeEnv(_VectorEnvBase):
         n = int(self.done_count.item())
         return self.done_env[:n]
 
-    def episode_stats(self) -> dict:
-        """Running integer episode statistics accumulated on the device since construction."""
-        vals = self.stats.tolist()
-        return dict(zip(STAT_NAMES, vals))
-
     def export_state(self, with_body: bool = False) -> dict:
         """Unpack the SoA state into int32 tensors (tests / checkpoints)."""
         n, dev = self.num_envs, self.device
@@ -285,28 +215,13 @@ class BatchedSnakeEnv(_VectorEnvBase):
         out = {k: torch.zeros(n, dtype=torch.int32, device=dev) for k in names}
         out["rng_counter"] = torch.zeros(n, dtype=torch.int32, device=dev)  # u32 bit pattern
         body = torch.full((n, self.grid_size ** 2), -1, dtype=torch.int32, device=dev) if with_body else None
-        with torch.cuda.device(dev):
-            rc = self.lib.beng_snake_export_state(
-                C.byref(self.params), C.byref(self._state), n, *[out[k].data_ptr() for k in names],
-                out["rng_counter"].data_ptr(), body.data_ptr() if with_body else None, stream_ptr(dev))
-        _lib.check(rc, "beng_snake_export_state")
+        self._call("beng_snake_export_state", C.byref(self.params), C.byref(self._state), n,
+                   *[out[k].data_ptr() for k in names], out["rng_counter"].data_ptr(),
+                   body.data_ptr() if with_body else None, stream_ptr(dev))
         out["rng_counter"] = out["rng_counter"].to(torch.int64) & 0xFFFFFFFF
         if with_body:
             out["body"] = body
         return out
-
-    def state_dict(self) -> dict:
-        return {"core": self._core.clone(), "ring": self._ring.clone(), "stats": self.stats.clone(),
-                "seed": int(self.params.seed), "env_id_base": int(self.params.env_id_base)}
-
-    def load_state_dict(self, sd: dict):
-        self._core.copy_(sd["core"])
-        self._ring.copy_(sd["ring"])
-        self.stats.copy_(sd["stats"])
-        self.params.seed = int(sd["seed"])
-        self.params.env_id_base = int(sd["env_id_base"])
-        self._obs_mirror_valid = False
-        self._needs_first_reset = False
 
     def render(self):
         """rgb_array frames (num_envs, G*20, G*20, 3) from the current observation: a 3-colour LUT like
@@ -316,9 +231,6 @@ class BatchedSnakeEnv(_VectorEnvBase):
         lut = torch.tensor([[0, 0, 0], [0, 255, 0], [255, 0, 0]], dtype=torch.uint8, device=self.device)
         img = lut[self.obs.long()]
         return img.repeat_interleave(20, 1).repeat_interleave(20, 2).cpu().numpy()
-
-    def close(self, **kwargs):
-        self.closed = True
 
 
 class SnakeEnvClassic(_EnvBase):

@@ -20,7 +20,7 @@ import torch
 
 from . import _lib
 from .spaces import Box, MultiDiscrete, batch_space
-from .vector import _EnvBase, AUTORESET_MODES, _VectorEnvBase, _mode_name, host_source, require_cuda, stream_ptr
+from .vector import _EnvBase, AUTORESET_MODES, _BatchedEnv, as_device_actions, host_source, stream_ptr
 
 # config.py:6-12,23
 DEFAULT_GRID_SIZE = (5, 5)
@@ -33,26 +33,25 @@ DIRECTIONS = ("NORTH", "EAST", "SOUTH", "WEST")                      # utils.py:
 TRAFFIC_STAT_NAMES = ("n_episodes", "sum_return", "sum_length")
 
 
-class BatchedTrafficManagementEnv(_VectorEnvBase):
+class BatchedTrafficManagementEnv(_BatchedEnv):
     """N independent TrafficManagementEnv instances; state resident in HBM as [field][env] integer arrays."""
 
     metadata = {"render_modes": [], "render_fps": 10, "autoreset_mode": "same_step"}
+    _reset_fn = "beng_traffic_reset"
+    _state_tensors = ("_light", "_passed", "_waiting", "_qmeta", "_qwait", "_misc", "_total_reward")
+    _stat_names = TRAFFIC_STAT_NAMES
+    _host_names = ("_actions", "obs", "reward", "terminated", "truncated")
 
     def __init__(self, num_envs: int, grid_size=DEFAULT_GRID_SIZE, num_intersections: int = DEFAULT_NUM_INTERSECTIONS,
                  max_vehicles: int = MAX_VEHICLES, spawn_rate: float = DEFAULT_SPAWN_RATE, render_mode=None, *,
                  device="cuda", seed: int = 0, env_id_base: int = 0, autoreset_mode="same_step",
                  max_timesteps: int = MAX_TIMESTEPS, time_limit_truncation: bool = False):
-        self.lib = _lib.load()
-        self.device = require_cuda(device)
-        self.num_envs = n = int(num_envs)
+        super().__init__(num_envs, device, autoreset_mode, render_mode)
+        n = self.num_envs
         self.grid_size = tuple(grid_size)
         self.num_intersections = ni = min(int(num_intersections), self.grid_size[0] * self.grid_size[1])  # :82
         self.max_vehicles = int(max_vehicles)
         self.spawn_rate = float(spawn_rate)
-        self.render_mode = render_mode
-        self.autoreset_mode = _mode_name(autoreset_mode)
-        self.metadata = dict(type(self).metadata, autoreset_mode=self.autoreset_mode)
-        self.closed = False
         self.obs_dim = ni * 14 + 4                                            # environment.py:116-122
 
         self.single_action_space = MultiDiscrete([3] * ni)                    # :113
@@ -91,8 +90,6 @@ class BatchedTrafficManagementEnv(_VectorEnvBase):
                                   self.truncated.data_ptr(), self.reward64.data_ptr(), self.ep_return.data_ptr(),
                                   self.ep_length.data_ptr(), self.stats.data_ptr(), self.timestep.data_ptr())
         self._infos_cache = None
-        self._host = None
-        self._needs_first_reset = True
 
     # ------------------------------------------------------------------ state views (all (n, ...) tensors)
     @property
@@ -158,105 +155,32 @@ class BatchedTrafficManagementEnv(_VectorEnvBase):
         return dict(self._infos_cache)
 
     # ------------------------------------------------------------------ VectorEnv API
-    def reset(self, *, seed=None, options=None):
-        """TrafficManagementEnv.reset for every env (environment.py:141-166) -> (obs, infos).  reset() itself draws
-        nothing; `seed` re-keys and rewinds the counter-based stream (the reference seeds the global RNGs, :145-147).
-        options={"reset_mask": bool tensor} resets only the selected envs."""
-        first = self._needs_first_reset
-        if seed is not None:
-            self.params.seed = int(seed)
-            first = True
-        mask = None if not options else options.get("reset_mask")
-        mask_ptr = None
-        if mask is not None:
-            if self._needs_first_reset:
-                raise RuntimeError("the first reset() must reset every env")
-            mask = torch.as_tensor(mask).to(device=self.device, dtype=torch.uint8).contiguous()
-            if mask.shape != (self.num_envs,):
-                raise ValueError("reset_mask must have shape (num_envs,)")
-            mask_ptr = mask.data_ptr()
-        with torch.cuda.device(self.device):
-            rc = self.lib.beng_traffic_reset(C.byref(self.params), C.byref(self._state), C.byref(self._io), mask_ptr,
-                                             self.num_envs, int(first), stream_ptr(self.device))
-        _lib.check(rc, "beng_traffic_reset")
-        self._needs_first_reset = False
+    def _reset_result(self):
+        """TrafficManagementEnv.reset (environment.py:141-166) -> (obs, infos).  reset() itself draws nothing (the
+        reference seeds the global RNGs, :145-147)."""
         return self.obs, self._infos()
-
-    def _device_actions(self, actions):
-        buf = self._actions
-        if isinstance(actions, torch.Tensor):
-            if actions.device == buf.device and actions.dtype == buf.dtype and actions.is_contiguous() \
-                    and actions.shape == buf.shape and actions.data_ptr() % 16 == 0:
-                return actions
-            buf.copy_(actions.reshape(buf.shape), non_blocking=True)
-            return buf
-        arr = np.asarray(actions)
-        if arr.shape != tuple(buf.shape):
-            raise ValueError(f"actions must have shape {tuple(buf.shape)}, got {arr.shape}")
-        buf.copy_(torch.from_numpy(np.ascontiguousarray(arr, dtype=np.int64)))
-        return buf
 
     def step(self, actions):
         """One step of every env (environment.py:168-203).  actions: int64 (n, ni), 0 keep / 1 NS_GREEN / 2 EW_GREEN."""
-        if self._needs_first_reset:
-            raise RuntimeError("call reset() before step()")
-        act = self._device_actions(actions)
-        with torch.cuda.device(self.device):
-            rc = self.lib.beng_traffic_step(C.byref(self.params), C.byref(self._state), act.data_ptr(),
-                                            C.byref(self._io), self.num_envs, stream_ptr(self.device))
-        _lib.check(rc, "beng_traffic_step")
+        self._require_reset()
+        act = as_device_actions(actions, self._actions)
+        self._call("beng_traffic_step", C.byref(self.params), C.byref(self._state), act.data_ptr(), C.byref(self._io),
+                   self.num_envs, stream_ptr(self.device))
         return self.obs, self.reward, self.terminated, self.truncated, self._infos()
 
     def step_host(self, actions, *, copy_obs: bool = True, sync: bool = True):
         """step() for callers holding HOST arrays (numpy in, numpy out) through `beng_traffic_step_host`."""
-        if self._needs_first_reset:
-            raise RuntimeError("call reset() before step()")
-        if self._host is None:
-            n = self.num_envs
-            pin = dict(pin_memory=True)
-            self._host = {"actions": torch.zeros((n, self.num_intersections), dtype=torch.int64, **pin),
-                          "obs": torch.zeros((n, self.obs_dim), dtype=torch.float32, **pin),
-                          "reward": torch.zeros(n, dtype=torch.float32, **pin),
-                          "terminated": torch.zeros(n, dtype=torch.bool, **pin),
-                          "truncated": torch.zeros(n, dtype=torch.bool, **pin)}
-        h = self._host
-        src = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions))
-        src = self._host_src = host_source(src, h["actions"])
-        with torch.cuda.device(self.device):
-            rc = self.lib.beng_traffic_step_host(
-                C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._io),
-                self.num_envs, src.data_ptr(), h["obs"].data_ptr() if copy_obs else None,
-                h["reward"].data_ptr(), h["terminated"].data_ptr(), h["truncated"].data_ptr(),
-                stream_ptr(self.device))
-            _lib.check(rc, "beng_traffic_step_host")
-            if sync:
-                torch.cuda.current_stream(self.device).synchronize()
+        self._require_reset()
+        h = self._host_buffers()
+        src = self._host_src = host_source(actions, h["_actions"])
+        self._call("beng_traffic_step_host", C.byref(self.params), C.byref(self._state), self._actions.data_ptr(),
+                   C.byref(self._io), self.num_envs, src.data_ptr(), h["obs"].data_ptr() if copy_obs else None,
+                   h["reward"].data_ptr(), h["terminated"].data_ptr(), h["truncated"].data_ptr(),
+                   stream_ptr(self.device))
+        if sync:
+            self._sync()
         obs = h["obs"].numpy() if copy_obs else self.obs
         return obs, h["reward"].numpy(), h["terminated"].numpy(), h["truncated"].numpy(), {}
-
-    # ------------------------------------------------------------------ extras
-    def episode_stats(self) -> dict:
-        return dict(zip(TRAFFIC_STAT_NAMES, self.stats.tolist()))
-
-    def state_dict(self) -> dict:
-        names = ("light", "passed", "waiting", "qmeta", "qwait", "misc", "total_reward")
-        sd = {k: getattr(self, "_" + k).clone() for k in names}
-        sd.update(stats=self.stats.clone(), seed=int(self.params.seed), env_id_base=int(self.params.env_id_base))
-        return sd
-
-    def load_state_dict(self, sd: dict):
-        for k in ("light", "passed", "waiting", "qmeta", "qwait", "misc", "total_reward"):
-            getattr(self, "_" + k).copy_(sd[k])
-        self.stats.copy_(sd["stats"])
-        self.params.seed = int(sd["seed"])
-        self.params.env_id_base = int(sd["env_id_base"])
-        self._needs_first_reset = False
-
-    def render(self):
-        return None  # pygame rendering is out of scope (SURVEY.md section 2)
-
-    def close(self, **kwargs):
-        self.closed = True
 
 
 class TrafficManagementEnv(_EnvBase):

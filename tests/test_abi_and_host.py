@@ -104,6 +104,34 @@ def test_spaces_and_batching():
     assert 0 <= d.sample() < 4
 
 
+def test_action_upload_shape_and_dtype_rules():
+    """vector.as_device_actions with CPU buffers: a tensor of the buffer's dtype and shape is used as it is, anything
+    else lands in the buffer in the buffer's dtype; arrays must have exactly the buffer's shape."""
+    from custom_gymnasium_environments_b200.vector import as_device_actions
+
+    buf = torch.zeros(5, dtype=torch.int64)
+    same = torch.arange(5)
+    assert as_device_actions(same, buf) is same
+    for src in (torch.arange(6)[1:], torch.arange(5, dtype=torch.int32), torch.arange(5).reshape(5, 1),
+                [0, 1, 2, 3, 4], np.arange(5, dtype=np.int16)):  # misaligned view, other dtype, other shape, list, numpy
+        buf.zero_()
+        out = as_device_actions(src, buf)
+        assert out is buf and out.dtype == torch.int64 and out.tolist() == list(torch.as_tensor(src).reshape(5).tolist())
+    for bad in (np.zeros((5, 1), np.int64), np.zeros(6, np.int64), np.zeros((1, 5), np.int64)):
+        with pytest.raises(ValueError, match="shape"):
+            as_device_actions(bad, buf)
+
+    for dtype, src in ((torch.float32, np.array([[1.0, 2.0], [3.0, 4.0]])), (torch.int8, np.array([[1, 0], [0, 1]]))):
+        buf = torch.zeros((2, 2), dtype=dtype)
+        out = as_device_actions(src, buf)
+        assert out is buf and out.dtype == dtype and np.array_equal(out.numpy(), src)
+        with pytest.raises(ValueError, match="shape"):
+            as_device_actions(src.T.reshape(4), buf)
+        t = torch.tensor(src, dtype=dtype)
+        out = as_device_actions(t, buf)
+        assert out.dtype == dtype and torch.equal(out, t)
+
+
 def test_shard_range_partitions_exactly():
     from custom_gymnasium_environments_b200.dist import shard_range
 
