@@ -111,4 +111,26 @@ __device__ __forceinline__ double div_const(double x) {
     return fma(r, y, q);
 }
 
+// NumPy's pairwise summation order (np.sum / np.mean / np.var, n <= 128) over f(0..n-1), without materialising the
+// array: the values are produced on demand so that the caller never holds all of them in registers.
+template <typename F>
+__device__ __forceinline__ double np_sum_fn(F f, int n) {
+    if (n < 8) {
+        double r = 0.0;
+        for (int i = 0; i < n; ++i) r += f(i);
+        return r;
+    }
+    double r[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) r[j] = f(j);
+    int i = 8;
+    for (; i < n - (n % 8); i += 8) {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) r[j] += f(i + j);
+    }
+    double res = ((r[0] + r[1]) + (r[2] + r[3])) + ((r[4] + r[5]) + (r[6] + r[7]));
+    for (; i < n; ++i) res += f(i);
+    return res;
+}
+
 }  // namespace beng

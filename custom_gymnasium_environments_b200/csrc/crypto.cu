@@ -113,7 +113,7 @@ __device__ __forceinline__ double next_price(const beng_crypto_params &p, Market
                                              double volume) {
     if (rng.random53() < 0.01) update_regime(m, rng);
     const double u1 = rng.random53(), u2 = rng.random53();  // np.random.normal(0, volatility): Box-Muller, RNG contract
-    const double z = sqrt(-2.0 * log(1.0 - u1)) * cos(2.0 * 3.141592653589793 * u2);
+    const double z = box_muller(u1, u2);
     return price_update(p, m, cur, z, 1.0 / (1.0 + volume * 0.1));
 }
 
@@ -164,26 +164,19 @@ __device__ __noinline__ WarmupResult warmup_window(double *close_arr, float4 *oh
 // All 32 lanes call this with identical arguments.  Bit-identical to warmup_window() (tests: sparse-reset rollouts).
 // 20 consecutive words of an env's stream, starting at the Philox block that holds draw `c`: five blocks computed up
 // front, no "is my block cached?" branch per draw (lanes of a warp sit at different alignments, so the lazy EnvStream
-// evaluated Philox up to once per draw: ~30 times per candle instead of 5).  Same draw -> value maps as EnvStream.
-struct WordWindow {
+// evaluated Philox up to once per draw: ~30 times per candle instead of 5).
+struct WordWindow : Draws<WordWindow> {
     uint32_t w[20];  // (indexed by a per-lane position: lives in local memory; this is the rare reset path)
     uint32_t pos;
     __device__ __forceinline__ WordWindow(uint64_t seed, uint64_t env, uint32_t c) : pos(c & 3u) {
 #pragma unroll
         for (int b = 0; b < 5; ++b) {
-            const Philox4 r = philox4x32_10((c >> 2) + b, (uint32_t)env, (uint32_t)(env >> 32), BENG_STREAM_ENV,
-                                            (uint32_t)seed, (uint32_t)(seed >> 32));
+            const Philox4 r = philox_block((c >> 2) + b, stream_key(env, BENG_STREAM_ENV, seed));
 #pragma unroll
             for (int q = 0; q < 4; ++q) w[4 * b + q] = r.v[q];
         }
     }
     __device__ __forceinline__ uint32_t u32() { return w[pos++]; }
-    __device__ __forceinline__ int randint(int a, int b) { return a + (int)__umulhi(u32(), (uint32_t)(b - a + 1)); }
-    __device__ __forceinline__ double random53() {
-        const uint32_t a = u32() >> 5, b = u32() >> 6;
-        return ((double)a * 67108864.0 + (double)b) * (1.0 / 9007199254740992.0);
-    }
-    __device__ __forceinline__ double uniform(double a, double b) { return a + (b - a) * random53(); }
 };
 
 __device__ __noinline__ WarmupResult coop_warmup_window(double *close_arr, float4 *ohlv_arr, long long n, long long env,
@@ -209,7 +202,7 @@ __device__ __noinline__ WarmupResult coop_warmup_window(double *close_arr, float
                     rt[h] = r.random53();
                 }
                 const double u1 = r.random53(), u2 = r.random53();
-                z[h] = sqrt(-2.0 * log(1.0 - u1)) * cos(2.0 * 3.141592653589793 * u2);
+                z[h] = box_muller(u1, u2);
                 vf[h] = 1.0 / (1.0 + volume[h] * 0.1);
                 uh[h] = r.uniform(1.0, 1.02);
                 ul[h] = r.uniform(0.98, 1.0);
@@ -263,38 +256,10 @@ __device__ __noinline__ WarmupResult coop_warmup_window(double *close_arr, float
     return WarmupResult{m, ctr + 14u * HIST + 3u * (uint32_t)changes, price};
 }
 
-// NumPy's pairwise summation order for 8 <= n <= 128 (np.mean / np.std in the reference), n static; the values are
-// produced on demand so that the caller never holds all of them in registers.
-template <int N, typename F>
-__device__ __forceinline__ double np_sum(F val) {
-    static_assert(N >= 8 && N < 24, "restated for the two sizes the reference uses (14, 20)");
-    double r[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) r[j] = val(j);
-    if (N >= 16) {
-#pragma unroll
-        for (int j = 0; j < 8; ++j) r[j] += val(8 + j);
-    }
-    double res = ((r[0] + r[1]) + (r[2] + r[3])) + ((r[4] + r[5]) + (r[6] + r[7]));
-#pragma unroll
-    for (int i = (N >= 16 ? 16 : 8); i < N; ++i) res += val(i);
-    return res;
-}
-
 // Streaming (evict-first) loads of the window.  Plain weak loads are enough for data written earlier in the SAME CTA:
 // bar.sync orders the global-memory accesses of the participating threads, and no other CTA touches this env's window.
 __device__ __forceinline__ double ld_win_f64(const double *p) { return __ldcs(p); }
 __device__ __forceinline__ float4 ld_win_f32x4(const float4 *p) { return __ldcs(p); }
-
-// x / 20 correctly rounded without the division subroutine (its slow-path CALL would force every value that is live
-// across it -- the prefetched window of the next unit -- into local memory).  Markstein: with y = RN(1/20),
-// q = RN(x y), r = x - 20 q (exact in an FMA), RN(q + r y) is the correctly rounded quotient for normal-range x.
-__device__ __forceinline__ double div20(double x) {
-    const double y = 0.05;
-    const double q = x * y;
-    const double r = __fma_rn(-20.0, q, x);
-    return __fma_rn(r, y, q);
-}
 
 // _execute_buy, :449-476.  Returns 1 when the order executed.
 template <typename RNG>
@@ -416,10 +381,9 @@ constexpr MacdWeights make_macd_weights() {
 constexpr MacdWeights k_macd_weights = make_macd_weights();
 __constant__ MacdWeights c_macd = k_macd_weights;
 
-// One env's pre-computed Philox words in shared memory (word j of thread t at w[j * NT]); same draw -> value maps as
-// EnvStream (beng_rng.cuh, contract in oracle/philox.py).
+// One env's pre-computed Philox words in shared memory (word j of thread t at w[j * NT]).
 template <int NT>
-struct TableStream {
+struct TableStream : Draws<TableStream<NT>> {
     const uint32_t *w;
     uint32_t pos, ctr;
     __device__ __forceinline__ uint32_t u32() {
@@ -428,12 +392,6 @@ struct TableStream {
         ++ctr;
         return v;
     }
-    __device__ __forceinline__ int randint(int a, int b) { return a + (int)__umulhi(u32(), (uint32_t)(b - a + 1)); }
-    __device__ __forceinline__ double random53() {
-        const uint32_t a = u32() >> 5, b = u32() >> 6;
-        return ((double)a * 67108864.0 + (double)b) * (1.0 / 9007199254740992.0);
-    }
-    __device__ __forceinline__ double uniform(double a, double b) { return a + (b - a) * random53(); }
 };
 
 // The dynamics of one 32-env unit `u`, run by ONE warp (lane = env), one thread per env, in the reference's float64
@@ -492,13 +450,12 @@ __device__ __forceinline__ unsigned dynamics_phase(const CArgs &a, long long u, 
         } else if (a.p.autoreset_mode == BENG_AUTORESET_NEXT_STEP && (flags & CFLAG_NEEDS_RESET)) {
             need_reset = true;  // the ring head moved by one slot with this call: whole window at the new rotation
         } else {
-            TableStream<NT> rng{tbl, ctr & 3u, ctr};
+            TableStream<NT> rng{{}, tbl, ctr & 3u, ctr};
             {
                 const uint32_t blk0 = ctr >> 2;
 #pragma unroll
                 for (int b = 0; b < C3_RNGW / 4; ++b) {
-                    const Philox4 r = philox4x32_10(blk0 + b, (uint32_t)gid, (uint32_t)(gid >> 32), BENG_STREAM_ENV,
-                                                    (uint32_t)a.p.seed, (uint32_t)(a.p.seed >> 32));
+                    const Philox4 r = philox_block(blk0 + b, stream_key(gid, BENG_STREAM_ENV, a.p.seed));
 #pragma unroll
                     for (int q = 0; q < 4; ++q) tbl[(4 * b + q) * NT] = r.v[q];
                 }
@@ -785,20 +742,22 @@ __device__ __forceinline__ void finish_unit(const ObsSmem &sm, int e, int g, flo
     } else if (g == 1) {  // RSI(14) over the last 14 deltas, :45-61; rsi/100 = gain / (gain + loss)
         const double *wl = sm.last + 5 * C3_SUB + e;  // the last 15 closes
         auto delta = [&](int i) { return wl[(i + 1) * C3_SUB] - wl[i * C3_SUB]; };
-        const double sg = np_sum<14>([&](int i) { const double d = delta(i); return d > 0 ? d : 0.0; });
-        const double sl = np_sum<14>([&](int i) { const double d = delta(i); return d < 0 ? -d : 0.0; });
+        const double sg = np_sum_fn([&](int i) { const double d = delta(i); return d > 0 ? d : 0.0; }, 14);
+        const double sl = np_sum_fn([&](int i) { const double d = delta(i); return d < 0 ? -d : 0.0; }, 14);
         dst[253] = (sl != 0) ? __fdividef((float)sg, (float)(sg + sl)) : 1.0f;
     } else if (g == 2) {  // Bollinger(20, 2 sigma, population std), :64-77 and :550-554
         // Mean and variance of the DIFFERENCES to the newest close (exact subtractions): a window of identical closes
         // -- a price pinned at the clip bound -- gives sma == close and sd == 0 exactly, like the reference, and the sums
-        // are 4-deep trees instead of NumPy's 8-deep pairwise chains.
+        // are 4-deep trees instead of NumPy's 8-deep pairwise chains.  div_const, not `/`: the division subroutine's
+        // slow-path CALL would force every value live across it -- the prefetched window of the next unit -- into
+        // local memory.
         const double *wl = sm.last + e;
         const double cur = wl[(C3_LAST - 1) * C3_SUB];
         auto dv = [&](int i) { return wl[i * C3_SUB] - cur; };
         const double s = tree_sum16(dv) + ((dv(16) + dv(17)) + (dv(18) + dv(19)));
-        const double mean_d = div20(s);
+        const double mean_d = div_const<20>(s);
         auto sq = [&](int i) { const double t = dv(i) - mean_d; return t * t; };
-        const double var = div20(tree_sum16(sq) + ((sq(16) + sq(17)) + (sq(18) + sq(19))));
+        const double var = div_const<20>(tree_sum16(sq) + ((sq(16) + sq(17)) + (sq(18) + sq(19))));
         const float var_f = (float)var;
         const double sd = (double)(var_f > 0.0f ? var_f * rsqrtf(var_f) : 0.0f);  // float32 accuracy: it only scales features
         const double sma = cur + mean_d;

@@ -45,27 +45,6 @@ struct TArgs {
     uint32_t inv_cols;  // ceil(2^16 / grid_cols): (start * inv_cols) >> 16 == start / grid_cols for start < 25
 };
 
-// NumPy's pairwise summation (np.var in _calculate_reward, n <= 128) over f(0..n-1), without materialising the array
-template <typename F>
-__device__ __forceinline__ double np_sum_fn(F f, int n) {
-    if (n < 8) {
-        double r = 0.0;
-        for (int i = 0; i < n; ++i) r += f(i);
-        return r;
-    }
-    double r[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) r[j] = f(j);
-    int i = 8;
-    for (; i < n - (n % 8); i += 8) {
-#pragma unroll
-        for (int j = 0; j < 8; ++j) r[j] += f(i + j);
-    }
-    double res = ((r[0] + r[1]) + (r[2] + r[3])) + ((r[4] + r[5]) + (r[6] + r[7]));
-    for (; i < n; ++i) res += f(i);
-    return res;
-}
-
 // (float)((double)a / (double)b) for non-negative integers.  When both are exactly representable in binary32 the
 // correctly rounded binary32 quotient is the same number (rounding a binary64 quotient of two binary32 values to
 // binary32 is innocuous: 53 >= 2*24+2), so the common case is one IEEE float division instead of an FP64 one.
@@ -81,13 +60,12 @@ __device__ __forceinline__ float ratio_f32(long long a, long long b) {
 constexpr int SPEC_BLOCKS = 3;
 
 __device__ __noinline__ uint32_t philox_draw(uint32_t idx, uint64_t env, uint64_t seed) {
-    const Philox4 p = philox4x32_10(idx >> 2, (uint32_t)env, (uint32_t)(env >> 32), BENG_STREAM_ENV, (uint32_t)seed,
-                                    (uint32_t)(seed >> 32));
+    const Philox4 p = philox_block(idx >> 2, stream_key(env, BENG_STREAM_ENV, seed));
     const uint32_t l = idx & 3u;
     return l == 0 ? p.v[0] : l == 1 ? p.v[1] : l == 2 ? p.v[2] : p.v[3];
 }
 
-struct CachedStream {
+struct CachedStream : Draws<CachedStream> {
     uint32_t ctr;
     uint32_t first;          // index of the first cached draw (a multiple of 4)
     const uint32_t *cache;   // [SPEC_BLOCKS * 4][32] in shared memory, already offset by the lane
@@ -96,11 +74,6 @@ struct CachedStream {
         const uint32_t idx = ctr++, rel = idx - first;
         if (rel < SPEC_BLOCKS * 4) return cache[rel * 32];
         return philox_draw(idx, env, seed);
-    }
-    __device__ __forceinline__ int randint(int a, int b) { return a + (int)__umulhi(u32(), (uint32_t)(b - a + 1)); }
-    __device__ __forceinline__ double random53() {
-        const uint32_t a = u32() >> 5, b = u32() >> 6;
-        return ((double)a * 67108864.0 + (double)b) * (1.0 / 9007199254740992.0);
     }
 };
 
@@ -439,8 +412,7 @@ __global__ void __maxnreg__(TRAFFIC_MAXREG) traffic_step_kernel(const TArgs a) {
             if (stepping) {
 #pragma unroll
                 for (int b = 0; b < SPEC_BLOCKS; ++b) {
-                    const Philox4 ph = philox4x32_10(blk0 + b, (uint32_t)env_id, (uint32_t)(env_id >> 32),
-                                                     BENG_STREAM_ENV, (uint32_t)a.p.seed, (uint32_t)(a.p.seed >> 32));
+                    const Philox4 ph = philox_block(blk0 + b, stream_key(env_id, BENG_STREAM_ENV, a.p.seed));
 #pragma unroll
                     for (int k = 0; k < 4; ++k) s_phx[(b * 4 + k) * WPI_E + lane] = ph.v[k];
                 }
@@ -452,7 +424,7 @@ __global__ void __maxnreg__(TRAFFIC_MAXREG) traffic_step_kernel(const TArgs a) {
             int spawn = -1;
             // _spawn_vehicles (:222-249)
             if (stepping && listed < a.p.max_vehicles) {
-                CachedStream rng{ctr, blk0 << 2, s_phx + lane, env_id, a.p.seed};
+                CachedStream rng{{}, ctr, blk0 << 2, s_phx + lane, env_id, a.p.seed};
                 if (rng.random53() < a.p.spawn_rate) {
                     int sp_i, sp_d, sp_lb;
                     spawn_route(a, rng, sp_i, sp_d, sp_lb);
