@@ -105,6 +105,8 @@ SIGNATURES = {
                                    C.c_int64, C.c_int32, C.c_void_p]),
     "beng_snake_step": (C.c_int, [C.POINTER(SnakeParams), C.POINTER(SnakeState), C.c_void_p, C.POINTER(SnakeIO),
                                   C.c_int64, C.c_void_p]),
+    "beng_snake_step_inplace": (C.c_int, [C.POINTER(SnakeParams), C.POINTER(SnakeState), C.c_void_p,
+                                          C.POINTER(SnakeIO), C.c_int64, C.c_void_p]),
     "beng_snake_step_host": (C.c_int, [C.POINTER(SnakeParams), C.POINTER(SnakeState), C.c_void_p, C.POINTER(SnakeIO),
                                        C.c_int64] + [C.c_void_p] * 8),
     "beng_snake_step_host_delta": (C.c_int, [C.POINTER(SnakeParams), C.POINTER(SnakeState), C.c_void_p,

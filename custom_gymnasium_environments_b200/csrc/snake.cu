@@ -7,13 +7,20 @@
 //   SnakeEnvClassic._place_food      snake_env_classic/snake_env.py:121-129
 //   SnakeEnvClassic._get_observation snake_env_classic/snake_env.py:131-143
 //
-// Design (DESIGN.md section 3):
+// Two step kernels with the same dynamics, results and state (DESIGN.md sections 3 and 6e):
+//   * snake_kernel (beng_snake_reset, beng_snake_step, the host-buffer calls) composes every
+//     observation row in full, into any buffer;
+//   * snake_patch_kernel (beng_snake_step_inplace) expects io.obs to hold the previous observation
+//     and writes only the cells that change -- at most two per env, the whole row on a reset -- with
+//     per-thread byte stores; the previous row doubles as the occupancy map (see the kernel).
+//
+// snake_kernel:
 //   * one THREAD per env does the integer dynamics out of a 16-byte state record (one LDG.128 /
 //     STG.128 per env, perfectly coalesced);
 //   * one CTA owns a TILE of T consecutive envs; their T x G*G observation bytes are contiguous in
 //     global memory, so the tile is composed in shared memory (zero fill, scatter body cells, food
 //     last) and drained with ONE bulk asynchronous copy (cp.async.bulk shared->global, the TMA
-//     engine, SASS UBLKCP) issued by a single thread -- no per-thread obs stores at all;
+//     engine, SASS UBLKCP) issued by a single thread -- no per-thread obs stores in this kernel;
 //   * CTAs are persistent over tiles with one tile buffer each; several CTAs per SM keep the copy
 //     engine draining one CTA's tile while the others compose theirs;
 //   * the shared-memory tile doubles as the O(1) occupancy map for self-collision and for the
@@ -22,8 +29,9 @@
 //     flushed with one set of global atomics per CTA; a warp-aggregated compaction emits the
 //     list of finished envs.
 //
-// The kernel is HBM-bound (450 algorithmic bytes per env-step, 400 of them the observation
-// write); there is nothing GEMM-shaped here and no tensor-core path is wanted.
+// Both are HBM-bound: snake_kernel moves 450 algorithmic bytes per env-step, 400 of them the
+// observation write; snake_patch_kernel about 150 (DESIGN.md section 6e).  There is nothing
+// GEMM-shaped here and no tensor-core path is wanted.
 #include <climits>
 #include <cstdint>
 #include <cstring>
@@ -83,11 +91,13 @@ struct Args {
 };
 
 // _place_food (snake_env.py:121-129): draw (row, col) until the cell is not part of the snake.
-// `row` holds 1 for every body cell at this point (the food mark is written afterwards), so the
-// membership test is one shared-memory byte load.  The reference never returns when the board is
-// full (length == G*G, unreachable at G = 20 within 1000 steps); there the engine and the oracle
+// `occupied(cell)` tells whether a cell holds part of the body; the callers answer it from an
+// observation row in which every body cell holds 1 and no food is marked (the food is written
+// afterwards), so the membership test is one byte load.  The reference never returns when the board
+// is full (length == G*G, unreachable at G = 20 within 1000 steps); there the engine and the oracle
 // both leave the board without food instead of spinning.
-__device__ __forceinline__ void place_food(Core &s, EnvStream &rng, const uint8_t *row, int G) {
+template <typename Occupied>
+__device__ __forceinline__ void place_food(Core &s, EnvStream &rng, int G, Occupied occupied) {
     if (s.length >= G * G) {
         s.food_r = s.food_c = FOOD_NONE;
         return;
@@ -95,7 +105,7 @@ __device__ __forceinline__ void place_food(Core &s, EnvStream &rng, const uint8_
     for (;;) {
         const int r = rng.randint(0, G - 1);
         const int c = rng.randint(0, G - 1);
-        if (row[r * G + c] == 0) {
+        if (!occupied(r * G + c)) {
             s.food_r = r;
             s.food_c = c;
             return;
@@ -103,8 +113,15 @@ __device__ __forceinline__ void place_food(Core &s, EnvStream &rng, const uint8_
     }
 }
 
-// reset (snake_env.py:49-65).  Expects `row` to be all zero.
-__device__ __forceinline__ void reset_env(Core &s, EnvStream &rng, uint8_t *row, int G) {
+// Row tests for place_food: a byte of the row (shared or global memory; the kernels write these rows themselves, so
+// the loads are plain coherent ones).
+__device__ __forceinline__ auto body_in(const uint8_t *row) {
+    return [row](int cell) { return row[cell] != 0; };
+}
+
+// The state record of reset (snake_env.py:49-65): a length-1 snake in the centre.  (The ring is not touched: it only
+// holds bodies of length >= 2.)
+__device__ __forceinline__ void reset_core(Core &s, int G) {
     const int center = G / 2;
     s.head_r = s.head_c = center;
     s.dir = 1;
@@ -112,8 +129,13 @@ __device__ __forceinline__ void reset_env(Core &s, EnvStream &rng, uint8_t *row,
     s.steps = 0;
     s.ring_head = 0;
     s.flags = 0;
-    row[center * G + center] = 1;  // (the ring is not touched: it only holds bodies of length >= 2)
-    place_food(s, rng, row, G);
+}
+
+// reset (snake_env.py:49-65).  Expects `row` to be all zero.
+__device__ __forceinline__ void reset_env(Core &s, EnvStream &rng, uint8_t *row, int G) {
+    reset_core(s, G);
+    row[s.head_r * G + s.head_c] = 1;
+    place_food(s, rng, G, body_in(row));
 }
 
 // Walk the body oldest -> newest, writing `mark` into the tile row.  Returns the tail cell and
@@ -181,6 +203,32 @@ __device__ __forceinline__ Loaded load_inputs(const Args &a, long long env) {
         else if (a.mask) l.selected = a.mask[env] != 0;
     }
     return l;
+}
+
+// Adds the episodes of one warp's finished envs (done_mask = ballot of `ended`) to the CTA's counters
+// s_stats = {n_episodes, sum_return, sum_length, sum_score, max_score}.
+__device__ __forceinline__ void add_warp_stats(int *s_stats, unsigned done_mask, bool ended, int ep_ret, int ep_len,
+                                               int ep_score, int lane) {
+    const int sr = __reduce_add_sync(0xFFFFFFFFu, ended ? ep_ret : 0);
+    const int sl = __reduce_add_sync(0xFFFFFFFFu, ended ? ep_len : 0);
+    const int ss = __reduce_add_sync(0xFFFFFFFFu, ended ? ep_score : 0);
+    const int mx = __reduce_max_sync(0xFFFFFFFFu, ended ? ep_score : INT_MIN);
+    if (lane == 0) {
+        atomicAdd(&s_stats[0], __popc(done_mask));
+        atomicAdd(&s_stats[1], sr);
+        atomicAdd(&s_stats[2], sl);
+        atomicAdd(&s_stats[3], ss);
+        atomicMax(&s_stats[4], mx);
+    }
+}
+
+// One set of global atomics per CTA for its counters (after a barrier that completes them).
+__device__ __forceinline__ void flush_stats(int64_t *stats, const int *s_stats, int tid) {
+    if (tid < 4) {
+        if (s_stats[tid] != 0) atomicAdd((unsigned long long *)&stats[tid], (unsigned long long)(long long)s_stats[tid]);
+    } else if (tid == 4) {
+        if (s_stats[4] != INT_MIN) atomicMax((long long *)&stats[4], (long long)s_stats[4]);
+    }
 }
 
 // OWNROW: every thread zero-fills its own env row with 16-byte stores (needs G*G % 16 == 0, and is
@@ -325,7 +373,7 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
                         if (eat) {  // :101-104
                             s.length += 1;
                             rew = 10.0f;
-                            place_food(s, rng, row, G);
+                            place_food(s, rng, G, body_in(row));
                         } else {
                             row[tail_cell] = 0;  // pop(), :107
                         }
@@ -406,19 +454,7 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
                     pend_mask = done_mask;
                     pend_env = (int)env;
                 }
-                if (a.io.stats) {
-                    const int sr = __reduce_add_sync(0xFFFFFFFFu, ended ? ep_ret : 0);
-                    const int sl = __reduce_add_sync(0xFFFFFFFFu, ended ? ep_len : 0);
-                    const int ss = __reduce_add_sync(0xFFFFFFFFu, ended ? ep_score : 0);
-                    const int mx = __reduce_max_sync(0xFFFFFFFFu, ended ? ep_score : INT_MIN);
-                    if (lane == 0) {
-                        atomicAdd(&s_stats[0], __popc(done_mask));
-                        atomicAdd(&s_stats[1], sr);
-                        atomicAdd(&s_stats[2], sl);
-                        atomicAdd(&s_stats[3], ss);
-                        atomicMax(&s_stats[4], mx);
-                    }
-                }
+                if (a.io.stats) add_warp_stats(s_stats, done_mask, ended, ep_ret, ep_len, ep_score, lane);
             }
         }
         // Fetch the next tile's tail ring entry now (its state record, requested at the top of this iteration,
@@ -444,13 +480,163 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
     if constexpr (!IS_RESET) {
         if (a.io.stats) {
             __syncthreads();
-            if (tid < 4) {
-                if (s_stats[tid] != 0)
-                    atomicAdd((unsigned long long *)&a.io.stats[tid], (unsigned long long)(long long)s_stats[tid]);
-            } else if (tid == 4) {
-                if (s_stats[4] != INT_MIN) atomicMax((long long *)&a.io.stats[4], (long long)s_stats[4]);
+            flush_stats(a.io.stats, s_stats, tid);
+        }
+    }
+}
+
+// Zero an observation row with the widest stores its alignment allows: 16-byte stores throughout when G*G % 16 == 0
+// (io->obs is 16-byte aligned, so every row then starts on a 16-byte boundary), byte stores around them otherwise.
+__device__ __forceinline__ void clear_row(uint8_t *row, int cells) {
+    uint8_t *p = row, *const end = row + cells;
+    while (((uintptr_t)p & 15) && p < end) *p++ = 0;
+    for (; p + 16 <= end; p += 16) *reinterpret_cast<uint4 *>(p) = make_uint4(0, 0, 0, 0);
+    while (p < end) *p++ = 0;
+}
+
+// reset (snake_env.py:49-65) of an env whose observation row lives in global memory: the row is cleared, then the
+// head and the food are written, as a BENG_OBS_DELTA_CLEAR record describes it.  The food test needs no memory read:
+// the only body cell is the head.
+__device__ __forceinline__ void reset_row(Core &s, EnvStream &rng, uint8_t *row, int G) {
+    clear_row(row, G * G);
+    reset_core(s, G);
+    const int head = s.head_r * G + s.head_c;
+    row[head] = 1;
+    place_food(s, rng, G, [head](int cell) { return cell == head; });
+    row[s.food_r * G + s.food_c] = 2;  // (a length-1 snake always leaves room for food)
+}
+
+// 6 CTAs of 256 threads per SM (<= 40 registers, no spills): the kernel is bound by the latency of its two dependent
+// rounds of loads (state + action, then the row byte + tail entry), so resident threads are what it runs on.  Measured on
+// B200 at 1M envs, G = 20: 61.5 us per step against 65.8 us at the 5 CTAs per SM that 46 registers give.
+constexpr int PATCH_THREADS = 256, PATCH_CTAS_PER_SM = 6;
+
+// The step kernel of beng_snake_step_inplace: same dynamics, rewards, flags, state and statistics as snake_kernel, but
+// io.obs must already hold the observation of the previous reset or step, and only the cells that change are written
+// (move: old tail -> 0, new head -> 1; eat: new head -> 1, new food -> 2; death / invalid action: nothing; reset: clear,
+// head -> 1, food -> 2 -- the order of the BENG_OBS_DELTA records).  One thread per env and no shared-memory tile:
+//   * the previous observation is the occupancy map, so self-collision (`new_head in self.snake`, tail included,
+//     snake_env.py:93) is the byte obs[new_cell] == 1 instead of a walk over the ring; the ring is read only for the
+//     tail cell a move of a length >= 2 snake clears, and written only where snake_kernel writes it;
+//   * the food rejection loop after a meal reads the same row, with the new head already written over the old food.
+// The row loads are plain coherent loads (no .nc / __ldg / __restrict__): this kernel writes those bytes itself.
+__global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_kernel(const Args a) {
+    __shared__ int s_stats[5];  // per-CTA: n_episodes, sum_return, sum_length, sum_score, max_score
+    const int tid = threadIdx.x;
+    const int lane = tid & 31;
+    const int G = a.G;
+    const int cells = G * G;
+    const long long env = (long long)blockIdx.x * PATCH_THREADS + tid;
+    const bool active = env < a.n_envs;
+
+    if (tid < 5) s_stats[tid] = (tid == 4) ? INT_MIN : 0;
+    pdl_launch_dependents();
+    pdl_wait();  // the previous step's state, observations and counters are complete from here on
+    if (blockIdx.x == 0 && tid == 0 && a.io.done_count_next) *a.io.done_count_next = 0;  // for the NEXT step
+    __syncthreads();
+
+    bool ended = false;
+    int ep_ret = 0, ep_len = 0, ep_score = 0;
+    if (active) {
+        const long long act = ld_stream_s64(a.actions + env);
+        Core s = unpack(ld_stream_u4(a.core + env));
+        uint8_t *row = reinterpret_cast<uint8_t *>(a.io.obs) + env * cells;
+        uint16_t *ring = a.ring + env * cells;
+        EnvStream rng(a.seed, a.env_id_base + (uint64_t)env, BENG_STREAM_ENV, s.ctr);
+        float rew = 0.0f;
+        int term = 0, trunc = 0;
+        // `invalid` is settled before any branch and used after them all, so that the action load is issued together
+        // with the state load instead of being sunk into the move branch, one memory round trip later
+        const bool needs_reset = a.mode == BENG_AUTORESET_NEXT_STEP && (s.flags & FLAG_NEEDS_RESET);
+        const bool invalid = !needs_reset && (act < 0 || act > 3);  // the env is left untouched (see snake_kernel)
+        bool reset = needs_reset;  // action ignored, reward 0, not terminated
+        if (!needs_reset && !invalid) {
+            const int action = (int)act;
+            int d = action - s.dir;
+            if (d < 0) d = -d;
+            if (d != 2) s.dir = action;  // reversal guard, snake_env.py:73-74
+            const int nr = s.head_r + (s.dir == 2) - (s.dir == 0);
+            const int nc = s.head_c + (s.dir == 1) - (s.dir == 3);
+            const bool wall = (unsigned)nr >= (unsigned)G || (unsigned)nc >= (unsigned)G;  // :88-90
+            const int new_cell = nr * G + nc;
+            const int head_cell = s.head_r * G + s.head_c;
+            const int food_cell = (s.food_r == FOOD_NONE) ? -2 : s.food_r * G + s.food_c;
+
+            bool self_hit = false;  // (a length-1 snake cannot hit itself)
+            int tail_cell = head_cell;
+            if (!wall && s.length > 1) {
+                tail_cell = ring[tail_index(s, cells)];  // (both loads are issued before either is used)
+                self_hit = row[new_cell] == 1;
+            }
+            const bool died = wall || self_hit;
+            if (died) {
+                rew = -10.0f;  // :90 / :94 -- nothing but `direction` was mutated, the row is unchanged
+                term = 1;
+            } else {
+                const bool eat = new_cell == food_cell;
+                if (s.length > 1 || eat) {  // insert(0, new_head), :97 (the lazy ring of snake_kernel)
+                    if (s.length == 1) ring[s.ring_head] = (uint16_t)head_cell;
+                    if (++s.ring_head == cells) s.ring_head = 0;
+                    ring[s.ring_head] = (uint16_t)new_cell;
+                }
+                s.head_r = nr;
+                s.head_c = nc;
+                if (eat) {  // :101-104
+                    row[new_cell] = 1;  // over the old food, before the rejection loop reads the row
+                    s.length += 1;
+                    rew = 10.0f;
+                    place_food(s, rng, G, body_in(row));
+                    if (s.food_r != FOOD_NONE) row[s.food_r * G + s.food_c] = 2;
+                } else {
+                    row[tail_cell] = 0;  // pop(), :107
+                    row[new_cell] = 1;
+                }
+                s.steps = min(s.steps + 1, 65535);  // :109
+                if (s.steps >= a.max_steps) {
+                    term = 1;  // :112-114, reported as terminated
+                    trunc = a.tl_trunc;
+                }
+            }
+            if (term && a.mode != BENG_AUTORESET_DISABLED) {
+                ended = true;
+                ep_score = s.length - 1;
+                ep_ret = 10 * ep_score - (died ? 10 : 0);
+                ep_len = s.steps + (died ? 1 : 0);  // the death step does not bump `steps`
+                if (a.mode == BENG_AUTORESET_SAME_STEP) reset = true;
+                else s.flags |= FLAG_NEEDS_RESET;
             }
         }
+        if (reset) reset_row(s, rng, row, G);
+        s.ctr = rng.ctr;
+
+        a.core[env] = pack(s);
+        a.io.reward[env] = rew;
+        a.io.terminated[env] = (uint8_t)term;
+        if (a.io.truncated) a.io.truncated[env] = (uint8_t)trunc;
+        if (invalid && a.io.invalid_count) atomicAdd(a.io.invalid_count, 1);
+        if (a.io.score) a.io.score[env] = s.length - 1;
+        if (a.io.snake_length) a.io.snake_length[env] = s.length;
+        if (ended) {
+            if (a.io.ep_return) a.io.ep_return[env] = (float)ep_ret;
+            if (a.io.ep_length) a.io.ep_length[env] = ep_len;
+            if (a.io.ep_score) a.io.ep_score[env] = ep_score;
+        }
+    }
+
+    // episode-done compaction + statistics (as snake_kernel, without its one-tile deferral)
+    const unsigned done_mask = __ballot_sync(0xFFFFFFFFu, ended);
+    if (done_mask) {
+        if (a.io.done_env) {
+            unsigned base = 0;
+            if (lane == 0) base = atomicAdd(a.io.done_count, (unsigned)__popc(done_mask));
+            base = __shfl_sync(0xFFFFFFFFu, base, 0);
+            if (ended) a.io.done_env[base + __popc(done_mask & ((1u << lane) - 1u))] = (int)env;
+        }
+        if (a.io.stats) add_warp_stats(s_stats, done_mask, ended, ep_ret, ep_len, ep_score, lane);
+    }
+    if (a.io.stats) {
+        __syncthreads();
+        flush_stats(a.io.stats, s_stats, tid);
     }
 }
 
@@ -556,15 +742,19 @@ Args make_args(const beng_snake_params *p, const beng_snake_state *st, const ben
     return a;
 }
 
-// beng_snake_step without its public name: `delta` non-null selects the DELTA kernel.
+// beng_snake_step without its public name: `delta` non-null selects the DELTA kernel, `in_place` the patch kernel.
 int step(const beng_snake_params *p, const beng_snake_state *st, const int64_t *actions_dev, const beng_snake_io *io,
-         int64_t n_envs, uint32_t *delta, cudaStream_t stream) {
+         int64_t n_envs, uint32_t *delta, bool in_place, cudaStream_t stream) {
     if (int rc = check_common(p, st, io, n_envs)) return rc;
     if (!actions_dev || !io->reward || !io->terminated) return BENG_ERR_BAD_ARG;
     if ((uintptr_t)actions_dev & 7) return BENG_ERR_BAD_ARG;  // 64-bit action loads (int64, or float32 pairs)
     if (n_envs == 0) return 0;
     Args a = make_args(p, st, io, n_envs);
     a.actions = (const long long *)actions_dev;
+    if (in_place) {
+        const long long blocks = (n_envs + PATCH_THREADS - 1) / PATCH_THREADS;
+        return (int)launch_pdl(snake_patch_kernel, dim3((unsigned)blocks), dim3(PATCH_THREADS), 0, stream, a);
+    }
     if (delta) {
         a.delta = delta;
         return launch<false, true>(a, stream);
@@ -587,7 +777,7 @@ int step_host(const beng_snake_params *p, const beng_snake_state *st, int64_t *a
     const size_t n = (size_t)n_envs, cells = (size_t)p->grid_size * p->grid_size;
     cudaError_t e = cudaMemcpyAsync(actions_dev, actions_host, n * sizeof(int64_t), cudaMemcpyHostToDevice, s);
     if (e != cudaSuccess) return (int)e;
-    if (int rc = step(p, st, actions_dev, io, n_envs, delta_dev, s)) return rc;
+    if (int rc = step(p, st, actions_dev, io, n_envs, delta_dev, false, s)) return rc;
     if (int rc = d2h(delta_host, delta_dev, n * sizeof(uint32_t), s)) return rc;
     if (int rc = d2h(reward_host, io->reward, n * sizeof(float), s)) return rc;
     if (int rc = d2h(terminated_host, io->terminated, n, s)) return rc;
@@ -647,7 +837,12 @@ int beng_snake_reset(const beng_snake_params *p, const beng_snake_state *st, con
 
 int beng_snake_step(const beng_snake_params *p, const beng_snake_state *st, const int64_t *actions_dev,
                     const beng_snake_io *io, int64_t n_envs, void *stream) {
-    return beng::step(p, st, actions_dev, io, n_envs, nullptr, (cudaStream_t)stream);
+    return beng::step(p, st, actions_dev, io, n_envs, nullptr, false, (cudaStream_t)stream);
+}
+
+int beng_snake_step_inplace(const beng_snake_params *p, const beng_snake_state *st, const int64_t *actions_dev,
+                            const beng_snake_io *io, int64_t n_envs, void *stream) {
+    return beng::step(p, st, actions_dev, io, n_envs, nullptr, true, (cudaStream_t)stream);
 }
 
 int beng_snake_step_host(const beng_snake_params *p, const beng_snake_state *st, int64_t *actions_dev,

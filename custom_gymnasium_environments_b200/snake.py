@@ -86,6 +86,8 @@ class BatchedSnakeEnv(_BatchedEnv):
         self._ios = [self._make_io(self.obs, 0), self._make_io(self.obs, 1)]
         self._ios_full = [self._make_io(self.obs, 0, True), self._make_io(self.obs, 1, True)]
         self._info_fresh = True
+        # True while self.obs holds the observation the last reset or step wrote, so that step() may patch it in place
+        self._obs_current = False
 
     # ------------------------------------------------------------------ plumbing
     def _make_io(self, obs: torch.Tensor, parity: int, with_info: bool | None = None) -> "_lib.SnakeIO":
@@ -137,7 +139,12 @@ class BatchedSnakeEnv(_BatchedEnv):
         """SnakeEnvClassic.reset (snake_env.py:49-65) -> (obs, infos).  (The reference ignores `seed` for food
         placement -- it draws from the global `random`, SURVEY.md section 3.1.)"""
         self._info_fresh = True
+        self._obs_current = True  # the reset kernel writes every row
         return self.obs, {"score": self._score, "snake_length": self._snake_length}
+
+    def load_state_dict(self, sd: dict):
+        super().load_state_dict(sd)
+        self._obs_current = False  # `obs` is not part of the state dict
 
     def step(self, actions, out_obs: torch.Tensor | None = None):
         """One step of every env (snake_env.py:67-119) -> (obs, rewards, terminations, truncations, infos).
@@ -145,18 +152,26 @@ class BatchedSnakeEnv(_BatchedEnv):
         `actions`: int64 tensor/array of shape (num_envs,) with values 0..3 (CUDA int64 is zero-copy).
         `out_obs`: optional (num_envs, G, G) int8 CUDA tensor to receive the observations (e.g. a slice
         of a rollout buffer) instead of the persistent `self.obs`.
+
+        Without `out_obs`, `self.obs` is engine state, like the world-builder's grid: while it holds the
+        previous observation, the step patches only the cells that change (`beng_snake_step_inplace`) and
+        reads it back for the self-collision test and the food placement.  Do not write into the returned
+        tensor: clone it, or pass `out_obs=`, to keep a copy you can change.  Every `out_obs=` call
+        composes full rows into that buffer.
         """
         self._require_reset()
         act = as_device_actions(actions, self._actions)
         io, obs = self._next_io(), self.obs
+        fn = "beng_snake_step_inplace" if self._obs_current else "beng_snake_step"
         if out_obs is not None:
             if out_obs.shape != self.obs.shape or out_obs.dtype != torch.int8 or not out_obs.is_contiguous() \
                     or out_obs.device != self.device:
                 raise ValueError("out_obs must be a contiguous int8 CUDA tensor of shape (num_envs, G, G)")
-            io, obs = self._make_io(out_obs, self._parity), out_obs
-        self._mirror_valid = False
-        self._call("beng_snake_step", C.byref(self.params), C.byref(self._state), act.data_ptr(), C.byref(io),
-                   self.num_envs, stream_ptr(self.device))
+            io, obs, fn = self._make_io(out_obs, self._parity), out_obs, "beng_snake_step"
+        self._mirror_valid = self._obs_current = False
+        self._call(fn, C.byref(self.params), C.byref(self._state), act.data_ptr(), C.byref(io), self.num_envs,
+                   stream_ptr(self.device))
+        self._obs_current = obs.data_ptr() == self.obs.data_ptr()
         if self.debug_checks:
             self._raise_on_invalid()
         return obs, self.reward, self.terminated, self.truncated, self._infos()
@@ -184,6 +199,7 @@ class BatchedSnakeEnv(_BatchedEnv):
         """
         delta = self._mirror_begin(delta_obs, sync, copy_obs)
         h = self._host_buffers()
+        self._obs_current = False
         src = self._host_src = host_source(actions, h["_actions"])
         head = (C.byref(self.params), C.byref(self._state), self._actions.data_ptr(), C.byref(self._next_io(True)),
                 self.num_envs, src.data_ptr())
@@ -194,6 +210,7 @@ class BatchedSnakeEnv(_BatchedEnv):
                        *results)
         else:
             self._call("beng_snake_step_host", *head, h["obs"].data_ptr() if copy_obs else None, *results)
+        self._obs_current = True  # both calls compose every row of self.obs (through _ios_full)
         if sync:
             self._sync()
         obs = self._mirror_end(delta, delta_obs, copy_obs)

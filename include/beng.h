@@ -115,8 +115,9 @@ typedef struct beng_snake_io {
                                    snake_env.py:69-70; here such an env is left untouched) */
 } beng_snake_io;
 
-/* Launch shape the step kernel uses for (grid_size, n_envs) on the current device: envs (= threads) per CTA
- * tile, tile buffers per CTA, resident CTAs per SM.  Informational (bench.py names the kernel with it). */
+/* Launch shape the observation-composing kernel of beng_snake_reset / beng_snake_step uses for (grid_size, n_envs) on
+ * the current device: envs (= threads) per CTA tile, tile buffers per CTA, resident CTAs per SM.  Informational
+ * (bench.py names the kernel with it).  beng_snake_step_inplace has no tile: one thread per env, 256 per CTA. */
 int beng_snake_launch_config(int32_t grid_size, int64_t n_envs, int32_t *tile, int32_t *stages, int32_t *ctas_per_sm);
 
 /* Bytes the caller must allocate. */
@@ -133,6 +134,16 @@ int beng_snake_reset(const beng_snake_params *p, const beng_snake_state *st, con
  * + the auto-reset named in p->autoreset_mode, for all n_envs envs, in ONE kernel launch. */
 int beng_snake_step(const beng_snake_params *p, const beng_snake_state *st, const int64_t *actions_dev,
                     const beng_snake_io *io, int64_t n_envs, void *stream);
+
+/* The same step for a caller that keeps the observations in place.  Precondition: io->obs holds, byte for byte, the
+ * observation that the last beng_snake_reset or step of these envs wrote (into any buffer); the function then writes
+ * only the cells that change -- at most two per env, or the whole row on an auto-reset -- and reads io->obs as the
+ * occupancy map of the bodies.  Results, state and statistics are those of beng_snake_step, and so is io->obs
+ * afterwards.  Same arguments, checks and error codes as beng_snake_step; one kernel launch, none when n_envs == 0.
+ * With any other io->obs content the observations, and the self-collision and food placement read from them, are
+ * undefined. */
+int beng_snake_step_inplace(const beng_snake_params *p, const beng_snake_state *st, const int64_t *actions_dev,
+                            const beng_snake_io *io, int64_t n_envs, void *stream);
 
 /* Same step with HOST action / result buffers (what a caller of the reference's numpy API holds):
  * enqueues H2D(actions) -> kernel -> D2H(obs, reward, terminated[, truncated, score, snake_length])
