@@ -318,7 +318,10 @@ __device__ __forceinline__ double warp_sum(double v) {
 //            is live across it), then one thread drains the tile with a bulk asynchronous copy (UBLKCP).
 // What keeps the reference's exact float64 operation order: everything that feeds back into the state (cash, holdings,
 // price walk, psychology, reward).  What does not: the 11 indicator features, float32 outputs checked at rtol 1e-5 /
-// atol 1e-6 (tests/test_crypto_gpu.py); their error against the oracle is ~1e-7.
+// atol 1e-6 (tests/test_crypto_gpu.py); their error against the oracle is ~1e-7, and tests/test_crypto_features_gpu.py
+// bounds it feature by feature.  A window of 20 identical closes (a price pinned at a clip bound) takes the reference's
+// own arithmetic for the Bollinger features, bit for bit (bollinger_constant).  The float32 shortcuts hold for prices
+// in [2^-100, 2^100], the domain check() enforces on the price bounds.
 //
 // In the step, the window comes in through the TMA: a ring of two 38.4 KB shared-memory stages filled by
 // cp.async.bulk.tensor (one [50 slots][32 envs] box of the close tensor and one of the open/high/low/volume tensor per
@@ -659,6 +662,13 @@ struct ObsSmem {
     double *last;           // [20][32] the last 20 closes
 };
 
+// 1 / cur without the division subroutine: float32 reciprocal + one Newton step in float64 (error ~4e-15).  For
+// cur inside the accepted price domain (check(): (float)cur is normal and below __fdividef's 2^126 limit).
+__device__ __forceinline__ double recip_price(double cur) {
+    const double r = (double)__fdividef(1.0f, (float)cur);
+    return __fma_rn(r, __fma_rn(-cur, r, 1.0), r);
+}
+
 // Thread (e, g): slots k = g + 16 i of env `env` -> tile row `dst`, partial sums -> shared memory.
 // DIRECT: read the window with ordinary loads (a reset rewrote it in this call, or there is no TMA stage at all); a
 // separate instantiation, so that the common path carries none of its (predicated-off, but still issued) instructions.
@@ -666,9 +676,7 @@ template <bool DIRECT>
 __device__ __forceinline__ void compose_unit(const CArgs &a, const ObsSmem &sm, int e, int g, long long env,
                                              const int (&slot_of)[OBS_PER], uint32_t pitch32, double cur, float4 newest,
                                              float *dst) {
-    // 1 / cur without the division subroutine: float32 reciprocal + one Newton step in float64 (error ~4e-15)
-    double inv_d = (double)__fdividef(1.0f, (float)cur);
-    inv_d = __fma_rn(inv_d, __fma_rn(-cur, inv_d, 1.0), inv_d);
+    const double inv_d = recip_price(cur);
     const float inv_f = (float)inv_d;
     const float4 *so = reinterpret_cast<const float4 *>(sm.stage_o);
     const float4 *go = reinterpret_cast<const float4 *>(a.st.ohlv) + env;
@@ -718,6 +726,38 @@ __device__ __forceinline__ double tree_sum16(F v) {  // sum of v(0..15), depth 4
     return ((a0 + a1) + (a2 + a3)) + ((a4 + a5) + (a6 + a7));
 }
 
+// x / y in float64 for a positive normal y without the IEEE division subroutine, whose slow-path CALL must not appear in
+// finish_unit (see the kernel comment): the hardware's approximate reciprocal as a seed, two Newton steps, and
+// Markstein's final correction, which rounds the quotient correctly unless the exact one lies within a tiny fraction
+// of an ulp of a rounding boundary; the float32 features cast from it cannot tell.
+__device__ __forceinline__ double div_rn_inline(double x, double y) {
+    double r;
+    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(y));
+    r = __fma_rn(r, __fma_rn(-y, r, 1.0), r);
+    r = __fma_rn(r, __fma_rn(-y, r, 1.0), r);
+    const double q = x * r;
+    return __fma_rn(__fma_rn(-y, q, x), r, q);
+}
+
+// Features 257..259 of a window of 20 identical closes c, as the reference computes them (:64-77, np.mean / np.std of
+// 20 copies).  NumPy's pairwise sum of 20 copies is exact for some c (100.0, 30000.0) and not for most others (1000.1):
+// then sma != c and std > 0.  t = c - sma is a few ulps of c, so t^2 and the 20-term sum of squares are exact, std is
+// |t| exactly, upper and lower are sma +- 2|t| exactly, and the features reduce to 0.75 / 0.25 / 0.5 (t > 0 / t < 0 /
+// t == 0), 4|t| / sma and t / sma (tests/test_crypto_features.py holds NumPy to this closed form).  Short on purpose:
+// even when it never runs, a longer branch here costs the step ~4 % (same-box A/B on a B200).
+__device__ __forceinline__ void bollinger_constant(double c, float *dst) {
+    // np_sum_fn over 20 copies, written out: the eight partial sums 2c and their tree (16c) are exact, the four
+    // remaining additions round
+    double s = c * 16.0;
+    s = s + c; s = s + c; s = s + c; s = s + c;
+    const double sma = div_const<20>(s);
+    const double t = c - sma;
+    const double q = div_rn_inline(t, sma);
+    dst[257] = t > 0.0 ? 0.75f : (t < 0.0 ? 0.25f : 0.5f);
+    dst[258] = (float)(4.0 * fabs(q));
+    dst[259] = (float)q;
+}
+
 // Warps 0..3 (lane e = env): the 11 features behind the window, features 250..260 of row `dst`.
 __device__ __forceinline__ void finish_unit(const ObsSmem &sm, int e, int g, float4 port, float *dst) {
     if (g == 0) {  // MACD(12, 26, 9) normalised by the close range, :538-547
@@ -746,11 +786,12 @@ __device__ __forceinline__ void finish_unit(const ObsSmem &sm, int e, int g, flo
         const double sl = np_sum_fn([&](int i) { const double d = delta(i); return d < 0 ? -d : 0.0; }, 14);
         dst[253] = (sl != 0) ? __fdividef((float)sg, (float)(sg + sl)) : 1.0f;
     } else if (g == 2) {  // Bollinger(20, 2 sigma, population std), :64-77 and :550-554
-        // Mean and variance of the DIFFERENCES to the newest close (exact subtractions): a window of identical closes
-        // -- a price pinned at the clip bound -- gives sma == close and sd == 0 exactly, like the reference, and the sums
-        // are 4-deep trees instead of NumPy's 8-deep pairwise chains.  div_const, not `/`: the division subroutine's
-        // slow-path CALL would force every value live across it -- the prefetched window of the next unit -- into
-        // local memory.
+        // Mean and variance of the DIFFERENCES to the newest close (exact subtractions), so the sums are 4-deep trees
+        // instead of NumPy's 8-deep pairwise chains.  div_const, not `/`: the division subroutine's slow-path CALL
+        // would force every value live across it -- the prefetched window of the next unit -- into local memory.
+        // The variance goes to float32 scaled by a power of two to the price's magnitude (var / 4^e, cur / 2^e in
+        // [1, 2)), so the band holds for every price of the accepted domain, and sd is scaled back exactly.  A window of identical closes (a price pinned at a clip bound)
+        // has var == 0 exactly; it takes the reference's arithmetic instead (bollinger_constant).
         const double *wl = sm.last + e;
         const double cur = wl[(C3_LAST - 1) * C3_SUB];
         auto dv = [&](int i) { return wl[i * C3_SUB] - cur; };
@@ -758,14 +799,21 @@ __device__ __forceinline__ void finish_unit(const ObsSmem &sm, int e, int g, flo
         const double mean_d = div_const<20>(s);
         auto sq = [&](int i) { const double t = dv(i) - mean_d; return t * t; };
         const double var = div_const<20>(tree_sum16(sq) + ((sq(16) + sq(17)) + (sq(18) + sq(19))));
-        const float var_f = (float)var;
-        const double sd = (double)(var_f > 0.0f ? var_f * rsqrtf(var_f) : 0.0f);  // float32 accuracy: it only scales features
-        const double sma = cur + mean_d;
-        const double upper = sma + (2 * sd), lower = sma - (2 * sd);
-        const float width = (float)(upper - lower), mid = (float)sma;
-        dst[257] = (upper > lower) ? __fdividef((float)(cur - lower), width) : 0.5f;
-        dst[258] = (sma > 0) ? __fdividef(width, mid) : 0.0f;
-        dst[259] = (sma > 0) ? __fdividef((float)-mean_d, mid) : 0.0f;  // (cur - sma) / sma
+        if (var > 0.0) {
+            // 2^-2e and 2^e for the binary exponent e of cur (cur / 2^e in [1, 2)), built from its bits: exact scalings
+            const int ex = (__double2hiint(cur) >> 20) - 1023;
+            const double down2 = __hiloint2double((1023 - 2 * ex) << 20, 0), up = __hiloint2double((1023 + ex) << 20, 0);
+            const float var_f = (float)(var * down2);
+            const double sd = (double)(var_f > 0.0f ? var_f * rsqrtf(var_f) : 0.0f) * up;  // float32 accuracy: it only scales features
+            const double sma = cur + mean_d;
+            const double upper = sma + (2 * sd), lower = sma - (2 * sd);
+            const float width = (float)(upper - lower), mid = (float)sma;
+            dst[257] = (upper > lower) ? __fdividef((float)(cur - lower), width) : 0.5f;
+            dst[258] = (sma > 0) ? __fdividef(width, mid) : 0.0f;
+            dst[259] = (sma > 0) ? __fdividef((float)-mean_d, mid) : 0.0f;  // (cur - sma) / sma
+        } else {
+            bollinger_constant(cur, dst);
+        }
     } else if (g == 3) {  // portfolio features :519-527, psychology :559
         dst[250] = port.x;
         dst[251] = port.y;
@@ -1074,6 +1122,10 @@ int check(const beng_crypto_params *p, const beng_crypto_state *st, const beng_c
     if (p->window_head < 0 || p->window_head >= HIST) return BENG_ERR_BAD_ARG;
     if (p->autoreset_mode < 0 || p->autoreset_mode > 2 || p->action_type < 0 || p->action_type > 1) return BENG_ERR_BAD_ARG;
     if (p->max_steps < 1 || p->max_steps > 65535) return BENG_ERR_UNSUPPORTED;
+    // Price domain (beng.h): every close lies in [min_price, max_price], so 1.02 x price, volume / price and the float32
+    // reciprocal of the price stay normal floats well below __fdividef's 2^126 limit.  Rejects NaN and infinite
+    // bounds, min_price <= 0 and min_price > max_price (the reference's np.clip would return max_price there).
+    if (!(p->min_price >= 0x1p-100 && p->min_price <= p->max_price && p->max_price <= 0x1p100)) return BENG_ERR_UNSUPPORTED;
     if (n >= (1LL << 26)) return BENG_ERR_UNSUPPORTED;  // 32-bit element offsets in the window addressing (49 * n < 2^32)
     return 0;
 }

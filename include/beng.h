@@ -207,8 +207,8 @@ typedef struct beng_crypto_params {
     double initial_balance;          /* 10000.0 */
     double trading_fee_rate;         /* 0.001 */
     double slippage_rate;            /* 0.0005 */
-    double min_price;                /* 100.0 */
-    double max_price;                /* 100000.0 */
+    double min_price;                /* 100.0    price domain: 2^-100 <= min_price <= max_price <= 2^100, otherwise */
+    double max_price;                /* 100000.0 reset / step return BENG_ERR_UNSUPPORTED (NaN bounds included) */
     double volatility_base;          /* 0.02 */
     double market_psychology_factor; /* 0.1 */
     int32_t max_steps;               /* 1000 (:298) */
