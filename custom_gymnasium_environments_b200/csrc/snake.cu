@@ -11,8 +11,8 @@
 //   * snake_kernel (beng_snake_reset, beng_snake_step, the host-buffer calls) composes every
 //     observation row in full, into any buffer;
 //   * snake_patch_kernel (beng_snake_step_inplace) expects io.obs to hold the previous observation
-//     and writes only the cells that change -- at most two per env, the whole row on a reset -- with
-//     per-thread byte stores; the previous row doubles as the occupancy map (see the kernel).
+//     and writes only what changes -- the 32-byte sectors around at most two cells per env, the whole
+//     row on a reset; the previous row doubles as the occupancy map (see the kernel).
 //
 // snake_kernel:
 //   * one THREAD per env does the integer dynamics out of a 16-byte state record (one LDG.128 /
@@ -30,7 +30,7 @@
 //     list of finished envs.
 //
 // Both are HBM-bound: snake_kernel moves 450 algorithmic bytes per env-step, 400 of them the
-// observation write; snake_patch_kernel about 150 (DESIGN.md section 6e).  There is nothing
+// observation write; snake_patch_kernel about 150 (DESIGN.md sections 6e and 6f).  There is nothing
 // GEMM-shaped here and no tensor-core path is wanted.
 #include <climits>
 #include <cstdint>
@@ -506,9 +506,56 @@ __device__ __forceinline__ void reset_row(Core &s, EnvStream &rng, uint8_t *row,
     row[s.food_r * G + s.food_c] = 2;  // (a length-1 snake always leaves room for food)
 }
 
+// Adds value `v` at byte `o` of 16 bytes held as four words (nothing when o is outside 0..15).
+__device__ __forceinline__ void put_byte(uint32_t (&w)[4], int o, uint32_t v) {
+    const uint32_t q = (uint32_t)o >> 2, bits = v << ((o & 3) * 8);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) w[j] |= q == (uint32_t)j ? bits : 0u;
+}
+
+// Writes the 32-byte sector of `row` that starts at cell `start` (32-byte aligned, inside the row): the body cells `head`
+// and `body` hold 1, `food` holds 2, every other byte 0.  Two 16-byte stores from one thread, each built just before it
+// is stored: one 256-bit store needs all eight words live at once, which costs the kernel spills at its 40 registers.
+__device__ __forceinline__ void store_sector(uint8_t *row, int start, int head, int body, int food) {
+#pragma unroll
+    for (int half = 0; half < 2; ++half) {
+        const int s16 = start + 16 * half;
+        uint32_t w[4] = {0, 0, 0, 0};
+        put_byte(w, head - s16, 1);
+        put_byte(w, body - s16, 1);
+        put_byte(w, food - s16, 2);
+        *reinterpret_cast<uint4 *>(row + s16) = make_uint4(w[0], w[1], w[2], w[3]);
+    }
+}
+
+// The observation writes of a step of a length-1 snake that neither dies nor resets.  The row afterwards is all zeros but
+// for the head (1), the food (2) and, after a meal, the old head (1), so every byte of it is known here: each 32-byte
+// sector holding a changed cell (old head -> 0 and head -> 1 on a move, head -> 1 and food -> 2 on a meal) is written
+// whole, once, instead of with byte stores.  A partly written sector costs a DRAM read of the sector before the write
+// (DESIGN.md section 6b); a whole one does not.  A sector that reaches into a neighbouring env's row keeps the byte
+// store, since that env's thread may be writing its own part of the sector.  The sector bounds come from the row's
+// address: io.obs is only 16-byte aligned and G*G need not be a multiple of 32.
+__device__ __forceinline__ void patch_len1(uint8_t *row, int cells, int old_head, int head, int food, bool ate) {
+    const int mis = (int)((uintptr_t)row & 31);  // the row starts `mis` bytes past a sector boundary
+    const int body = ate ? old_head : -1;
+    const int a = ate ? head : old_head, b = ate ? food : head;  // the two changed cells, and their new values:
+    const uint8_t va = ate ? 1 : 0, vb = ate ? 2 : 1;
+    const int sa = ((a + mis) & ~31) - mis, sb = ((b + mis) & ~31) - mis;  // first cell of their sectors
+    const bool whole_a = sa >= 0 && sa + 32 <= cells, whole_b = sb >= 0 && sb + 32 <= cells;
+    if (whole_a) store_sector(row, sa, head, body, food);
+    else row[a] = va;
+    if (whole_b) {
+        if (sb != sa) store_sector(row, sb, head, body, food);
+    } else {
+        row[b] = vb;
+    }
+}
+
 // 6 CTAs of 256 threads per SM (<= 40 registers, no spills): the kernel is bound by the latency of its two dependent
 // rounds of loads (state + action, then the row byte + tail entry), so resident threads are what it runs on.  Measured on
-// B200 at 1M envs, G = 20: 61.5 us per step against 65.8 us at the 5 CTAs per SM that 46 registers give.
+// B200 at 1M envs, G = 20: 61.5 us per step against 65.8 us at the 5 CTAs per SM that 46 registers give.  Measured shape
+// of the whole-sector writes (DESIGN.md section 6f): two 16-byte stores per sector at these 6 CTAs per SM, 55.6 us per
+// step.  One 256-bit store per sector needs 48 registers for no spills, i.e. 5 CTAs per SM; not timed.
 constexpr int PATCH_THREADS = 256, PATCH_CTAS_PER_SM = 6;
 
 // The step kernel of beng_snake_step_inplace: same dynamics, rewards, flags, state and statistics as snake_kernel, but
@@ -518,7 +565,10 @@ constexpr int PATCH_THREADS = 256, PATCH_CTAS_PER_SM = 6;
 //   * the previous observation is the occupancy map, so self-collision (`new_head in self.snake`, tail included,
 //     snake_env.py:93) is the byte obs[new_cell] == 1 instead of a walk over the ring; the ring is read only for the
 //     tail cell a move of a length >= 2 snake clears, and written only where snake_kernel writes it;
-//   * the food rejection loop after a meal reads the same row, with the new head already written over the old food.
+//   * the food rejection loop after a meal reads the same row, with the new head already written over the old food;
+//   * a step of a length-1 snake (about 91 % of env-steps at G = 20 with random actions) that does not reset writes
+//     the 32-byte sectors holding its changed cells whole, with two 16-byte stores each (patch_len1), and byte stores
+//     only where a sector reaches into a neighbouring row; longer snakes, deaths and resets keep the stores above.
 // The row loads are plain coherent loads (no .nc / __ldg / __restrict__): this kernel writes those bytes itself.
 __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_kernel(const Args a) {
     __shared__ int s_stats[5];  // per-CTA: n_episodes, sum_return, sum_length, sum_score, max_score
@@ -550,6 +600,7 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
         const bool needs_reset = a.mode == BENG_AUTORESET_NEXT_STEP && (s.flags & FLAG_NEEDS_RESET);
         const bool invalid = !needs_reset && (act < 0 || act > 3);  // the env is left untouched (see snake_kernel)
         bool reset = needs_reset;  // action ignored, reward 0, not terminated
+        int len1_old_head = -1;    // >= 0: a length-1 snake moved or ate; its row is written by patch_len1
         if (!needs_reset && !invalid) {
             const int action = (int)act;
             int d = action - s.dir;
@@ -581,13 +632,17 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
                 }
                 s.head_r = nr;
                 s.head_c = nc;
+                const bool len1 = s.length == 1;
+                if (len1) len1_old_head = head_cell;
                 if (eat) {  // :101-104
-                    row[new_cell] = 1;  // over the old food, before the rejection loop reads the row
+                    // The rejection loop reads the row, with the new head marked over the old food.  A length-1 snake
+                    // leaves its row to patch_len1: there the old food's 2 marks the new head just as well.
+                    if (!len1) row[new_cell] = 1;
                     s.length += 1;
                     rew = 10.0f;
                     place_food(s, rng, G, body_in(row));
-                    if (s.food_r != FOOD_NONE) row[s.food_r * G + s.food_c] = 2;
-                } else {
+                    if (!len1 && s.food_r != FOOD_NONE) row[s.food_r * G + s.food_c] = 2;
+                } else if (!len1) {
                     row[tail_cell] = 0;  // pop(), :107
                     row[new_cell] = 1;
                 }
@@ -606,7 +661,10 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
                 else s.flags |= FLAG_NEEDS_RESET;
             }
         }
-        if (reset) reset_row(s, rng, row, G);
+        if (reset) {
+            reset_row(s, rng, row, G);
+            len1_old_head = -1;  // (set here rather than tested below: then it is not live across reset_row)
+        }
         s.ctr = rng.ctr;
 
         a.core[env] = pack(s);
@@ -621,6 +679,8 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
             if (a.io.ep_length) a.io.ep_length[env] = ep_len;
             if (a.io.ep_score) a.io.ep_score[env] = ep_score;
         }
+        if (len1_old_head >= 0)
+            patch_len1(row, cells, len1_old_head, s.head_r * G + s.head_c, s.food_r * G + s.food_c, s.length == 2);
     }
 
     // episode-done compaction + statistics (as snake_kernel, without its one-tile deferral)
