@@ -42,7 +42,7 @@ class CryptoState(C.Structure):
 class CryptoIO(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in (
         "obs", "reward", "terminated", "truncated", "reward64", "portfolio_value", "current_price", "trade_kind",
-        "ep_return_out", "ep_length", "stats")]
+        "ep_return_out", "ep_length", "stats", "window_head_dev")]
 
 
 class TrafficParams(C.Structure):

@@ -102,6 +102,9 @@ class BatchedCryptoTradingEnv(_BatchedEnv):
             self.ep_return = z(n, dt=torch.float64)
             self.ep_length = z(n, dt=torch.int32)
             self.stats = z(4, dt=torch.float64)
+            # {window head, arrivals}: the slot of the newest candle, advanced by the step kernel itself, so that a
+            # step's arguments never change (a CUDA graph can capture it) and no host state moves per step
+            self._head = z(2, dt=torch.int32)
             self._actions = z(n, 2, dt=torch.float32) if action_type == "continuous" else z(n, dt=torch.int64)
         self._state = _lib.CryptoState(self._scal.data_ptr(), self._meta.data_ptr(), self._ep_return.data_ptr(),
                                        self._close.data_ptr(), self._ohlv.data_ptr())
@@ -109,7 +112,7 @@ class BatchedCryptoTradingEnv(_BatchedEnv):
         self._io = _lib.CryptoIO(self.obs.data_ptr(), self.reward.data_ptr(), self.terminated.data_ptr(),
                                  self.truncated.data_ptr(), ptr(self.reward64), ptr(self.portfolio_value),
                                  ptr(self.current_price), ptr(self.trade_kind), self.ep_return.data_ptr(),
-                                 self.ep_length.data_ptr(), self.stats.data_ptr())
+                                 self.ep_length.data_ptr(), self.stats.data_ptr(), self._head.data_ptr())
         self._info_cache = None
 
     # ------------------------------------------------------------------ state views
@@ -145,7 +148,7 @@ class BatchedCryptoTradingEnv(_BatchedEnv):
     def price_history(self) -> torch.Tensor:
         """(n, 50, 5) float64 window, oldest first: open, high, low, close, volume (open/high/low/volume are
         kept in float32 on the device)."""
-        order = [(self.params.window_head + 1 + k) % HISTORY for k in range(HISTORY)]
+        order = (self._head[0].long() + 1 + torch.arange(HISTORY, device=self.device)) % HISTORY
         n = self.num_envs
         close = self._close[order][:, :n]                # (50, n)
         ohlv = self._ohlv[order][:, :n].to(torch.float64)  # (50, n, 4)
@@ -171,12 +174,15 @@ class BatchedCryptoTradingEnv(_BatchedEnv):
     def step(self, actions):
         """One step of every env (:342-398) -> (obs, rewards, terminations, truncations, infos).
         Discrete: int64 (n,) with 0=hold 1=buy 5% 2=buy 20% 3=sell 5% 4=sell 20% (anything else holds, like the
-        reference).  Continuous: float32 (n, 2) = [buy, sell], clipped to [0, 1] x 10 % caps (:408-422)."""
+        reference).  Continuous: float32 (n, 2) = [buy, sell], clipped to [0, 1] x 10 % caps (:408-422).
+
+        One kernel launch with the same arguments every call and no host state that changes per step (the window head
+        lives on the device), so a loop of step() calls with device-resident actions can be captured once with
+        torch.cuda.graph and replayed, interleaved with eager steps as needed."""
         self._require_reset()
         act = as_device_actions(actions, self._actions)
         self._call("beng_crypto_step", C.byref(self.params), C.byref(self._state), act.data_ptr(), C.byref(self._io),
                    self.num_envs, stream_ptr(self.device))
-        self.params.window_head = (self.params.window_head + 1) % HISTORY
         return self.obs, self.reward, self.terminated, self.truncated, self._infos()
 
     def step_host(self, actions, *, copy_obs: bool = True, sync: bool = True):
@@ -188,7 +194,6 @@ class BatchedCryptoTradingEnv(_BatchedEnv):
                    C.byref(self._io), self.num_envs, src.data_ptr(), h["obs"].data_ptr() if copy_obs else None,
                    h["reward"].data_ptr(), h["terminated"].data_ptr(), h["truncated"].data_ptr(),
                    stream_ptr(self.device))
-        self.params.window_head = (self.params.window_head + 1) % HISTORY
         if sync:
             self._sync()
         obs = h["obs"].numpy() if copy_obs else self.obs
@@ -196,11 +201,14 @@ class BatchedCryptoTradingEnv(_BatchedEnv):
 
     # ------------------------------------------------------------------ extras
     def state_dict(self) -> dict:
-        return dict(super().state_dict(), window_head=int(self.params.window_head), config=asdict(self.config))
+        return dict(super().state_dict(), window_head=int(self._head[0].item()), config=asdict(self.config))
 
     def load_state_dict(self, sd: dict):
+        head = int(sd["window_head"])
+        if not 0 <= head < HISTORY:
+            raise ValueError(f"window_head must be in 0..{HISTORY - 1}, got {head}")
         super().load_state_dict(sd)
-        self.params.window_head = int(sd["window_head"])
+        self._head.copy_(torch.tensor([head, 0], dtype=torch.int32))
 
 
 class CryptoTradingEnv(_EnvBase):
@@ -231,7 +239,7 @@ class CryptoTradingEnv(_EnvBase):
 
     def step(self, action):
         v = self._vec
-        cash0, hold0, price0 = self.cash, self.holdings, float(v._close[v.params.window_head, 0].item())
+        cash0, hold0, price0 = self.cash, self.holdings, float(v._close[v._head[0].long(), 0].item())
         if self.action_type == "continuous":
             act = np.asarray(action, dtype=np.float32).reshape(1, 2)
         else:

@@ -51,6 +51,32 @@ __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.p
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
+// ---- launch-uniform state that the launch advances itself -------------------------------------------------------------
+// A value every CTA of a step needs and every step changes (crypto's window head, snake's done-counter parity), kept in
+// device memory instead of in the kernel arguments: the launch then has the same arguments every step, so a launch
+// captured in a CUDA graph is the right program on every replay.  Call once per launch, after pdl_wait(), from every
+// thread of every CTA of a 1-D grid (it contains a __syncthreads()).  Returns *word as it was when the launch started;
+// the last CTA to arrive on *arrivals writes next(value) to *word and rewinds *arrivals to 0 (it must be 0 when the
+// launch starts).  Every CTA arrives only after it holds the value, so no CTA can read the advanced one; the next launch
+// reads *word after its own pdl_wait(), i.e. after this grid has completed and flushed its memory -- with PDL, without
+// it, and across a programmatic edge of a graph alike.
+template <typename Next>
+__device__ __forceinline__ uint32_t grid_uniform_advance(uint32_t *word, uint32_t *arrivals, Next next) {
+    __shared__ uint32_t s_value;
+    if (threadIdx.x == 0) s_value = __ldcg(word);
+    __syncthreads();
+    const uint32_t v = s_value;
+    if (threadIdx.x == 0) {
+        __threadfence();  // this CTA's read of *word is ordered before its arrival
+        if (atomicAdd(arrivals, 1u) == gridDim.x - 1) {
+            __threadfence();  // ... and every other CTA's read before the write below
+            *word = next(v);
+            *arrivals = 0;
+        }
+    }
+    return v;
+}
+
 // Launch `kern<<<grid, block, smem, stream>>>(args...)` with the PDL attribute (BENG_NO_PDL=1 disables it) and count
 // the attempt in g_launch_count.
 template <typename Kern, typename... Args>

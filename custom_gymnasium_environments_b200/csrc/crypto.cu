@@ -12,9 +12,10 @@
 // Design (DESIGN.md section 7; the kernel's own comment below has the details):
 //   * state arrays are [slot/field][env] (env fastest), open/high/low/volume as one 16-byte record per (slot, env),
 //     so every access of a warp is contiguous and 64/128-bit wide;
-//   * the window is a ring over 50 slots with ONE head shared by all envs (params.window_head): a step
-//     overwrites the oldest slot, a reset rewrites all 50 slots in rotation -- heads never diverge between
-//     envs, so the layout stays coalesced whatever the episode boundaries are;
+//   * the window is a ring over 50 slots with ONE head shared by all envs (params.window_head, or the device word
+//     io.window_head_dev that the step advances itself): a step overwrites the oldest slot, a reset rewrites all 50
+//     slots in rotation -- heads never diverge between envs, so the layout stays coalesced whatever the episode
+//     boundaries are;
 //   * money, prices and market state are float64 in the reference's operation order; the closes are kept in float64
 //     (the MACD is a difference of two EMAs of ~5e4-magnitude prices: float32 closes would break the 1e-5
 //     tolerance); open/high/low/volume only feed the observation and are stored and normalised in float32;
@@ -428,7 +429,7 @@ __device__ __forceinline__ unsigned dynamics_phase(const CArgs &a, long long u, 
         long long act_pre = 0;
         float2 actf_pre = make_float2(0.0f, 0.0f);
         if constexpr (!IS_RESET) {
-            price_pre = a.st.close[(long long)a.p.window_head * pitch + env];
+            price_pre = a.st.close[(long long)(head == 0 ? HIST - 1 : head - 1) * pitch + env];  // the newest candle
             if (a.p.action_type == 1) actf_pre = reinterpret_cast<const float2 *>(a.actions)[env];
             else act_pre = reinterpret_cast<const long long *>(a.actions)[env];
         }
@@ -867,6 +868,21 @@ __device__ __forceinline__ void issue_window_loads(uint8_t *smem_raw, int stage,
     tma_load_2d(smem_u32(smem_raw + OFF_STAGE_C + (size_t)stage * STAGE_C), tm_close, env0, 0, bar);
 }
 
+// The window head of this launch, after pdl_wait(), from every thread (contains a __syncthreads()): the slot holding the
+// newest candle before the call, from params.window_head or, when io.window_head_dev is set, from that device word.  A
+// step (ADVANCE) moves the device word on by one slot for the next launch; the caller advances params.window_head.
+template <bool ADVANCE>
+__device__ __forceinline__ int window_head(const CArgs &a) {
+    uint32_t *const dev = reinterpret_cast<uint32_t *>(a.io.window_head_dev);  // {head, arrivals}
+    if (!dev) {
+        __syncthreads();
+        return a.p.window_head;
+    }
+    if constexpr (ADVANCE) return (int)grid_uniform_advance(dev, dev + 1, [](uint32_t h) { return h + 1 == HIST ? 0u : h + 1; });
+    __syncthreads();
+    return (int)__ldcg(dev);
+}
+
 // ---- crypto4: bulk-synchronous -------------------------------------------------------------------------------------
 constexpr size_t C4_OFF_CUR = OFF_COMMON_END;                        // double [512]
 constexpr size_t C4_OFF_NEWX = C4_OFF_CUR + (size_t)OBS_T * 8;       // float4 [512]
@@ -887,22 +903,21 @@ __global__ void __launch_bounds__(OBS_T, 1) crypto4_kernel(const CArgs a) {
     const long long n = a.n;
     const long long n_units = (n + C3_SUB - 1) / C3_SUB;
     const uint32_t pitch32 = (uint32_t)a.pitch;
-    const int head = a.p.window_head;
-    const int oldest = head + 1 == HIST ? 0 : head + 1;
     const double inv_ib = 1.0 / a.p.initial_balance;  // (features divide by it; the product differs by <= 1 ulp of float64)
     // units of this CTA: u(q) = blockIdx.x + gridDim.x * q, q = 0 .. total-1
     const long long total = n_units > blockIdx.x ? (n_units - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
     auto unit_of = [&](long long q) { return (long long)blockIdx.x + (long long)gridDim.x * q; };
 
+    pdl_launch_dependents();  // the next step's grid may become resident as this one drains ...
+    pdl_wait();               // ... and this one touches nothing before the previous step's grid has flushed
+    const int head = window_head<false>(a);
+    const int oldest = head + 1 == HIST ? 0 : head + 1;
     int slot_of[OBS_PER];  // ring slot of this thread's i-th candle (k = wid + 16 i, oldest first)
 #pragma unroll
     for (int i = 0; i < OBS_PER; ++i) {
         const int slot = oldest + wid + OBS_WARPS * i;
         slot_of[i] = slot >= HIST ? slot - HIST : slot;
     }
-    pdl_launch_dependents();  // the next step's grid may become resident as this one drains ...
-    pdl_wait();               // ... and this one touches nothing before the previous step's grid has flushed
-    __syncthreads();
 
 #pragma unroll 1
     for (long long q0 = 0; q0 < total; q0 += OBS_WARPS) {
@@ -979,7 +994,6 @@ __global__ void __launch_bounds__(C5_T, 1) crypto5_kernel(const CArgs a, const _
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const long long n = a.n;
     const long long n_units = (n + C3_SUB - 1) / C3_SUB;
-    const int head = a.p.window_head + 1 == HIST ? 0 : a.p.window_head + 1;
     const long long total = n_units > blockIdx.x ? (n_units - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
     auto unit_of = [&](long long q) { return (long long)blockIdx.x + (long long)gridDim.x * q; };
 
@@ -990,7 +1004,9 @@ __global__ void __launch_bounds__(C5_T, 1) crypto5_kernel(const CArgs a, const _
     }
     pdl_launch_dependents();  // the next step's grid may become resident as this one drains ...
     pdl_wait();               // ... and this one touches nothing before the previous step's grid has flushed
-    __syncthreads();          // (the only CTA-wide barrier: the two roles part ways here)
+    // (the only CTA-wide barrier is in here: the two roles part ways after it)
+    const int newest = window_head<true>(a);
+    const int head = newest + 1 == HIST ? 0 : newest + 1;  // the slot this step's candle goes to
 
     if (wid >= OBS_WARPS) {
         // =================================================================================== dynamics warps
@@ -1119,7 +1135,8 @@ int check(const beng_crypto_params *p, const beng_crypto_state *st, const beng_c
     if (!p || !st || !io || n < 0) return BENG_ERR_BAD_ARG;
     if (!st->scal || !st->meta || !st->ep_return || !st->close || !st->ohlv || !io->obs) return BENG_ERR_BAD_ARG;
     if (((uintptr_t)io->obs & 15) || ((uintptr_t)st->close & 7) || ((uintptr_t)st->ohlv & 15)) return BENG_ERR_BAD_ARG;
-    if (p->window_head < 0 || p->window_head >= HIST) return BENG_ERR_BAD_ARG;
+    if (io->window_head_dev ? ((uintptr_t)io->window_head_dev & 7) != 0 : (p->window_head < 0 || p->window_head >= HIST))
+        return BENG_ERR_BAD_ARG;  // (a device head replaces params.window_head, which is then not read)
     if (p->autoreset_mode < 0 || p->autoreset_mode > 2 || p->action_type < 0 || p->action_type > 1) return BENG_ERR_BAD_ARG;
     if (p->max_steps < 1 || p->max_steps > 65535) return BENG_ERR_UNSUPPORTED;
     // Price domain (beng.h): every close lies in [min_price, max_price], so 1.02 x price, volume / price and the float32

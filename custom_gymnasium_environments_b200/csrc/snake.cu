@@ -113,6 +113,25 @@ __device__ __forceinline__ void place_food(Core &s, EnvStream &rng, int G, Occup
     }
 }
 
+// The finished-env counter of this launch is io.done_count + done_counter(io).  Called after pdl_wait(), from every
+// thread (contains a __syncthreads()); block 0 zeroes the other counter for the next launch.  With
+// io.done_count_next == io.done_count the pointer is the self-managed block {count0, count1, parity, arrivals} of beng.h:
+// this launch counts into count[parity], zeroes count[parity ^ 1] and flips the parity; otherwise the offset is 0 and the
+// caller's two counters are used as they are.  (An offset rather than a pointer: it costs the register-bound patch kernel
+// one register across its body instead of two.)
+__device__ __forceinline__ uint32_t done_counter(const beng_snake_io &io) {
+    uint32_t *const count = io.done_count;
+    uint32_t parity = 0, *next = io.done_count_next;
+    if (count && next == count) {
+        parity = grid_uniform_advance(count + 2, count + 3, [](uint32_t p) { return p ^ 1u; });
+        next = count + (parity ^ 1u);
+    } else {
+        __syncthreads();
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0 && next) *next = 0;
+    return parity;
+}
+
 // Row tests for place_food: a byte of the row (shared or global memory; the kernels write these rows themselves, so
 // the loads are plain coherent ones).
 __device__ __forceinline__ auto body_in(const uint8_t *row) {
@@ -254,8 +273,7 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
     // grid to have completed and flushed before touching anything it wrote (state, counters).
     pdl_launch_dependents();
     pdl_wait();
-    if (blockIdx.x == 0 && tid == 0 && a.io.done_count_next) *a.io.done_count_next = 0;  // for the NEXT step
-    __syncthreads();
+    [[maybe_unused]] const uint32_t done_slot = done_counter(a.io);  // (a reset only zeroes the next counter)
 
     // deferred finished-env list entries of the previous tile (the global atomic's result is consumed one
     // iteration later so that its latency is off the critical path)
@@ -450,7 +468,7 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
             if (done_mask) {
                 if (a.io.done_env) {
                     // one global atomic per warp reserves the slots; the slots are written next iteration
-                    if (lane == 0) pend_base = atomicAdd(a.io.done_count, (unsigned)__popc(done_mask));
+                    if (lane == 0) pend_base = atomicAdd(a.io.done_count + done_slot, (unsigned)__popc(done_mask));
                     pend_mask = done_mask;
                     pend_env = (int)env;
                 }
@@ -582,8 +600,7 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
     if (tid < 5) s_stats[tid] = (tid == 4) ? INT_MIN : 0;
     pdl_launch_dependents();
     pdl_wait();  // the previous step's state, observations and counters are complete from here on
-    if (blockIdx.x == 0 && tid == 0 && a.io.done_count_next) *a.io.done_count_next = 0;  // for the NEXT step
-    __syncthreads();
+    const uint32_t done_slot = done_counter(a.io);
 
     bool ended = false;
     int ep_ret = 0, ep_len = 0, ep_score = 0;
@@ -688,7 +705,7 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
     if (done_mask) {
         if (a.io.done_env) {
             unsigned base = 0;
-            if (lane == 0) base = atomicAdd(a.io.done_count, (unsigned)__popc(done_mask));
+            if (lane == 0) base = atomicAdd(a.io.done_count + done_slot, (unsigned)__popc(done_mask));
             base = __shfl_sync(0xFFFFFFFFu, base, 0);
             if (ended) a.io.done_env[base + __popc(done_mask & ((1u << lane) - 1u))] = (int)env;
         }
@@ -784,6 +801,8 @@ int check_common(const beng_snake_params *p, const beng_snake_state *st, const b
     if (p->autoreset_mode < 0 || p->autoreset_mode > 2) return BENG_ERR_BAD_ARG;
     if (((uintptr_t)st->core & 15) || ((uintptr_t)io->obs & 15)) return BENG_ERR_BAD_ARG;
     if (io->done_env && !io->done_count) return BENG_ERR_BAD_ARG;
+    if (io->done_count && io->done_count_next == io->done_count && ((uintptr_t)io->done_count & 15))
+        return BENG_ERR_BAD_ARG;  // the self-managed counter block (beng.h)
     return 0;
 }
 

@@ -75,36 +75,39 @@ class BatchedSnakeEnv(_BatchedEnv):
             self.ep_return = torch.zeros(n, dtype=torch.float32, device=dev)
             self.ep_length = torch.zeros(n, dtype=torch.int32, device=dev)
             self.ep_score = torch.zeros(n, dtype=torch.int32, device=dev)
-            self._done_counts = torch.zeros(2, dtype=torch.int32, device=dev)  # ping-pong, zeroed in-kernel
-            self._parity = 0
+            # {count0, count1, parity, arrivals}: each launch counts into count[parity], zeroes the other counter and
+            # flips the parity itself (beng.h), so a step's arguments never change and a CUDA graph can capture it
+            self._done_counts = torch.zeros(4, dtype=torch.int32, device=dev)
+            self._parity = 0  # (not used by the class; callers that drive the C functions through _make_io flip it)
             self.done_env = torch.zeros(n, dtype=torch.int32, device=dev)
             self.stats = torch.zeros(5, dtype=torch.int64, device=dev)
             self.invalid_count = torch.zeros(1, dtype=torch.int32, device=dev)
             self._actions = torch.zeros(n, dtype=torch.int64, device=dev)
             self.stats[4] = torch.iinfo(torch.int64).min
         self._state = _lib.SnakeState(self._core.data_ptr(), self._ring.data_ptr())
-        self._ios = [self._make_io(self.obs, 0), self._make_io(self.obs, 1)]
-        self._ios_full = [self._make_io(self.obs, 0, True), self._make_io(self.obs, 1, True)]
+        self._ios = [self._make_io(self.obs)]
+        self._ios_full = [self._make_io(self.obs, with_info=True)]
         self._info_fresh = True
         # True while self.obs holds the observation the last reset or step wrote, so that step() may patch it in place
         self._obs_current = False
 
     # ------------------------------------------------------------------ plumbing
-    def _make_io(self, obs: torch.Tensor, parity: int, with_info: bool | None = None) -> "_lib.SnakeIO":
+    def _make_io(self, obs: torch.Tensor, parity: int = 0, with_info: bool | None = None) -> "_lib.SnakeIO":
+        """The io block of a launch writing `obs`.  Both counter pointers name the self-managed counter block, so
+        `parity` is not used: the kernels pick the counter themselves."""
         cnt = self._done_counts.data_ptr()
         info = self.materialize_info if with_info is None else with_info
         return _lib.SnakeIO(obs.data_ptr(), self.reward.data_ptr(), self.terminated.data_ptr(),
                             self.truncated.data_ptr(), self._score.data_ptr() if info else None,
                             self._snake_length.data_ptr() if info else None,
                             self.ep_return.data_ptr(), self.ep_length.data_ptr(), self.ep_score.data_ptr(),
-                            cnt + 4 * parity, self.done_env.data_ptr(), cnt + 4 * (1 - parity),
+                            cnt, self.done_env.data_ptr(), cnt,
                             self.stats.data_ptr(), self.invalid_count.data_ptr())
 
     def _next_io(self, full: bool = False):
-        """The io block of this step; the two finished-env counters alternate (the kernel zeroes the other)."""
-        self._parity ^= 1
+        """The io block of this step (`full`: with the info outputs)."""
         self._info_fresh = full or self.materialize_info
-        return (self._ios_full if full else self._ios)[self._parity]
+        return (self._ios_full if full else self._ios)[0]
 
     @property
     def snake_length(self) -> torch.Tensor:
@@ -122,7 +125,9 @@ class BatchedSnakeEnv(_BatchedEnv):
 
     @property
     def done_count(self) -> torch.Tensor:
-        return self._done_counts[self._parity:self._parity + 1]
+        """(1,) int32: the number of envs the last step listed in `done_env`, read lazily on the device (count[parity ^ 1]
+        of the counter block; no synchronisation)."""
+        return self._done_counts[(self._done_counts[2:3] ^ 1).long()]
 
     def _infos(self):
         info = LazyInfos({"episode": {"r": self.ep_return, "l": self.ep_length, "score": self.ep_score},
@@ -158,6 +163,13 @@ class BatchedSnakeEnv(_BatchedEnv):
         reads it back for the self-collision test and the food placement.  Do not write into the returned
         tensor: clone it, or pass `out_obs=`, to keep a copy you can change.  Every `out_obs=` call
         composes full rows into that buffer.
+
+        One kernel launch with the same arguments every call (the finished-env counters are managed on the
+        device), so a loop of step() calls with device-resident actions can be captured once with
+        torch.cuda.graph and replayed.  Captured steps without `out_obs` patch `self.obs` in place: replay
+        them only while `self.obs` is current, i.e. not after a step(out_obs=...), step_host(copy_obs=False)
+        or load_state_dict() (eager step() calls between replays are fine).  debug_checks=True reads the
+        invalid-action count back, which synchronises and cannot be captured.
         """
         self._require_reset()
         act = as_device_actions(actions, self._actions)
@@ -167,7 +179,7 @@ class BatchedSnakeEnv(_BatchedEnv):
             if out_obs.shape != self.obs.shape or out_obs.dtype != torch.int8 or not out_obs.is_contiguous() \
                     or out_obs.device != self.device:
                 raise ValueError("out_obs must be a contiguous int8 CUDA tensor of shape (num_envs, G, G)")
-            io, obs, fn = self._make_io(out_obs, self._parity), out_obs, "beng_snake_step"
+            io, obs, fn = self._make_io(out_obs), out_obs, "beng_snake_step"
         self._mirror_valid = self._obs_current = False
         self._call(fn, C.byref(self.params), C.byref(self._state), act.data_ptr(), C.byref(io), self.num_envs,
                    stream_ptr(self.device))

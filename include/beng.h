@@ -108,6 +108,12 @@ typedef struct beng_snake_io {
     int32_t *done_env;      /* [n_envs] LOCAL env indices */
     uint32_t *done_count_next; /* [1] nullable; zeroed BY this launch so it can serve as `done_count` of the
                                   next step (ping-pong two counters: no memset launch between steps) */
+    /* Self-managed counters: done_count_next == done_count (non-NULL) means that done_count points to
+     * uint32_t[4] = {count0, count1, parity, arrivals}, 16-byte aligned, zero before the first call.  Every step and
+     * reset launch then counts its finished envs into count[parity], zeroes count[parity ^ 1] and flips parity for
+     * the next launch; `arrivals` is the launch's scratch counter and is 0 again when it ends.  The counter of the
+     * last launch is count[parity ^ 1].  A step's arguments are then the same every call (a CUDA graph captures it
+     * once and replays it), and no host state changes per step.  Every other combination is the contract above. */
     /* running episode statistics, integer (exact, order independent):
      * {n_episodes, sum_return, sum_length, sum_score, max_score} */
     int64_t *stats;         /* [5] accumulated across steps; caller zeroes / all-reduces */
@@ -216,7 +222,8 @@ typedef struct beng_crypto_params {
     int32_t action_type;             /* 0 = Discrete(5) int64[n]; 1 = Box(-1,1,(2,)) float32[n][2]  (:288-296) */
     int32_t window_head;             /* slot (0..49) holding the NEWEST candle of every env before this call.
                                         A step writes the new candle to (window_head+1)%50 -- the caller then
-                                        advances window_head by one; a reset leaves it unchanged. */
+                                        advances window_head by one; a reset leaves it unchanged.  Ignored when
+                                        io->window_head_dev is set (the head then lives on the device). */
     int32_t time_limit_truncation;   /* 1: also set `truncated` when current_step reaches max_steps (gym.make's
                                         TimeLimit, crypto_trading_env.py:739-743); 0: never (raw class, :388) */
     int32_t reserved;
@@ -251,6 +258,14 @@ typedef struct beng_crypto_io {
     double *ep_return_out;   /* [n] */
     int32_t *ep_length;      /* [n] */
     double *stats;           /* [4] running {n_episodes, sum_return, sum_length, sum_final_value}; nullable */
+    /* State that the launch itself advances, so that a step's arguments are the same every call (a CUDA graph
+     * captures a step once and replays it):
+     * NULL     : params.window_head is the head, as documented there (the caller advances it).
+     * non-NULL : int32_t[2] = {head, arrivals}, 8-byte aligned, head 0..49 and arrivals 0 before the first call.
+     *            params.window_head is then ignored (not validated).  beng_crypto_step reads the head and leaves it
+     *            advanced by one slot (mod 50) for the next call; beng_crypto_reset reads it and leaves it as it is.
+     *            `arrivals` is the launch's scratch counter and is 0 again when the launch ends. */
+    int32_t *window_head_dev;
 } beng_crypto_io;
 
 /* Row pitch (in envs) of beng_crypto_state.close / .ohlv for a batch of n_envs. */
