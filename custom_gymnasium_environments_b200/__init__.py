@@ -8,11 +8,12 @@ from ._build import build_library
 from .builder import BatchedWorldBuilderEnv, WorldBuilderEnv
 from .climate import BatchedSmartClimateEnv, SmartClimateEnv
 from .crypto import BatchedCryptoTradingEnv, CryptoTradingEnv, TradingConfig
+from .normalize import RunningMeanStd, VecNormalize
 from .snake import BatchedSnakeEnv, SnakeEnvClassic
 from .traffic import BatchedTrafficManagementEnv, TrafficManagementEnv
 from .registration import register_all
 
-__all__ = ["BatchedSnakeEnv", "SnakeEnvClassic", "BatchedCryptoTradingEnv", "CryptoTradingEnv", "TradingConfig", "BatchedSmartClimateEnv", "SmartClimateEnv", "BatchedWorldBuilderEnv", "WorldBuilderEnv", "BatchedTrafficManagementEnv", "TrafficManagementEnv", "build_library", "register_all", "_lib"]
+__all__ = ["BatchedSnakeEnv", "SnakeEnvClassic", "BatchedCryptoTradingEnv", "CryptoTradingEnv", "TradingConfig", "BatchedSmartClimateEnv", "SmartClimateEnv", "BatchedWorldBuilderEnv", "WorldBuilderEnv", "BatchedTrafficManagementEnv", "TrafficManagementEnv", "VecNormalize", "RunningMeanStd", "build_library", "register_all", "_lib"]
 __version__ = "0.1.0"
 
 register_all()

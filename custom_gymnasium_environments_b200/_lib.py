@@ -90,6 +90,19 @@ class BuilderIO(C.Structure):
                                           "invalid_count")]
 
 
+class NormalizeParams(C.Structure):
+    _fields_ = [("clip_obs", C.c_double), ("clip_reward", C.c_double), ("epsilon", C.c_double), ("gamma", C.c_double),
+                ("flags", C.c_uint32), ("reserved", C.c_int32)]
+
+
+class NormalizeIO(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("obs", "reward", "terminated", "truncated", "returns", "obs_rms", "ret_rms",
+                                          "workspace", "obs_out", "reward_out")]
+
+
+NORM_OBS, NORM_REWARD, NORM_UPDATE = 1, 2, 4
+
+
 # name -> (restype, argtypes); also the list of symbols include/beng.h declares (tests check it).
 SIGNATURES = {
     "beng_version": (C.c_int, []),
@@ -142,6 +155,9 @@ SIGNATURES = {
     "beng_builder_apply_obs_delta": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32]),
     "beng_snake_export_state": (C.c_int, [C.POINTER(SnakeParams), C.POINTER(SnakeState), C.c_int64] +
                                 [C.c_void_p] * 10),
+    "beng_normalize_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32]),
+    "beng_normalize": (C.c_int, [C.POINTER(NormalizeParams), C.POINTER(NormalizeIO), C.c_int64, C.c_int32,
+                                 C.c_void_p]),
 }
 
 

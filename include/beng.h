@@ -503,6 +503,58 @@ int beng_builder_step_host_delta(const beng_builder_params *p, const beng_builde
 int beng_builder_apply_obs_delta(const uint32_t *delta_host, int8_t *grid_host, int64_t n_envs, int32_t grid_size,
                                  int32_t n_threads);
 
+/* ------------------------------------------------------------------------------------------
+ * Running normalization of observations and rewards (Stable-Baselines3 VecNormalize semantics), for any env's
+ * float32 [n][dim] observations and float32 [n] rewards.  INTEGRATION.md section "Normalizing observations and rewards"
+ * states the semantics.
+ * ------------------------------------------------------------------------------------------ */
+
+#define BENG_NORM_OBS 1u    /* normalize io->obs into io->obs_out (skipped when obs_out is NULL) */
+#define BENG_NORM_REWARD 2u /* normalize io->reward into io->reward_out (nullable) and zero io->returns where
+                               terminated or truncated is set */
+#define BENG_NORM_UPDATE 4u /* training: first update obs_rms with the batch (with BENG_NORM_OBS) and
+                               returns = returns * gamma + reward, then ret_rms with the new returns (with BENG_NORM_REWARD) */
+
+typedef struct beng_normalize_params {
+    double clip_obs;    /* obs_out = clip((obs - mean) / sqrt(var + epsilon), -clip_obs, clip_obs) in float64, as float32 */
+    double clip_reward; /* reward_out = clip(reward / sqrt(ret_var + epsilon), -clip_reward, clip_reward) */
+    double epsilon;
+    double gamma;
+    uint32_t flags;     /* BENG_NORM_* */
+    int32_t reserved;
+} beng_normalize_params;
+
+/* Running statistics records (float64, caller-owned, initialised to mean 0, var 1, count 1e-4):
+ *   obs_rms : double[2 * dim + 1] = mean[dim], var[dim], count
+ *   ret_rms : double[3]           = mean, var, count */
+typedef struct beng_normalize_io {
+    const float *obs;          /* [n][dim] row-major, 4-byte aligned (rows need not be 16-byte multiples) */
+    const float *reward;       /* [n] */
+    const uint8_t *terminated; /* [n] nullable (no env finished) */
+    const uint8_t *truncated;  /* [n] nullable */
+    double *returns;           /* [n] discounted running return of every env */
+    double *obs_rms;
+    double *ret_rms;
+    void *workspace;           /* beng_normalize_workspace_bytes(n, dim) bytes, 16-byte aligned, zero before the first
+                                  call; its arrival counter is 0 again when each call's launches end */
+    float *obs_out;            /* [n][dim] nullable; must not overlap obs */
+    float *reward_out;         /* [n] nullable */
+} beng_normalize_io;
+
+/* Workspace bytes beng_normalize needs for (n_envs, dim); 0 for n_envs < 0 or dim < 1. */
+size_t beng_normalize_workspace_bytes(int64_t n_envs, int32_t dim);
+
+/* One update / normalize of n_envs envs.  With BENG_NORM_UPDATE: two launches, a moments pass (every CTA sums its rows
+ * shifted by row 0 in float64; the last CTA to arrive adds the partials in CTA order and merges the batch into obs_rms /
+ * ret_rms with Chan's update) and an apply pass; without it only the apply pass.  None when n_envs == 0 or there is
+ * nothing to write.  The statistics depend only on the inputs and (n_envs, dim): bit-identical run to run, on every
+ * device and from a CUDA graph.  Pointers the flags need are checked (non-NULL, aligned: float / uint8 4 / 1 bytes,
+ * double 8) before anything launches: BENG_ERR_BAD_ARG, also for n_envs < 0, dim < 1, unknown flags and negative or NaN
+ * clip / epsilon / gamma.  obs and obs_rms are read only with BENG_NORM_OBS, dim is then the observation width;
+ * reward / returns / ret_rms only with BENG_NORM_REWARD. */
+int beng_normalize(const beng_normalize_params *p, const beng_normalize_io *io, int64_t n_envs, int32_t dim,
+                   void *stream);
+
 #ifdef __cplusplus
 }
 #endif
