@@ -123,6 +123,15 @@ __device__ __forceinline__ long long ld_stream_s64(const long long *p) {
     asm volatile("ld.global.L1::no_allocate.s64 %0, [%1];" : "=l"(r) : "l"(p));
     return r;
 }
+// ... and the same load with an L2 evict-first policy, for an input that no later launch reads again (a step's action
+// tensor): its lines are the first the L2 gives up, so they do not push out lines the next launch would hit.
+__device__ __forceinline__ long long ld_once_s64(const long long *p) {
+    uint64_t policy;
+    long long r;
+    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(policy));
+    asm volatile("ld.global.L1::no_allocate.L2::cache_hint.s64 %0, [%1], %2;" : "=l"(r) : "l"(p), "l"(policy));
+    return r;
+}
 
 // Correctly rounded x / B (float64) for a compile-time integer B without the IEEE division subroutine (a ~60-instruction
 // call on sm_100a): y = RN(1 / B), q = RN(x * y), r = x - B * q exactly (FMA), result RN(q + r * y) -- Markstein's

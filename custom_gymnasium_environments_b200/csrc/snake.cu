@@ -546,17 +546,20 @@ __device__ __forceinline__ void store_sector(uint8_t *row, int start, int head, 
     }
 }
 
-// The observation writes of a step of a length-1 snake that neither dies nor resets.  The row afterwards is all zeros but
-// for the head (1), the food (2) and, after a meal, the old head (1), so every byte of it is known here: each 32-byte
-// sector holding a changed cell (old head -> 0 and head -> 1 on a move, head -> 1 and food -> 2 on a meal) is written
-// whole, once, instead of with byte stores.  A partly written sector costs a DRAM read of the sector before the write
-// (DESIGN.md section 6b); a whole one does not.  A sector that reaches into a neighbouring env's row keeps the byte
-// store, since that env's thread may be writing its own part of the sector.  The sector bounds come from the row's
-// address: io.obs is only 16-byte aligned and G*G need not be a multiple of 32.
-__device__ __forceinline__ void patch_len1(uint8_t *row, int cells, int old_head, int head, int food, bool ate) {
+// The observation writes of a step that neither dies nor resets, of a snake whose whole row is known in registers: a
+// length-1 snake (move or meal) and a length-2 snake that does not eat.  The row afterwards is all zeros but for the
+// head (1), the food (2) and, unless a length-1 snake moved, the old head (1).  Each 32-byte sector holding a changed
+// cell -- `clear` -> 0 and head -> 1 on a move (`clear` is the old head of a length-1 snake, the tail of a length-2
+// one), head -> 1 and food -> 2 on a length-1 meal (`clear` < 0) -- is written whole, once, instead of with byte
+// stores.  A partly written sector costs a DRAM read of the sector before the write (DESIGN.md section 6b); a whole one
+// does not.  A sector that reaches into a neighbouring env's row keeps the byte store, since that env's thread may be
+// writing its own part of the sector.  The sector bounds come from the row's address: io.obs is only 16-byte aligned
+// and G*G need not be a multiple of 32.
+__device__ __forceinline__ void patch_known_row(uint8_t *row, int cells, int old_head, int clear, int head, int food) {
     const int mis = (int)((uintptr_t)row & 31);  // the row starts `mis` bytes past a sector boundary
-    const int body = ate ? old_head : -1;
-    const int a = ate ? head : old_head, b = ate ? food : head;  // the two changed cells, and their new values:
+    const bool ate = clear < 0;
+    const int body = clear != old_head ? old_head : -1;
+    const int a = ate ? head : clear, b = ate ? food : head;  // the two changed cells, and their new values:
     const uint8_t va = ate ? 1 : 0, vb = ate ? 2 : 1;
     const int sa = ((a + mis) & ~31) - mis, sb = ((b + mis) & ~31) - mis;  // first cell of their sectors
     const bool whole_a = sa >= 0 && sa + 32 <= cells, whole_b = sb >= 0 && sb + 32 <= cells;
@@ -573,7 +576,7 @@ __device__ __forceinline__ void patch_len1(uint8_t *row, int cells, int old_head
 // rounds of loads (state + action, then the row byte + tail entry), so resident threads are what it runs on.  Measured on
 // B200 at 1M envs, G = 20: 61.5 us per step against 65.8 us at the 5 CTAs per SM that 46 registers give.  Measured shape
 // of the whole-sector writes (DESIGN.md section 6f): two 16-byte stores per sector at these 6 CTAs per SM, 55.6 us per
-// step.  One 256-bit store per sector needs 48 registers for no spills, i.e. 5 CTAs per SM; not timed.
+// step.  One 256-bit store per sector compiles to 46 registers without spills, i.e. 5 CTAs per SM; not timed.
 constexpr int PATCH_THREADS = 256, PATCH_CTAS_PER_SM = 6;
 
 // The step kernel of beng_snake_step_inplace: same dynamics, rewards, flags, state and statistics as snake_kernel, but
@@ -581,12 +584,19 @@ constexpr int PATCH_THREADS = 256, PATCH_CTAS_PER_SM = 6;
 // (move: old tail -> 0, new head -> 1; eat: new head -> 1, new food -> 2; death / invalid action: nothing; reset: clear,
 // head -> 1, food -> 2 -- the order of the BENG_OBS_DELTA records).  One thread per env and no shared-memory tile:
 //   * the previous observation is the occupancy map, so self-collision (`new_head in self.snake`, tail included,
-//     snake_env.py:93) is the byte obs[new_cell] == 1 instead of a walk over the ring; the ring is read only for the
-//     tail cell a move of a length >= 2 snake clears, and written only where snake_kernel writes it;
+//     snake_env.py:93) is the byte obs[new_cell] == 1 instead of a walk over the ring (for length 2, new_cell == tail);
+//     the ring is read only for the tail cell a move of a length >= 2 snake clears, and written only where
+//     snake_kernel writes it;
 //   * the food rejection loop after a meal reads the same row, with the new head already written over the old food;
-//   * a step of a length-1 snake (about 91 % of env-steps at G = 20 with random actions) that does not reset writes
-//     the 32-byte sectors holding its changed cells whole, with two 16-byte stores each (patch_len1), and byte stores
-//     only where a sector reaches into a neighbouring row; longer snakes, deaths and resets keep the stores above.
+//   * a step that does not reset of a length-1 snake (about 91 % of env-steps at G = 20 with random actions), or a
+//     non-eating move of a length-2 snake (about 6 %), writes the 32-byte sectors holding its changed cells whole, with
+//     two 16-byte stores each (patch_known_row), and byte stores only where a sector reaches into a neighbouring row;
+//     longer snakes, length-2 meals, deaths and resets keep the stores above;
+//   * with the self-managed counter block, the launch's parity reverses the order of the CTAs' env tiles every other
+//     launch, so the envs a step writes last are the ones the next step reads and rewrites first, while their state
+//     records and observation sectors may still be in L2 (DESIGN.md section 6h); callers with their own two counters
+//     keep the ascending order;
+//   * the action tensor is read once per step and loaded with an L2 evict-first policy.
 // The row loads are plain coherent loads (no .nc / __ldg / __restrict__): this kernel writes those bytes itself.
 __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_kernel(const Args a) {
     __shared__ int s_stats[5];  // per-CTA: n_episodes, sum_return, sum_length, sum_score, max_score
@@ -594,18 +604,20 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
     const int lane = tid & 31;
     const int G = a.G;
     const int cells = G * G;
-    const long long env = (long long)blockIdx.x * PATCH_THREADS + tid;
-    const bool active = env < a.n_envs;
 
     if (tid < 5) s_stats[tid] = (tid == 4) ? INT_MIN : 0;
     pdl_launch_dependents();
     pdl_wait();  // the previous step's state, observations and counters are complete from here on
     const uint32_t done_slot = done_counter(a.io);
+    const unsigned tile = done_slot ? gridDim.x - 1 - blockIdx.x : blockIdx.x;
+    // (32-bit index math, n_envs < 2^32: a 64-bit product costs this register-bound kernel a spill)
+    const long long env = tile * PATCH_THREADS + tid;
+    const bool active = env < a.n_envs;
 
     bool ended = false;
     int ep_ret = 0, ep_len = 0, ep_score = 0;
     if (active) {
-        const long long act = ld_stream_s64(a.actions + env);
+        const long long act = ld_once_s64(a.actions + env);
         Core s = unpack(ld_stream_u4(a.core + env));
         uint8_t *row = reinterpret_cast<uint8_t *>(a.io.obs) + env * cells;
         uint16_t *ring = a.ring + env * cells;
@@ -617,7 +629,8 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
         const bool needs_reset = a.mode == BENG_AUTORESET_NEXT_STEP && (s.flags & FLAG_NEEDS_RESET);
         const bool invalid = !needs_reset && (act < 0 || act > 3);  // the env is left untouched (see snake_kernel)
         bool reset = needs_reset;  // action ignored, reward 0, not terminated
-        int len1_old_head = -1;    // >= 0: a length-1 snake moved or ate; its row is written by patch_len1
+        int known_old_head = -1;   // >= 0: the row is written by patch_known_row, with this old head ...
+        int known_clear = -1;      // ... and this cell cleared (< 0: a length-1 meal)
         if (!needs_reset && !invalid) {
             const int action = (int)act;
             int d = action - s.dir;
@@ -634,7 +647,8 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
             int tail_cell = head_cell;
             if (!wall && s.length > 1) {
                 tail_cell = ring[tail_index(s, cells)];  // (both loads are issued before either is used)
-                self_hit = row[new_cell] == 1;
+                // a length-2 body is the head, which the new head never is, and the tail: no row load
+                self_hit = s.length == 2 ? new_cell == tail_cell : row[new_cell] == 1;
             }
             const bool died = wall || self_hit;
             if (died) {
@@ -650,16 +664,20 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
                 s.head_r = nr;
                 s.head_c = nc;
                 const bool len1 = s.length == 1;
-                if (len1) len1_old_head = head_cell;
+                const bool known = len1 || (s.length == 2 && !eat);
+                if (known) {
+                    known_old_head = head_cell;
+                    known_clear = eat ? -1 : tail_cell;  // (a length-1 snake's tail_cell is its old head)
+                }
                 if (eat) {  // :101-104
                     // The rejection loop reads the row, with the new head marked over the old food.  A length-1 snake
-                    // leaves its row to patch_len1: there the old food's 2 marks the new head just as well.
+                    // leaves its row to patch_known_row: there the old food's 2 marks the new head just as well.
                     if (!len1) row[new_cell] = 1;
                     s.length += 1;
                     rew = 10.0f;
                     place_food(s, rng, G, body_in(row));
                     if (!len1 && s.food_r != FOOD_NONE) row[s.food_r * G + s.food_c] = 2;
-                } else if (!len1) {
+                } else if (!known) {
                     row[tail_cell] = 0;  // pop(), :107
                     row[new_cell] = 1;
                 }
@@ -680,7 +698,7 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
         }
         if (reset) {
             reset_row(s, rng, row, G);
-            len1_old_head = -1;  // (set here rather than tested below: then it is not live across reset_row)
+            known_old_head = -1;  // (set here rather than tested below: then it is not live across reset_row)
         }
         s.ctr = rng.ctr;
 
@@ -696,8 +714,8 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
             if (a.io.ep_length) a.io.ep_length[env] = ep_len;
             if (a.io.ep_score) a.io.ep_score[env] = ep_score;
         }
-        if (len1_old_head >= 0)
-            patch_len1(row, cells, len1_old_head, s.head_r * G + s.head_c, s.food_r * G + s.food_c, s.length == 2);
+        if (known_old_head >= 0)
+            patch_known_row(row, cells, known_old_head, known_clear, s.head_r * G + s.head_c, s.food_r * G + s.food_c);
     }
 
     // episode-done compaction + statistics (as snake_kernel, without its one-tile deferral)
@@ -831,6 +849,7 @@ int step(const beng_snake_params *p, const beng_snake_state *st, const int64_t *
     Args a = make_args(p, st, io, n_envs);
     a.actions = (const long long *)actions_dev;
     if (in_place) {
+        if (n_envs > (int64_t)UINT32_MAX) return BENG_ERR_UNSUPPORTED;  // the patch kernel's 32-bit env index
         const long long blocks = (n_envs + PATCH_THREADS - 1) / PATCH_THREADS;
         return (int)launch_pdl(snake_patch_kernel, dim3((unsigned)blocks), dim3(PATCH_THREADS), 0, stream, a);
     }

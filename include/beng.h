@@ -113,7 +113,10 @@ typedef struct beng_snake_io {
      * reset launch then counts its finished envs into count[parity], zeroes count[parity ^ 1] and flips parity for
      * the next launch; `arrivals` is the launch's scratch counter and is 0 again when it ends.  The counter of the
      * last launch is count[parity ^ 1].  A step's arguments are then the same every call (a CUDA graph captures it
-     * once and replays it), and no host state changes per step.  Every other combination is the contract above. */
+     * once and replays it), and no host state changes per step.  Every other combination is the contract above.
+     * beng_snake_step_inplace also takes the parity as its sweep direction: on the self-managed block it visits the
+     * env tiles in descending order every other launch (results are the same either way; only the order of
+     * done_env, which is unspecified, differs), under the contract above always in ascending order. */
     /* running episode statistics, integer (exact, order independent):
      * {n_episodes, sum_return, sum_length, sum_score, max_score} */
     int64_t *stats;         /* [5] accumulated across steps; caller zeroes / all-reduces */
