@@ -46,9 +46,16 @@ constexpr uint32_t FLAG_NEEDS_RESET = 1u;  // NEXT_STEP auto-reset bookkeeping
 constexpr int FOOD_NONE = 255;             // board full: no food on the grid (see place_food)
 
 // ---- 16-byte state record ---------------------------------------------------------------------
+// Byte 0 of v.y: bits 0-1 `dir`, bits 2-3 `last_move` (the direction of the last step that moved the head), bit 4
+// `tail_known` (last_move is valid).  A length-2 body is the head and the cell the head last moved from, so with
+// tail_known its tail is head - delta(last_move) and the ring is not needed (see tail_of).  Deaths and invalid actions
+// do not move the head and leave both fields as they are; a reset clears them.
+constexpr uint32_t DIR_MASK = 3u, LAST_MOVE_SHIFT = 2, TAIL_KNOWN_BIT = 1u << 4;
+
 struct Core {
     int head_r, head_c, food_r, food_c;
-    int dir;
+    int dir, last_move;
+    bool tail_known;
     uint32_t flags;
     int length, steps, ring_head;
     uint32_t ctr;
@@ -60,7 +67,9 @@ __device__ __forceinline__ Core unpack(const uint4 v) {
     s.head_c = (v.x >> 8) & 0xFF;
     s.food_r = (v.x >> 16) & 0xFF;
     s.food_c = (v.x >> 24) & 0xFF;
-    s.dir = v.y & 0xFF;
+    s.dir = v.y & DIR_MASK;
+    s.last_move = (v.y >> LAST_MOVE_SHIFT) & DIR_MASK;
+    s.tail_known = (v.y & TAIL_KNOWN_BIT) != 0;
     s.flags = (v.y >> 8) & 0xFF;
     s.length = (v.y >> 16) & 0xFFFF;
     s.steps = v.z & 0xFFFF;
@@ -72,7 +81,8 @@ __device__ __forceinline__ Core unpack(const uint4 v) {
 __device__ __forceinline__ uint4 pack(const Core &s) {
     uint4 v;
     v.x = (uint32_t)s.head_r | ((uint32_t)s.head_c << 8) | ((uint32_t)s.food_r << 16) | ((uint32_t)s.food_c << 24);
-    v.y = (uint32_t)s.dir | (s.flags << 8) | ((uint32_t)s.length << 16);
+    v.y = (uint32_t)s.dir | ((uint32_t)s.last_move << LAST_MOVE_SHIFT) | (s.tail_known ? TAIL_KNOWN_BIT : 0u) |
+          (s.flags << 8) | ((uint32_t)s.length << 16);
     v.z = (uint32_t)s.steps | ((uint32_t)s.ring_head << 16);
     v.w = s.ctr;
     return v;
@@ -139,11 +149,13 @@ __device__ __forceinline__ auto body_in(const uint8_t *row) {
 }
 
 // The state record of reset (snake_env.py:49-65): a length-1 snake in the centre.  (The ring is not touched: it only
-// holds bodies of length >= 2.)
+// holds bodies of length >= 3.)
 __device__ __forceinline__ void reset_core(Core &s, int G) {
     const int center = G / 2;
     s.head_r = s.head_c = center;
     s.dir = 1;
+    s.last_move = 0;
+    s.tail_known = false;
     s.length = 1;
     s.steps = 0;
     s.ring_head = 0;
@@ -157,15 +169,33 @@ __device__ __forceinline__ void reset_env(Core &s, EnvStream &rng, uint8_t *row,
     place_food(s, rng, G, body_in(row));
 }
 
+// Index of the tail entry in the ring (valid for length >= 3, and for a length-2 snake whose tail is not known).
+__device__ __forceinline__ int tail_index(const Core &s, int cells) {
+    const int idx = s.ring_head - (s.length - 1);
+    return idx < 0 ? idx + cells : idx;
+}
+
+// The tail cell of a length >= 2 snake.  The ring holds bodies of length >= 3 only: a length-2 body is the head and the
+// cell it last moved from, head - delta(last_move), which the state record holds once the snake has moved (tail_known).
+// A length-2 state without the bit (a record written before the bit existed, or built by hand) keeps its tail in the
+// ring, at tail_index; its next move sets the bit.
+__device__ __forceinline__ int tail_of(const Core &s, const uint16_t *ring, int cells, int G) {
+    if (s.length == 2 && s.tail_known) {
+        const int d = s.last_move;  // 0 up, 1 right, 2 down, 3 left
+        return (s.head_r - (d == 2) + (d == 0)) * G + s.head_c - (d == 1) + (d == 3);
+    }
+    return ring[tail_index(s, cells)];
+}
+
 // Walk the body oldest -> newest, writing `mark` into the tile row.  Returns the tail cell and
 // reports whether `probe` is one of the body cells (`new_head in self.snake`, snake_env.py:93).
-// Only called for length >= 2.  `pre_tail` >= 0 is the tail entry fetched one tile ahead; the newest
-// entry always equals the head held in the state record, so a length-2 snake needs no ring load here.
+// Only called for length >= 2.  `pre_tail` >= 0 is the tail cell fetched one tile ahead; the newest
+// entry always equals the head held in the state record, so a length-2 snake needs no ring load here
+// beyond its tail's (none when tail_of finds the tail in the state record).
 __device__ __forceinline__ int scan_body(const Core &s, const uint16_t *ring, uint8_t *row, int cells, int G,
                                          uint8_t mark, int probe, bool &hit, int pre_tail = -1) {
-    int idx = s.ring_head - (s.length - 1);
-    if (idx < 0) idx += cells;
-    const int tail = (pre_tail >= 0) ? pre_tail : (int)ring[idx];
+    int idx = tail_index(s, cells);
+    const int tail = (pre_tail >= 0) ? pre_tail : tail_of(s, ring, cells, G);
     row[tail] = mark;
     hit |= (tail == probe);
     for (int i = 1; i < s.length - 1; ++i) {
@@ -188,12 +218,6 @@ __device__ __forceinline__ uint32_t food_pair(const Core &s, int G) {
 // After reset_env: the row was cleared, then the head and the food were written.
 __device__ __forceinline__ uint32_t reset_record(const Core &s, int G) {
     return BENG_OBS_DELTA_CLEAR | delta_pair(s.head_r * G + s.head_c, 1) | (food_pair(s, G) << 14);
-}
-
-// Index of the tail entry in the ring (valid for length >= 2).
-__device__ __forceinline__ int tail_index(const Core &s, int cells) {
-    const int idx = s.ring_head - (s.length - 1);
-    return idx < 0 ? idx + cells : idx;
 }
 
 // Per-env inputs of one tile, loaded one tile ahead of their use (software pipeline).
@@ -281,12 +305,12 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
     int pend_env = 0;
 
     Loaded cur = load_inputs<IS_RESET>(a, (long long)blockIdx.x * T + tid);
-    // tail ring entry of this thread's env, fetched one tile ahead (-1: not fetched / not needed)
+    // tail cell of this thread's env, fetched one tile ahead (-1: not fetched / not needed)
     int pre_tail = -1;
     if constexpr (!IS_RESET) {
         const long long env0 = (long long)blockIdx.x * T + tid;
         const Core c0 = unpack(cur.raw);
-        if (env0 < a.n_envs && c0.length > 1) pre_tail = a.ring[env0 * cells + tail_index(c0, cells)];
+        if (env0 < a.n_envs && c0.length > 1) pre_tail = tail_of(c0, a.ring + env0 * cells, cells, G);
     }
     int it = 0;
     for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
@@ -377,17 +401,25 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
                         term = 1;
                     } else {
                         const bool eat = new_cell == food_cell;
-                        // insert(0, new_head), :97.  The ring is only maintained for length >= 2: a length-1
-                        // body IS the head held in the state record, which spares 93 % of the envs a scattered
-                        // 2-byte store (a partial-sector write costs a DRAM read-modify-write).
-                        if (s.length > 1 || eat) {
-                            if (s.length == 1) ring[s.ring_head] = (uint16_t)head_cell;
+                        // insert(0, new_head), :97.  The ring is only maintained for length >= 3: a length-1
+                        // body IS the head held in the state record, and a length-2 body the head and the cell
+                        // it came from (last_move, see tail_of).  That spares ~98 % of the env-steps a scattered
+                        // 2-byte store (a partial-sector write costs a DRAM read-modify-write).  The meal that
+                        // makes length 3 writes all three entries, tail first, where tail_index finds them.
+                        if (s.length > 2 || (s.length == 2 && eat)) {
+                            if (s.length == 2) {
+                                ring[s.ring_head] = (uint16_t)tail_cell;
+                                if (++s.ring_head == cells) s.ring_head = 0;
+                                ring[s.ring_head] = (uint16_t)head_cell;
+                            }
                             if (++s.ring_head == cells) s.ring_head = 0;
                             ring[s.ring_head] = (uint16_t)new_cell;
                         }
                         row[new_cell] = 1;
                         s.head_r = nr;
                         s.head_c = nc;
+                        s.last_move = s.dir;
+                        s.tail_known = true;
                         if (eat) {  // :101-104
                             s.length += 1;
                             rew = 10.0f;
@@ -413,7 +445,7 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
                         if (a.mode == BENG_AUTORESET_SAME_STEP) {
                             if (draw) {  // un-draw the body so the row is clean again
                                 // Self-hit death: the body is unchanged.  Time limit: the body is the moved one
-                                // (new head in the state record, everything older in the ring).
+                                // (new head and last_move in the state record, everything older in the ring).
                                 bool hit = false;
                                 if (s.length == 1) row[s.head_r * G + s.head_c] = 0;
                                 else scan_body(s, ring, row, cells, G, 0, -1, hit);
@@ -475,14 +507,14 @@ __global__ void __launch_bounds__(T) snake_kernel(const Args a) {
                 if (a.io.stats) add_warp_stats(s_stats, done_mask, ended, ep_ret, ep_len, ep_score, lane);
             }
         }
-        // Fetch the next tile's tail ring entry now (its state record, requested at the top of this iteration,
-        // has arrived by now) so that the dependent ring load is not exposed at the start of the next tile.
+        // Fetch the next tile's tail cell now (its state record, requested at the top of this iteration, has
+        // arrived by now) so that a dependent ring load is not exposed at the start of the next tile.
         if constexpr (!IS_RESET) {
             pre_tail = -1;
             if (tile_next < n_tiles) {
                 const long long env_n = tile_next * T + tid;
                 const Core cn = unpack(nxt.raw);
-                if (env_n < a.n_envs && cn.length > 1) pre_tail = a.ring[env_n * cells + tail_index(cn, cells)];
+                if (env_n < a.n_envs && cn.length > 1) pre_tail = tail_of(cn, a.ring + env_n * cells, cells, G);
             }
         }
         cur = nxt;
@@ -572,12 +604,14 @@ __device__ __forceinline__ void patch_known_row(uint8_t *row, int cells, int old
     }
 }
 
-// 6 CTAs of 256 threads per SM (<= 40 registers, no spills): the kernel is bound by the latency of its two dependent
-// rounds of loads (state + action, then the row byte + tail entry), so resident threads are what it runs on.  Measured on
-// B200 at 1M envs, G = 20: 61.5 us per step against 65.8 us at the 5 CTAs per SM that 46 registers give.  Measured shape
-// of the whole-sector writes (DESIGN.md section 6f): two 16-byte stores per sector at these 6 CTAs per SM, 55.6 us per
-// step.  One 256-bit store per sector compiles to 46 registers without spills, i.e. 5 CTAs per SM; not timed.
-constexpr int PATCH_THREADS = 256, PATCH_CTAS_PER_SM = 6;
+// 1536 resident threads per SM (<= 40 registers, no spills): the kernel is bound by the latency of its dependent rounds
+// of loads (state + action, then, for a snake of length >= 3, the row byte + tail entry), so resident threads are what
+// it runs on.  Measured on B200 at 1M envs, G = 20: 61.5 us per step against 65.8 us at the 5 x 256 threads per SM that
+// 46 registers give.  Measured shape of the whole-sector writes (DESIGN.md section 6f): two 16-byte stores per sector,
+// 55.6 us per step.  One 256-bit store per sector compiles to 46 registers without spills; not timed.  At the same 1536
+// threads per SM, fewer and larger CTAs are faster, since every CTA pays a fixed prologue and epilogue (the parity read,
+// the arrival, barriers, the statistics flush): 2 CTAs of 768 threads, the fewest that keep 1536 (DESIGN.md section 6i).
+constexpr int PATCH_THREADS = 768, PATCH_CTAS_PER_SM = 2;
 
 // The step kernel of beng_snake_step_inplace: same dynamics, rewards, flags, state and statistics as snake_kernel, but
 // io.obs must already hold the observation of the previous reset or step, and only the cells that change are written
@@ -585,9 +619,11 @@ constexpr int PATCH_THREADS = 256, PATCH_CTAS_PER_SM = 6;
 // head -> 1, food -> 2 -- the order of the BENG_OBS_DELTA records).  One thread per env and no shared-memory tile:
 //   * the previous observation is the occupancy map, so self-collision (`new_head in self.snake`, tail included,
 //     snake_env.py:93) is the byte obs[new_cell] == 1 instead of a walk over the ring (for length 2, new_cell == tail);
-//     the ring is read only for the tail cell a move of a length >= 2 snake clears, and written only where
-//     snake_kernel writes it;
-//   * the food rejection loop after a meal reads the same row, with the new head already written over the old food;
+//     the ring is read only for the tail cell a move of a length >= 3 snake clears (a length-2 tail comes from the
+//     state record, tail_of), and written only where snake_kernel writes it, so a length <= 2 step loads nothing but
+//     the state record and the action;
+//   * the food rejection loop after a meal of a length >= 3 snake reads the same row, with the new head already
+//     written over the old food; shorter snakes test their two or three body cells in registers;
 //   * a step that does not reset of a length-1 snake (about 91 % of env-steps at G = 20 with random actions), or a
 //     non-eating move of a length-2 snake (about 6 %), writes the 32-byte sectors holding its changed cells whole, with
 //     two 16-byte stores each (patch_known_row), and byte stores only where a sector reaches into a neighbouring row;
@@ -646,7 +682,9 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
             bool self_hit = false;  // (a length-1 snake cannot hit itself)
             int tail_cell = head_cell;
             if (!wall && s.length > 1) {
-                tail_cell = ring[tail_index(s, cells)];  // (both loads are issued before either is used)
+                // length 2: the tail from the state record (a ring load only for a record without tail_known);
+                // length >= 3: the ring entry and the row byte, both loads issued before either is used
+                tail_cell = tail_of(s, ring, cells, G);
                 // a length-2 body is the head, which the new head never is, and the tail: no row load
                 self_hit = s.length == 2 ? new_cell == tail_cell : row[new_cell] == 1;
             }
@@ -656,13 +694,19 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
                 term = 1;
             } else {
                 const bool eat = new_cell == food_cell;
-                if (s.length > 1 || eat) {  // insert(0, new_head), :97 (the lazy ring of snake_kernel)
-                    if (s.length == 1) ring[s.ring_head] = (uint16_t)head_cell;
+                if (s.length > 2 || (s.length == 2 && eat)) {  // insert(0, new_head), :97 (the lazy ring of snake_kernel)
+                    if (s.length == 2) {
+                        ring[s.ring_head] = (uint16_t)tail_cell;
+                        if (++s.ring_head == cells) s.ring_head = 0;
+                        ring[s.ring_head] = (uint16_t)head_cell;
+                    }
                     if (++s.ring_head == cells) s.ring_head = 0;
                     ring[s.ring_head] = (uint16_t)new_cell;
                 }
                 s.head_r = nr;
                 s.head_c = nc;
+                s.last_move = s.dir;
+                s.tail_known = true;
                 const bool len1 = s.length == 1;
                 const bool known = len1 || (s.length == 2 && !eat);
                 if (known) {
@@ -670,12 +714,17 @@ __global__ void __launch_bounds__(PATCH_THREADS, PATCH_CTAS_PER_SM) snake_patch_
                     known_clear = eat ? -1 : tail_cell;  // (a length-1 snake's tail_cell is its old head)
                 }
                 if (eat) {  // :101-104
-                    // The rejection loop reads the row, with the new head marked over the old food.  A length-1 snake
-                    // leaves its row to patch_known_row: there the old food's 2 marks the new head just as well.
+                    // The rejection loop of a length-1 or length-2 snake tests the body cells it holds in registers
+                    // (new head, old head, tail; a length-1 snake's tail_cell is its old head); a longer one reads
+                    // the row, with the new head marked over the old food.  A length-1 snake leaves its row to
+                    // patch_known_row.
+                    const bool short_body = s.length <= 2;
                     if (!len1) row[new_cell] = 1;
                     s.length += 1;
                     rew = 10.0f;
-                    place_food(s, rng, G, body_in(row));
+                    place_food(s, rng, G, [=](int cell) {
+                        return short_body ? cell == new_cell || cell == head_cell || cell == tail_cell : row[cell] != 0;
+                    });
                     if (!len1 && s.food_r != FOOD_NONE) row[s.food_r * G + s.food_c] = 2;
                 } else if (!known) {
                     row[tail_cell] = 0;  // pop(), :107
@@ -750,12 +799,14 @@ __global__ void __launch_bounds__(256) snake_export_kernel(const uint4 *__restri
     if (steps) steps[e] = s.steps;
     if (length) length[e] = s.length;
     if (ctr) ctr[e] = s.ctr;
-    if (body) {
+    if (body) {  // newest -> oldest; a length-1 body and a length-2 one with tail_known are in the state record
         const int cells = G * G;
+        const int head = s.head_r * G + s.head_c;
+        const bool in_core = s.length == 1 || (s.length == 2 && s.tail_known);
         int idx = s.ring_head;
         for (int i = 0; i < cells; ++i) {
             int c = -1;
-            if (i < s.length) c = (s.length == 1) ? s.head_r * G + s.head_c : (int)ring[e * cells + idx];
+            if (i < s.length) c = !in_core ? (int)ring[e * cells + idx] : i == 0 ? head : tail_of(s, ring, cells, G);
             body[e * cells + i] = c;
             if (--idx < 0) idx = cells - 1;
         }

@@ -83,9 +83,14 @@ typedef struct beng_snake_params {
  *   core : n_envs x 16 B record {u8 head_r, head_c, food_r, food_c; u8 direction; u8 flags;
  *          u16 length; u16 steps; u16 ring_head; u32 rng_counter}  -- one 128-bit load per env.
  *          (`score` is not stored: score == length - 1 always, snake_env.py:57,102 vs :97,107.)
+ *          The direction byte: bits 0-1 the direction, bits 2-3 the direction of the last step
+ *          that moved the head, bit 4 set when bits 2-3 are valid (every move or meal sets them,
+ *          a reset clears them).
  *   ring : n_envs x (grid_size^2) u16 body cells (r * G + c); newest at ring_head, oldest
  *          (the tail) at ring_head - length + 1 (mod G^2).  Replaces the Python list
- *          `self.snake` (snake_env.py:54,97,107). */
+ *          `self.snake` (snake_env.py:54,97,107).  Only maintained from length 3 on: a length-1
+ *          body is the head, a length-2 body with bit 4 set is the head and the cell one step
+ *          against the last move; a length-2 record without bit 4 keeps its tail in the ring. */
 typedef struct beng_snake_state {
     void *core;     /* uint4[n_envs] */
     uint16_t *ring; /* uint16_t[n_envs * grid_size * grid_size] */
